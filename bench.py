@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W [--config NAME]   # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K ...         # the CPU path (oracle restatement) on the host cores
+  python bench.py ... --dump-outputs DIR                          # also save the last timed step's outputs (see dump_outputs)
 
 A "step" is one tick of every env of the batch (one hk_step call per GPU): physics, contact sensing, rewards,
 observation write, in-kernel opponents and auto-reset.  Workloads (`--config`, BASELINE.json `configs`):
@@ -41,6 +42,8 @@ ALGO_BYTES_FUSED, ALGO_BYTES_EXTERNAL = 285, 317
 STORED_BYTES_FUSED = 256 + 256 + 72 + 4 + 1 + 16
 ISSUE_PEAK_WARP_INST_PER_S = 148 * 4 * 1.965e9  # SURVEY 8(d): 148 SMs x 4 schedulers x 1 warp-inst/clk x 1.965 GHz
 PREROLL_TICKS = 400
+DUMP_BYTES = 60 << 20  # --dump-outputs: above this, a fixed sample of env rows is written (keeps a dump under 64 MB)
+DUMP_SAMPLE_SEED = 0
 
 CONFIGS = {
     "normal65k": dict(mode="NORMAL", p1="strong", p2="strong", per_gpu=65536, total=None,
@@ -227,6 +230,35 @@ def cpu_baseline(args, c, budget_s=12.0):
             "sample": f"{n} of {c['n']} envs x {steps} ticks after a {PREROLL_TICKS}+ tick pre-roll, {cores} threads, {dt:.1f} s"}
 
 
+def dump_outputs(out_dir, arrays, rank, world):
+    """--dump-outputs: writes what the last timed step returned to its caller as out_dir/<name>.npy (float32), in global
+    env order (gathered from all ranks), so that two builds can be compared output for output.  env_index.npy (float64)
+    names the rows: all envs, or, when that would exceed DUMP_BYTES, one fixed seeded sample of them for every array."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    arrays = {k: v.to(torch.float32).contiguous() for k, v in arrays.items()}
+    if world > 1:
+        for k, v in arrays.items():
+            g = v.new_empty((world * v.shape[0],) + tuple(v.shape[1:]))
+            dist.all_gather_into_tensor(g, v)
+            arrays[k] = g
+    if rank != 0:
+        return None
+    total = next(iter(arrays.values())).shape[0]
+    row_bytes = 8 + sum(4 * v[0].numel() for v in arrays.values())
+    rows = min(total, DUMP_BYTES // row_bytes)
+    idx = np.arange(total)
+    if rows < total:
+        idx = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(total, rows, replace=False))
+    dev_idx = torch.from_numpy(idx).to(next(iter(arrays.values())).device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.index_select(0, dev_idx).cpu().numpy())
+    return {"dir": out_dir, "arrays": ["env_index"] + sorted(arrays), "rows": int(rows), "of_envs": int(total)}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -246,7 +278,10 @@ def main():
                     help="HockeyVecEnv.step_host mode: one D2H copy of the packed record after the tick (default), DMA of the fast "
                          "tier's rows overlapped with the general tier, or zero-copy stores only")
     ap.add_argument("--rollout-k", type=int, default=64, help="ticks per hk_rollout call of the fused-rollout leg (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -281,9 +316,9 @@ def main():
     ev_actor = []
 
     def tick(timed=False):
+        """Returns what the step hands its caller: HockeyVecEnv.step's tuple and player 1's actions (None if in-kernel)."""
         if actor is None:
-            env.step()
-            return
+            return env.step(), None
         with torch.no_grad():
             if timed:
                 a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -292,7 +327,7 @@ def main():
             if timed:
                 a1.record()
                 ev_actor.append((a0, a1))
-            env.step(a)
+            return env.step(a), a
 
     def barrier():
         torch.cuda.synchronize(dev)
@@ -331,10 +366,18 @@ def main():
         if flush is not None:
             flush.zero_()
         ev[k][0].record()
-        tick(timed=True)
+        last = tick(timed=True)
         ev[k][1].record()
     barrier()
     clocks = sampler.stop()
+    dumped = None
+    if args.dump_outputs:  # before the legs below step the env again and overwrite its output buffers
+        (obs, reward, done, truncated, info), action = last
+        arrays = {"obs": obs, "reward": reward, "done": done, "truncated": truncated}
+        arrays.update({f"info_{k}": v for k, v in info.items()})
+        if action is not None:
+            arrays["action"] = action
+        dumped = dump_outputs(args.dump_outputs, arrays, rank, world)
     kernel_ms = sum(a.elapsed_time(b) for a, b in ev)
     actor_ms = sum(a.elapsed_time(b) for a, b in ev_actor)
     ktimes, ksteps = env.kernel_times()
@@ -483,6 +526,8 @@ def main():
                             "ms_per_step": actor_ms / args.steps, "share_of_step": actor_ms / max(kernel_ms, 1e-9),
                             "weights": "tests/golden/td3_actors.npz:stage_3 (pretrained/stage_3/models/td3_best.pt)",
                             "flops_per_env": 2 * (18 * 256 + 256 * 256 + 256 * 4)}
+        if dumped is not None:
+            out["dump_outputs"] = dumped
         if st[0] <= 0:
             out["warning"] = "no episode finished in the timed region"
         if world == 1 and not args.no_cpu_baseline:
