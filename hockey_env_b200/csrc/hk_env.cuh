@@ -138,8 +138,9 @@ HK_HD void getObs2(const Env& e, float* o) {
 }
 
 // _get_info / get_info_agent_two (hockey_env.py:542-591): out = winner, closeness, touch, direction
-HK_NI_FASTA void getInfo(const Config& cfg, const Env& e, bool agent_two, double* out) {
+HK_NI_FASTA void getInfo(const Env& e, bool agent_two, double* out) {
   const Body &p1 = e.b[B_R1], &p2 = e.b[B_R2], &pk = e.b[B_PUCK];
+  const int max_timesteps = maxTimesteps(e.mode);
   double closeness = 0;
   bool cond = agent_two ? ((double)pk.p.x > HK_CENTER_X && (double)pk.v.x >= 0) : ((double)pk.p.x < HK_CENTER_X && (double)pk.v.x <= 0);
   if (cond) {
@@ -147,12 +148,12 @@ HK_NI_FASTA void getInfo(const Config& cfg, const Env& e, bool agent_two, double
     double dist = sqrt((double)d.x * (double)d.x + (double)d.y * (double)d.y);
     double max_dist = 250. / HK_SCALE;
     double max_reward = -30.;
-    double factor = max_reward / (max_dist * cfg.max_timesteps / 2);
+    double factor = max_reward / (max_dist * max_timesteps / 2);
     closeness += dist * factor;
   }
   double touch = 0.;
   if ((agent_two ? e.has2 : e.has1) == HK_MAX_TIME_KEEP_PUCK) touch = 1.;
-  double factor = (agent_two ? -1.0 : 1.0) / (cfg.max_timesteps * HK_MAX_PUCK_SPEED);
+  double factor = (agent_two ? -1.0 : 1.0) / (max_timesteps * HK_MAX_PUCK_SPEED);
   out[0] = agent_two ? -e.winner : e.winner;
   out[1] = closeness;
   out[2] = touch;
@@ -211,7 +212,7 @@ HK_NI_POLICY void basicAct(const Config& cfg, const float* obs, bool weak, doubl
 // reset (hockey_env.py:345-418): overwrite per-env state; the scene itself is constant
 // reset_seed >= 0 (HockeyEnv.reset(seed=...), hockey_env.py:347 `self.seed(seed)`): the draws are a function of that seed
 // alone -- the same seed gives the same start state on any env of any batch; otherwise they come from the env's own
-// stream (library seed, global env id, episode counter)
+// stream (library seed, global env id, episode counter).  The mode never enters a draw's key.
 #define HK_SEEDED_RESET_TAG 0x5EEDED5EEDull
 HK_HD double resetDraw(const Config& cfg, uint64_t env_id, uint32_t episode, int64_t reset_seed, int idx, double lo, double hi) {
   U4 r = reset_seed >= 0 ? philox((uint64_t)reset_seed, HK_SEEDED_RESET_TAG, 0u, (uint32_t)HK_STREAM_RESET | ((uint32_t)(idx >> 1) << 8))
@@ -241,13 +242,17 @@ HK_HD void createDynamicBody(const Scene& S, Env& e, int bi, double px, double p
   e.fat[bi].hx = a.hx + HK_AABB_EXTENSION;
   e.fat[bi].hy = a.hy + HK_AABB_EXTENSION;
 }
+// next_mode: HK_MODE_* of the episode this reset starts (the reference's `mode` setter / reset(mode=...) takes effect
+// here, hockey_env.py:350-364), -1 = keep the env's mode
 HK_NI_RARE void envReset(const Scene& S, const Config& cfg, Env& e, uint64_t env_id, int one_starting /* -1 = alternate */,
-                             int64_t reset_seed = -1) {
+                             int64_t reset_seed = -1, int next_mode = -1) {
   e.done = false;
   e.winner = 0;
   e.time = 0;
+  if (next_mode >= 0) e.mode = next_mode;
+  const int mode = e.mode;
   // the reference does not clear player{1,2}_has_puck on reset
-  if (cfg.mode == 0) {
+  if (mode == 0) {
     if (one_starting >= 0) e.one_starts = one_starting != 0;
     else e.one_starts = !e.one_starts;
   }
@@ -259,17 +264,17 @@ HK_NI_RARE void envReset(const Scene& S, const Config& cfg, Env& e, uint64_t env
   e.moved = 15u;
   createDynamicBody(S, e, B_R1, HK_W / 5, HK_H / 2);
   int draw = 0;
-  if (cfg.mode != 0) {
+  if (mode != 0) {
     double dx = resetDraw(cfg, env_id, e.episode, reset_seed, draw++, -HK_W / 3, HK_W / 6);
     double dy = resetDraw(cfg, env_id, e.episode, reset_seed, draw++, -HK_H / 4, HK_H / 4);
     createDynamicBody(S, e, B_R2, 4 * HK_W / 5 + dx, HK_H / 2 + dy);
   } else {
     createDynamicBody(S, e, B_R2, 4 * HK_W / 5, HK_H / 2);
   }
-  if (cfg.mode == 0 || cfg.mode == 1) {
+  if (mode == 0 || mode == 1) {
     double dx = resetDraw(cfg, env_id, e.episode, reset_seed, draw++, HK_H / 8, HK_H / 4);
     double dy = resetDraw(cfg, env_id, e.episode, reset_seed, draw++, -HK_H / 8, HK_H / 8);
-    if (e.one_starts || cfg.mode == 1) createDynamicBody(S, e, B_PUCK, HK_W / 2 - dx, HK_H / 2 + dy);
+    if (e.one_starts || mode == 1) createDynamicBody(S, e, B_PUCK, HK_W / 2 - dx, HK_H / 2 + dy);
     else createDynamicBody(S, e, B_PUCK, HK_W / 2 + dx, HK_H / 2 + dy);
   } else {
     double dx = resetDraw(cfg, env_id, e.episode, reset_seed, draw++, 0, HK_W / 3);
@@ -363,8 +368,8 @@ HK_HD_NOINLINE void envStepActions(const Scene& S, const Config& cfg, Env& e, co
     }
   }
 }
-HK_HD void envStepAfterWorld(const Config& cfg, Env& e) {
-  if (e.time >= cfg.max_timesteps) e.done = true;
+HK_HD void envStepAfterWorld(Env& e) {
+  if (e.time >= maxTimesteps(e.mode)) e.done = true;
   e.time += 1;
   ++e.tick;
 }
@@ -372,7 +377,7 @@ HK_HD_NOINLINE void envStep(const Scene& S, const Config& cfg, const Cache& cach
   envStepActions(S, cfg, e, action);
   worldStep(S, cfg, cache, e, (float)(1.0 / HK_FPS), 6 * 30, 2 * 30);
   if (e.aborted) return;
-  envStepAfterWorld(cfg, e);
+  envStepAfterWorld(e);
 }
 
 }  // namespace hk

@@ -257,7 +257,7 @@ HK_HD bool envStepTouch(const Scene& S, const Config& cfg, const Cache& cache, E
   e.allowToiEvents = true;
   e.aborted = false;
   if (!worldStepTouch(S, cfg, cache, e, (float)(1.0 / HK_FPS))) return false;
-  envStepAfterWorld(cfg, e);
+  envStepAfterWorld(e);
   return true;
 }
 
@@ -275,7 +275,7 @@ HK_HD bool envStepFast(const Scene& S, const Config& cfg, Env& e, const float ac
     puck.ldamp = puck_speed > HK_MAX_PUCK_SPEED ? 10.0f : 0.05f;
   }
   if (!worldStepFast(S, cfg, e, (float)(1.0 / HK_FPS))) return false;
-  if (e.time >= cfg.max_timesteps) e.done = true;
+  if (e.time >= maxTimesteps(e.mode)) e.done = true;
   e.time += 1;
   ++e.tick;
   return true;

@@ -170,7 +170,8 @@ __global__ void __launch_bounds__(kBlock) k_create(KParams P) {
   storeEnv(P.core, P.n, i, e);
 }
 
-__global__ void __launch_bounds__(kBlock) k_reset(KParams P, const uint8_t* mask, const int8_t* one_starting, const int64_t* seeds, float* obs) {
+__global__ void __launch_bounds__(kBlock) k_reset(KParams P, const uint8_t* mask, const int8_t* one_starting, const int64_t* seeds,
+                                                  const uint8_t* modes, float* obs) {
   __shared__ Scene S;
   stageScene(&S);
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -178,7 +179,8 @@ __global__ void __launch_bounds__(kBlock) k_reset(KParams P, const uint8_t* mask
   if (mask && !mask[i]) return;
   Env e;
   loadEnv(P.core, P.n, i, e);
-  envReset(S, P.cfg, e, (uint64_t)(P.env_id_offset + i), one_starting ? (int)one_starting[i] : -1, seeds ? seeds[i] : -1);
+  envReset(S, P.cfg, e, (uint64_t)(P.env_id_offset + i), one_starting ? (int)one_starting[i] : -1, seeds ? seeds[i] : -1,
+           modes ? (int)modes[i] : -1);
   storeEnv(P.core, P.n, i, e);
   if (obs) {
     float o[18];
@@ -355,7 +357,7 @@ __global__ void __launch_bounds__(kTouchBlock, 1) k_touch(KParams P, StepIO io) 
   __syncthreads();
   if (live) live = worldStepTouchFinish(S, cache, e);
   if (live) {
-    envStepAfterWorld(P.cfg, e);
+    envStepAfterWorld(e);
     tickFinish(S, P.cfg, e, (uint64_t)(P.env_id_offset + i), (size_t)i, io, io.write != 0, st, had1, had2);
     storeEnv(P.core, P.n, i, e);
   }
@@ -755,7 +757,7 @@ __device__ __forceinline__ void generalTick(const KParams& P, const StepIO& io, 
   if (valid) {  // phase 4: commit, rewards, outputs, auto-reset, store
     if (!e.aborted) {
       worldStepFinish(cache, e);
-      envStepAfterWorld(P.cfg, e);
+      envStepAfterWorld(e);
       tf1 = clock64();
       if (P.trace && e.done) atomicAdd(&sFin[3], 1u);
       tickFinish(S, P.cfg, e, env_id, (size_t)i, io, laneWrite, st, had1, had2);
@@ -1201,11 +1203,11 @@ __global__ void __launch_bounds__(kBlock) k_get_info(KParams P, float* info, flo
   loadEnv(P.core, P.n, i, e);
   double v[4];
   if (info) {
-    getInfo(P.cfg, e, false, v);
+    getInfo(e, false, v);
     for (int k = 0; k < 4; ++k) info[4 * i + k] = (float)v[k];
   }
   if (info2) {
-    getInfo(P.cfg, e, true, v);
+    getInfo(e, true, v);
     for (int k = 0; k < 4; ++k) info2[4 * i + k] = (float)v[k];
   }
 }
@@ -1218,7 +1220,9 @@ __global__ void __launch_bounds__(kBlock) k_get_state(KParams P, uint32_t* rec) 
   Cache cache;
   cache.base = P.cache + i;
   cache.stride = (size_t)P.n;
-  packRecord(e, cache, rec + (size_t)HK_STATE_WORDS * i);
+  uint32_t* r = rec + (size_t)HK_STATE_WORDS * i;
+  packRecord(e, cache, r);
+  r[HK_S_MODE] = modeWord(e, P.cfg.mode);
 }
 
 __global__ void __launch_bounds__(kBlock) k_set_state(KParams P, const uint32_t* rec) {
@@ -1228,8 +1232,18 @@ __global__ void __launch_bounds__(kBlock) k_set_state(KParams P, const uint32_t*
   Cache cache;
   cache.base = P.cache + i;
   cache.stride = (size_t)P.n;
-  unpackRecord(rec + (size_t)HK_STATE_WORDS * i, e, cache);
+  const uint32_t* r = rec + (size_t)HK_STATE_WORDS * i;
+  unpackRecord(r, e, cache);
+  e.mode = modeOfWord(r[HK_S_MODE], P.cfg.mode);
   storeEnv(P.core, P.n, i, e);
+}
+
+__global__ void __launch_bounds__(kBlock) k_get_modes(KParams P, uint8_t* modes) {
+  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.n) return;
+  Env e;
+  loadEnv(P.core, P.n, i, e);
+  modes[i] = (uint8_t)e.mode;
 }
 
 __global__ void __launch_bounds__(kBlock) k_set_obs_state(KParams P, const float* obs18) {
@@ -1261,6 +1275,7 @@ struct hk_env {
   float* actBuf;
   uint32_t* trace;
   const uint8_t* pol2v = nullptr;  // hk_set_opponent_policies
+  const uint8_t* resetModes = nullptr;  // hk_set_reset_modes
   bool fused = false;     // HK_FUSED=1: hk_rollout = ONE launch of k_rollout_fused instead of K x the per-tick cascade (measured
                           // slower on B200: profiles/README.md, fused rollout)
   int fusedFastRun = 4;   // HK_FUSED_FAST_RUN: consecutive fast ticks a lane takes with its state in registers before it is re-queued
@@ -1427,9 +1442,22 @@ __global__ void k_sum_stats(const double* rows, double* out) {  // <<<1, HK_STAT
   out[threadIdx.x] = s;
 }
 
-__global__ void k_check_codes(const uint8_t* codes, int64_t n, int* bad) {
+__global__ void k_check_codes(const uint8_t* codes, int64_t n, int maxCode, int* bad) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n && codes[i] > HK_POLICY_ZERO) atomicAdd(bad, 1);
+  if (i < n && codes[i] > maxCode) atomicAdd(bad, 1);
+}
+// one-time validation of the initial contents of a per-env code table (later rewrites are the caller's responsibility)
+static int checkCodes(const hk_env* h, const uint8_t* codes_dev, int maxCode, const char* msg) {
+  DeviceGuard guard(h->device);
+  int* bad = nullptr;
+  int hostBad = 0;
+  HK_CUDA(cudaMalloc(&bad, sizeof(int)));
+  cudaMemset(bad, 0, sizeof(int));
+  k_check_codes<<<h->grid(), kBlock>>>(codes_dev, h->n, maxCode, bad);
+  cudaError_t err = cudaMemcpy(&hostBad, bad, sizeof(int), cudaMemcpyDeviceToHost);
+  cudaFree(bad);
+  HK_CUDA(err);
+  return hostBad ? fail(HK_E_INVALID, msg) : HK_OK;
 }
 
 extern "C" {
@@ -1455,7 +1483,7 @@ int hk_create(hk_env** out, int64_t n_envs, int mode, int keep_mode, int device,
   h->env_id_offset = env_id_offset;
   h->cfg.mode = mode;
   h->cfg.keep_mode = keep_mode ? 1 : 0;
-  h->cfg.max_timesteps = mode == HK_MODE_NORMAL ? 250 : 80;  // hockey_env.py:357-364
+  h->cfg.max_timesteps = maxTimesteps(mode);
   h->cfg.seed = seed;
   h->core = nullptr;
   h->cache = nullptr;
@@ -1596,7 +1624,7 @@ int hk_reset_seeded(hk_env* h, const uint8_t* mask_dev, const int8_t* one_starti
                     void* stream) {
   if (!h) return fail(HK_E_INVALID, "hk_reset: NULL handle");
   DeviceGuard guard(h->device);
-  k_reset<<<h->grid(), kBlock, 0, (cudaStream_t)stream>>>(h->params(), mask_dev, one_starting_dev, seeds_dev, obs_dev);
+  k_reset<<<h->grid(), kBlock, 0, (cudaStream_t)stream>>>(h->params(), mask_dev, one_starting_dev, seeds_dev, h->resetModes, obs_dev);
   HK_CUDA(cudaGetLastError());
   return HK_OK;
 }
@@ -1631,6 +1659,7 @@ int hk_step(hk_env* h, const float* action_dev, int action_stride, int p1_policy
   io.pol1 = p1_policy;
   io.pol2 = perEnv ? HK_POLICY_ZERO : p2_policy;
   io.pol2v = perEnv ? h->pol2v : nullptr;
+  io.resetModes = h->resetModes;
   io.flags = flags;
   io.obs = obs_dev;
   io.obs2 = obs2_dev;
@@ -1734,6 +1763,7 @@ int hk_step_host(hk_env* h, const float* action_host, int action_stride, int p1_
   io.pol1 = p1_policy;
   io.pol2 = perEnv ? HK_POLICY_ZERO : p2_policy;
   io.pol2v = perEnv ? h->pol2v : nullptr;
+  io.resetModes = h->resetModes;
   io.flags = flags;
   io.write = 1;
   StepIO ioDev = recordIO(io, record_dev, off, with_final_obs);
@@ -1757,19 +1787,29 @@ int hk_step_host(hk_env* h, const float* action_host, int action_stride, int p1_
 
 int hk_set_opponent_policies(hk_env* h, const uint8_t* codes_dev) {
   if (!h) return fail(HK_E_INVALID, "hk_set_opponent_policies: NULL handle");
-  if (codes_dev) {  // one-time validation of the initial contents (later rewrites are the caller's responsibility)
-    DeviceGuard guard(h->device);
-    int* bad = nullptr;
-    int hostBad = 0;
-    HK_CUDA(cudaMalloc(&bad, sizeof(int)));
-    cudaMemset(bad, 0, sizeof(int));
-    k_check_codes<<<h->grid(), kBlock>>>(codes_dev, h->n, bad);
-    cudaError_t err = cudaMemcpy(&hostBad, bad, sizeof(int), cudaMemcpyDeviceToHost);
-    cudaFree(bad);
-    HK_CUDA(err);
-    if (hostBad) return fail(HK_E_INVALID, "hk_set_opponent_policies: codes must be HK_POLICY_EXTERNAL..HK_POLICY_ZERO");
+  if (codes_dev) {
+    const int rc = checkCodes(h, codes_dev, HK_POLICY_ZERO, "hk_set_opponent_policies: codes must be HK_POLICY_EXTERNAL..HK_POLICY_ZERO");
+    if (rc != HK_OK) return rc;
   }
   h->pol2v = codes_dev;
+  return HK_OK;
+}
+
+int hk_set_reset_modes(hk_env* h, const uint8_t* modes_dev) {
+  if (!h) return fail(HK_E_INVALID, "hk_set_reset_modes: NULL handle");
+  if (modes_dev) {
+    const int rc = checkCodes(h, modes_dev, HK_MODE_TRAIN_DEFENSE, "hk_set_reset_modes: modes must be HK_MODE_NORMAL..HK_MODE_TRAIN_DEFENSE");
+    if (rc != HK_OK) return rc;
+  }
+  h->resetModes = modes_dev;
+  return HK_OK;
+}
+
+int hk_get_modes(hk_env* h, uint8_t* modes_dev, void* stream) {
+  if (!h || !modes_dev) return fail(HK_E_INVALID, "hk_get_modes: NULL argument");
+  DeviceGuard guard(h->device);
+  k_get_modes<<<h->grid(), kBlock, 0, (cudaStream_t)stream>>>(h->params(), modes_dev);
+  HK_CUDA(cudaGetLastError());
   return HK_OK;
 }
 
@@ -1783,6 +1823,7 @@ int hk_rollout(hk_env* h, int k_steps, int p1_policy, int p2_policy, float* obs_
   std::memset(&io, 0, sizeof(io));
   io.pol1 = p1_policy;
   io.pol2 = p2_policy;
+  io.resetModes = h->resetModes;
   io.flags = HK_STEP_AUTORESET;
   io.obs = obs_dev;
   if (h->mono) {  // K ticks fused in one launch, state in registers between ticks (the round-1 baseline kernel)

@@ -54,7 +54,7 @@ HK_HD void envToGroups(const Env& e, F4* g) {
   g[6] = F4{pk.a, pk.w, pk.f.x, pk.f.y};
   uint32_t flags = (r1.awake ? 1u : 0u) | (r2.awake ? 2u : 0u) | (pk.awake ? 4u : 0u) | (e.done ? 8u : 0u) |
                    (e.one_starts ? 16u : 0u) | ((uint32_t)(e.winner + 1) << 5) | ((e.moved & 15u) << 8) |
-                   ((uint32_t)e.ncontacts << 12);
+                   ((uint32_t)e.ncontacts << 12) | ((uint32_t)e.mode << 16);
   g[7] = F4{r1.sleep, r2.sleep, pk.sleep, u2f(flags)};
   for (int k = 0; k < 3; ++k) g[8 + k] = F4{e.fat[k].lx, e.fat[k].ly, e.fat[k].hx, e.fat[k].hy};
   dbl2words(e.phase[0], &g[11].x, &g[11].y);
@@ -86,6 +86,7 @@ HK_HD void groupsToEnv(const F4* g, Env& e) {
   e.winner = (int)((flags >> 5) & 3u) - 1;
   e.moved = (flags >> 8) & 15u;
   e.ncontacts = (int)((flags >> 12) & 15u);
+  e.mode = (int)((flags >> 16) & 3u);
   for (int k = 0; k < 3; ++k) {
     e.fat[k].lx = g[8 + k].x; e.fat[k].ly = g[8 + k].y; e.fat[k].hx = g[8 + k].z; e.fat[k].hy = g[8 + k].w;
   }
@@ -277,6 +278,12 @@ HK_HD void unpackRecord(const uint32_t* r, Env& e, const Cache& cache) {
   e.dbgEvalClk = e.dbgEventClk = 0;
   e.toiPreFlag = 0;
 }
+
+// record word HK_S_MODE (56).  createMode = the handle's creation mode (Config::mode): the word holds 0 while the env
+// plays it, else mode + 1, so that the records of single-mode handles do not depend on it.  On reading, 1..3 = mode
+// 0..2; 0 (single-mode records, records of builds without per-env modes) and any other value = createMode.
+HK_HD uint32_t modeWord(const Env& e, int createMode) { return e.mode == createMode ? 0u : (uint32_t)e.mode + 1u; }
+HK_HD int modeOfWord(uint32_t w, int createMode) { return w >= 1u && w <= 3u ? (int)w - 1 : createMode; }
 
 // HockeyEnv.set_state (hockey_env.py:594-608): 18 visible values; goes through b2Body::SetTransform
 // / SetLinearVelocity / SetAngularVelocity semantics like the reference's property setters.

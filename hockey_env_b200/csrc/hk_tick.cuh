@@ -12,6 +12,7 @@ struct StepIO {
   int stride;
   int pol1, pol2, flags;
   const uint8_t* pol2v;  // per-env player-2 policy codes (HK_POLICY_PER_ENV) or null
+  const uint8_t* resetModes = nullptr;  // per-env HK_MODE_* of the episode an auto-reset starts (hk_set_reset_modes) or null: keep
   float* obs;        // [n,18]
   float* obs2;       // [n,18] or null
   float* reward;     // [n] or null
@@ -87,8 +88,8 @@ __device__ __forceinline__ void warpStoreRows18(float* __restrict__ dst, const f
 HK_NI_FASTA void tickFinish(const Scene& S, const Config& cfg, Env& e, uint64_t env_id, size_t i, const StepIO& io, bool write,
                       TickStats& st, int had1, int had2, bool* deferRows = nullptr) {
   double inf[4], inf2[4];
-  getInfo(cfg, e, false, inf);
-  getInfo(cfg, e, true, inf2);
+  getInfo(e, false, inf);
+  getInfo(e, true, inf2);
   const double cr = computeReward(e);
   const double r = cr + inf[1];
   const double r2 = -cr + inf2[1];
@@ -125,7 +126,7 @@ HK_NI_FASTA void tickFinish(const Scene& S, const Config& cfg, Env& e, uint64_t 
     st.ret2 += e.ret[1];
     st.ret1sq += e.ret[0] * e.ret[0];
     st.len += e.time;
-    envReset(S, cfg, e, env_id, -1);
+    envReset(S, cfg, e, env_id, -1, -1, io.resetModes ? (int)io.resetModes[i] : -1);
   }
   if (write) {
     float o[18];
@@ -195,6 +196,7 @@ HK_HD bool envTickTouch(const Scene& S, const Config& cfg, const Cache& cache, E
 HK_HD void envCreate(const Scene& S, const Config& cfg, Env& e, uint64_t env_id) {
   e.has1 = e.has2 = 0;
   e.one_starts = true;
+  e.mode = cfg.mode;
   e.episode = 0;
   e.tick = 0;
   e.nVelIters = e.nToiEvents = e.nOverflow = 0;

@@ -76,6 +76,7 @@ struct Env {
   Body b[3];
   int has1, has2, time, winner;
   bool done, one_starts;
+  int mode;  // HK_MODE_* of the running episode (chosen at its reset)
   AABB fat[3];
   uint32_t moved;  // bit0-2: buffered proxy moves (r1, r2, puck); bit3: new fixtures since last step
   double phase[2];
@@ -119,9 +120,13 @@ HK_HD void setSep(Env& e, int pid, float bound, V2 normal) {
 }
 
 struct Config {
-  int mode, keep_mode, max_timesteps;
+  int mode;           // the handle's creation mode: the mode of new envs, and what record word HK_S_MODE = 0 stands for
+  int keep_mode;
+  int max_timesteps;  // of the creation mode; a tick reads its env's own limit, maxTimesteps(e.mode)
   uint64_t seed;
 };
+// max_timesteps of an episode in `mode` (hockey_env.py:357-364)
+HK_HD int maxTimesteps(int mode) { return mode == 0 ? 250 : 80; }
 
 HK_HD int clistGet(uint64_t l, int i) { return (int)((l >> (5 * i)) & 31u); }
 HK_HD int getCount(const Env& e, int pid) { return (int)((e.pcount >> (2 * pid)) & 3u); }

@@ -93,6 +93,13 @@ class HockeyVecEnv:
     p2='per_env': every env has its own opponent code (`set_opponent_policies`), the batched form of drawing an
     opponent per episode from a pool (rl/training/opponent_manager.py:62-91); `step` then takes [N,8] actions whose
     columns 4..7 are only read by the envs whose code is 'external' (e.g. a self-play snapshot's output).
+
+    mode: one Mode (or name / int) for every env, or one per env (a sequence or a uint8 tensor [N]).  Per-env modes are
+    the batched form of the reference's `mode` setter: the handle is created, the modes are set as reset codes
+    (`set_reset_modes`) and every env is reset once with one_starting=True, so that this reset starts each env's
+    episode 1 (episode 0 is the creation's own reset, hockey_env.py:155).  Every later reset -- `reset` or an
+    auto-reset -- starts the next episode in the mode `reset_modes` holds for the env; `modes()` gives the mode each
+    env plays now.
     """
 
     def __init__(self, num_envs, mode=Mode.NORMAL, keep_mode=True, device="cuda:0", seed=0, env_id_offset=0,
@@ -104,6 +111,10 @@ class HockeyVecEnv:
         if self.device.type != "cuda":
             raise ValueError("HockeyVecEnv needs a CUDA device")
         self.num_envs = int(num_envs)
+        per_env_modes = None
+        if isinstance(mode, torch.Tensor) or (isinstance(mode, (list, tuple, np.ndarray)) and np.ndim(mode) == 1):
+            per_env_modes = mode
+            mode = Mode.NORMAL  # the creation mode: record word HK_S_MODE = 0 stands for it
         self._mode = _as_mode(mode)
         self.keep_mode = bool(keep_mode)
         self.auto_reset = bool(auto_reset)
@@ -112,8 +123,8 @@ class HockeyVecEnv:
         if self.p1 == _lib.POLICY_PER_ENV:
             raise ValueError("'per_env' is a player-2 policy")
         self.opponent_codes = None
+        self.reset_modes = None
         self.want_agent_two = bool(want_agent_two)
-        self.max_timesteps = 250 if self._mode == Mode.NORMAL else 80
         dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
         h = C.c_void_p()
         _lib.check(self.L.hk_create(C.byref(h), self.num_envs, self._mode.value, int(self.keep_mode), dev_index,
@@ -135,6 +146,10 @@ class HockeyVecEnv:
             _lib.check(self.L.hk_get_obs(self._h, _ptr(self.obs), _ptr(self.obs2), self._stream()))
         if self.p2 == _lib.POLICY_PER_ENV:
             self.set_opponent_policies(torch.full((n,), _lib.POLICY_BASIC_WEAK, dtype=torch.uint8, device=d))
+        self._modes = torch.empty(n, dtype=torch.uint8, device=d)
+        if per_env_modes is not None:
+            self.set_reset_modes(per_env_modes)
+            self.reset(one_starting=True)
 
     def set_opponent_policies(self, codes):
         """Per-env player-2 policy codes: uint8 CUDA tensor [N] of 0 external / 1 weak / 2 strong / 3 random / 4 zero
@@ -150,6 +165,41 @@ class HockeyVecEnv:
             _lib.check(self.L.hk_set_opponent_policies(self._h, _ptr(codes)))
         self.opponent_codes = codes
         return codes
+
+    def _mode_codes(self, modes, name):
+        """A scalar mode (Mode / name / int) broadcast to [N], or N of them, as a uint8 device tensor."""
+        if isinstance(modes, torch.Tensor):
+            return self._per_env(modes, torch.uint8, name)
+        if isinstance(modes, (list, tuple, np.ndarray)) and np.ndim(modes) == 1:
+            return self._per_env(np.array([_as_mode(m).value for m in modes], dtype=np.uint8), torch.uint8, name)
+        return self._per_env(_as_mode(modes).value, torch.uint8, name)
+
+    def set_reset_modes(self, modes):
+        """Mode of the episode every later reset of an env starts (explicit `reset` or auto-reset): one Mode for all,
+        a sequence of N, or a uint8 CUDA tensor [N] of 0 NORMAL / 1 TRAIN_SHOOTING / 2 TRAIN_DEFENSE.  The tensor is kept
+        as `env.reset_modes` and read by every reset; rewrite it in place (e.g. `env.reset_modes[done.bool()] = m`) to
+        move envs between modes per episode without a host round trip.  None clears it: every env keeps its mode."""
+        codes = None if modes is None else self._mode_codes(modes, "modes")
+        with torch.cuda.device(self.device):
+            torch.cuda.current_stream(self.device).synchronize()  # the library validates the codes on the default stream
+            _lib.check(self.L.hk_set_reset_modes(self._h, _ptr(codes)))
+        self.reset_modes = codes
+        return codes
+
+    def modes(self):
+        """uint8 [N] device tensor: the mode of each env's running episode (a persistent buffer, overwritten by the next
+        call; asynchronous like `step`)."""
+        with torch.cuda.device(self.device):
+            _lib.check(self.L.hk_get_modes(self._h, _ptr(self._modes), self._stream()))
+        return self._modes
+
+    @property
+    def max_timesteps(self):
+        """250 (NORMAL) or 80 while every env plays the constructor's mode; None once envs may play other modes
+        (reset codes are set): see `modes()`."""
+        if self.reset_modes is not None:
+            return None
+        return 250 if self._mode == Mode.NORMAL else 80
 
     # -- plumbing ---------------------------------------------------------------------------------
     def _stream(self):
@@ -168,7 +218,8 @@ class HockeyVecEnv:
 
     @property
     def mode(self):
-        return self._mode
+        """The constructor's mode while every env plays it; None once envs may play other modes (see `modes()`)."""
+        return None if self.reset_modes is not None else self._mode
 
     @property
     def action_dim(self):
@@ -192,15 +243,26 @@ class HockeyVecEnv:
             raise ValueError(f"{name} must be a scalar or have shape ({self.num_envs},), got {tuple(t.shape)}")
         return t.to(device=self.device, dtype=dtype).contiguous()
 
-    def reset(self, mask=None, one_starting=None, seed=None):
+    def reset(self, mask=None, one_starting=None, seed=None, mode=None):
         """HockeyEnv.reset (hockey_env.py:345-418) for the envs selected by `mask` (bool/uint8 [N], None = all).
         one_starting: None = alternate like the reference, a bool, or an int8 array/tensor [N] (1 / 0 / -1 = alternate).
         seed: None = every env continues its own random stream; an int s = env i is reset with seed s + i (the
         gymnasium vector convention); an int64 array/tensor [N] = one seed per env (negative = own stream).  A seeded
-        reset draws from that seed alone, like the reference's reseeding (hockey_env.py:347): same seed, same start."""
+        reset draws from that seed alone, like the reference's reseeding (hockey_env.py:347): same seed, same start.
+        mode: None = the mode `reset_modes` holds (or keep), a Mode for all or N of them = the reference's
+        reset(mode=...): the reset envs' codes in `reset_modes` are rewritten first, so that their later auto-resets
+        keep that mode too."""
         m = None
         if mask is not None:
             m = self._per_env(mask, torch.uint8, "mask")
+        if mode is not None:
+            codes = self._mode_codes(mode, "mode")
+            if self.reset_modes is None:
+                self.set_reset_modes(self.modes().clone())
+            if m is None:
+                self.reset_modes.copy_(codes)
+            else:
+                self.reset_modes.copy_(torch.where(m.bool(), codes, self.reset_modes))
         o = None
         if one_starting is not None:
             o = self._per_env(one_starting, torch.int8, "one_starting")
@@ -214,7 +276,7 @@ class HockeyVecEnv:
             _lib.check(self.L.hk_reset_seeded(self._h, _ptr(m), _ptr(o), _ptr(sd), None, self._stream()))
             _lib.check(self.L.hk_get_obs(self._h, _ptr(self.obs), _ptr(self.obs2), self._stream()))
             _lib.check(self.L.hk_get_info(self._h, _ptr(self.info), _ptr(self.info2), self._stream()))
-            if m is not None or o is not None or sd is not None:
+            if m is not None or o is not None or sd is not None or mode is not None:
                 torch.cuda.current_stream(self.device).synchronize()  # the argument tensors may be temporaries
         return self.obs, self._info_dict(self.info)
 
@@ -469,6 +531,7 @@ class HockeyEnv(_EnvBase):
         seed = int(np.random.SeedSequence().entropy % (1 << 63)) if seed is None else int(seed)
         self._vec = HockeyVecEnv(1, mode=self._mode, keep_mode=keep_mode, device=device, seed=seed, auto_reset=False,
                                  p2=_p2, want_agent_two=True)
+        self._vec_mode = self._mode  # the mode the library resets the env in
         self.max_timesteps = self._vec.max_timesteps
         self.time = 0
         self.one_starts = True
@@ -487,6 +550,7 @@ class HockeyEnv(_EnvBase):
 
     @mode.setter
     def mode(self, value):
+        """Takes effect at the next reset, as in the reference (reset reads it, hockey_env.py:357-364)."""
         self._mode = _as_mode(value)
 
     def seed(self, seed=None):
@@ -504,8 +568,12 @@ class HockeyEnv(_EnvBase):
                 "reward_puck_direction": float(v[3])}
 
     def reset(self, one_starting=None, mode=None, seed=None, options=None):
-        if mode is not None and _as_mode(mode) != self._mode:
-            raise ValueError("the mode of a HockeyEnv is fixed at construction in this implementation")
+        if mode is not None:
+            self.mode = mode
+        self.max_timesteps = 250 if self._mode == Mode.NORMAL else 80
+        new_mode = None
+        if self._mode != self._vec_mode:
+            new_mode = self._vec_mode = self._mode
         if self._mode == Mode.NORMAL:
             self.one_starts = bool(one_starting) if one_starting is not None else (not self.one_starts)
         if seed is not None:
@@ -513,7 +581,7 @@ class HockeyEnv(_EnvBase):
         pending = getattr(self, "_seed", None)
         self._seed = None
         self._vec.reset(one_starting=self.one_starts if self._mode == Mode.NORMAL else None,
-                        seed=None if pending is None else torch.tensor([pending], dtype=torch.int64))
+                        seed=None if pending is None else torch.tensor([pending], dtype=torch.int64), mode=new_mode)
         self.done = False
         self.winner = 0
         self.time = 0

@@ -6,6 +6,8 @@ The dense networks are plain torch modules (library matmuls): they are the ops n
 * `OpponentPool`        per-env opponent selection: weak / strong BasicOpponent (in-kernel) or self-play snapshots
                         (batched actor inference on obs_agent_two()), re-drawn per episode
                         (rl/training/opponent_manager.py:19-91, rl/training/self_play.py:7-68, hockey_env.py:908-922)
+* `ModeMix`             per-env game mode: NORMAL / TRAIN_SHOOTING / TRAIN_DEFENSE drawn per episode from probabilities
+                        that may change between calls (curriculum), with per-mode win / loss / draw counters on the device
 * `DeviceReplayBuffer`  ring buffer in HBM fed straight from step outputs (rl/replay/base_buffer.py:21-41,
                         rl/replay/uniform_buffer.py) -- `push` is one batched copy per tick instead of N Python calls
 * `evaluate`            the Evaluator protocol (rl/utils/evaluator.py:10-35): win / draw / loss rates and mean return
@@ -84,6 +86,72 @@ class OpponentPool:
         out = self.env.step(torch.cat([a1, self.opponent_actions()], dim=1).contiguous())
         self.resample(out[2])
         return out
+
+
+class ModeMix:
+    """Draws, per env and per episode, the game mode out of {NORMAL, TRAIN_SHOOTING, TRAIN_DEFENSE} with probabilities
+    `probs` (change them between calls with `set_probs`, e.g. to anneal a curriculum).  The draws go to the env's reset
+    codes (`HockeyVecEnv.set_reset_modes`), which the library reads AT each reset: each episode's mode is therefore
+    drawn one episode ahead -- when the previous episode of that env starts (or at construction) -- and an auto-reset
+    starts the episode in the mode drawn before it.  Call `update(done, winner)` after every step of the env (or use
+    `step`); it credits each finished episode to the mode it was played in and re-draws the codes of the envs that
+    just auto-reset.  Counters `counts` [3 modes, 4]: episodes, wins, losses, draws (float64, on the device: no host
+    sync per tick).  Explicit `env.reset` calls outside `reset` are not seen by the helper."""
+
+    EPISODES, WINS, LOSSES, DRAWS = 0, 1, 2, 3
+
+    def __init__(self, env, probs=(1 / 3, 1 / 3, 1 / 3), seed=0):
+        if not env.auto_reset:
+            raise ValueError("ModeMix needs HockeyVecEnv(..., auto_reset=True)")
+        self.env = env
+        self.gen = torch.Generator(device=env.device)
+        self.gen.manual_seed(seed)
+        self.set_probs(probs)
+        self.counts = torch.zeros((3, 4), dtype=torch.float64, device=env.device)
+        self.playing = env.modes().clone()  # mode of each env's running episode
+        self.codes = env.set_reset_modes(self._draw())  # mode of each env's next episode
+
+    def set_probs(self, probs):
+        """Probabilities of NORMAL, TRAIN_SHOOTING, TRAIN_DEFENSE for the draws from now on (normalised)."""
+        p = torch.as_tensor(probs, dtype=torch.float32).to(self.env.device).reshape(3)
+        if bool((p < 0).any()) or float(p.sum()) <= 0:
+            raise ValueError("probs must be three non-negative numbers with a positive sum")
+        self.probs = p / p.sum()
+
+    def _draw(self):
+        n = self.env.num_envs
+        return torch.multinomial(self.probs.expand(n, -1), 1, replacement=True, generator=self.gen).squeeze(1).to(torch.uint8)
+
+    def reset(self, **kwargs):
+        """env.reset(**kwargs) of every env (no mask): the episodes it starts play the drawn codes; draws the next ones."""
+        if "mask" in kwargs or "mode" in kwargs:
+            raise ValueError("ModeMix.reset resets every env in its drawn mode")
+        out = self.env.reset(**kwargs)
+        self.playing.copy_(self.codes)
+        self.codes.copy_(self._draw())
+        return out
+
+    def update(self, done, winner):
+        """After a step: credit the finished episodes (`done` [N], `winner` = info[:, 0]) to the mode they were played
+        in, then let the envs that auto-reset play their code and draw the code of their following episode."""
+        d = done.to(torch.bool)
+        w = winner.to(torch.float64)
+        rows = torch.stack([torch.ones_like(w), (w == 1).to(torch.float64), (w == -1).to(torch.float64),
+                            (w == 0).to(torch.float64)], 1) * d.unsqueeze(1).to(torch.float64)
+        self.counts.index_add_(0, self.playing.long(), rows)
+        self.playing.copy_(torch.where(d, self.codes, self.playing))
+        self.codes.copy_(torch.where(d, self._draw(), self.codes))  # in place: the library reads this very tensor
+
+    def step(self, action=None):
+        """One env tick followed by `update`; returns the env's step tuple."""
+        out = self.env.step(action)
+        self.update(out[2], out[4]["winner"])
+        return out
+
+    def stats(self):
+        """{mode name: {episodes, wins, losses, draws}} (synchronises the host)."""
+        c = self.counts.cpu().tolist()
+        return {m.name: dict(zip(("episodes", "wins", "losses", "draws"), c[m.value])) for m in Mode}
 
 
 class DeviceReplayBuffer:

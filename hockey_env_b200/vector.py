@@ -5,7 +5,8 @@ caller of the reference (hockey_env.py:875-903), as one batched env on the GPU:
 
   * `num_envs`, `single_observation_space`, `single_action_space`, batched `observation_space` / `action_space`;
   * `reset(seed=, options=) -> (obs, infos)`: seed = None / int (env i gets seed + i, gymnasium's convention) / list of
-    ints; options may hold "reset_mask" (bool [N], gymnasium >= 1.1) and "one_starting" (the reference's reset argument);
+    ints; options may hold "reset_mask" (bool [N], gymnasium >= 1.1), "one_starting" and "mode" (the reference's reset
+    arguments; "mode" is one Mode or one per env and also governs the later auto-resets of the reset envs);
   * `step(actions) -> (obs, rewards, terminations, truncations, infos)` with SAME-STEP auto-reset: the returned obs of a
     finished env is the first obs of its next episode, its terminal observation is infos["final_obs"][i] and its
     terminal info (winner, reward terms) infos["final_info"][key][i], selected by the boolean masks infos["_final_obs"]
@@ -38,7 +39,8 @@ class HockeyGymVectorEnv(_VectorEnvBase):
     spec = None
 
     def __init__(self, num_envs, mode=Mode.NORMAL, opponent="strong", device="cuda:0", seed=0, numpy_io=True, keep_mode=True):
-        """opponent: 'weak' / 'strong' (HockeyEnv_BasicOpponent semantic, 4-d actions) or None (HockeyEnv, 8-d actions)."""
+        """opponent: 'weak' / 'strong' (HockeyEnv_BasicOpponent semantic, 4-d actions) or None (HockeyEnv, 8-d actions).
+        mode: one Mode for all envs or one per env (HockeyVecEnv)."""
         self.env = HockeyVecEnv(num_envs, mode=mode, keep_mode=keep_mode, device=device, seed=seed, auto_reset=True, p2=opponent)
         self.num_envs = int(num_envs)
         self.numpy_io = bool(numpy_io)
@@ -72,7 +74,8 @@ class HockeyGymVectorEnv(_VectorEnvBase):
         options = options or {}
         if seed is not None and not isinstance(seed, (int, np.integer)):
             seed = np.asarray([-1 if s is None else int(s) for s in seed], dtype=np.int64)
-        obs, _ = self.env.reset(mask=options.get("reset_mask"), one_starting=options.get("one_starting"), seed=seed)
+        obs, _ = self.env.reset(mask=options.get("reset_mask"), one_starting=options.get("one_starting"), seed=seed,
+                                mode=options.get("mode"))
         return self._out(obs), self._infos()
 
     def step(self, actions):

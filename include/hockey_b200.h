@@ -83,6 +83,10 @@ enum {
   HK_S_TICK = 49,     /* u32 ticks executed since creation (RNG counter for per-tick draws) */
   HK_S_RET = 50,      /* 2 f64: running episode return of player 1 and player 2 (statistics only) */
   HK_S_PUCK_C0 = 54,  /* 2 f32: b2Sweep::c0 of the puck (only read if the puck is woken mid-step while asleep) */
+  HK_S_MODE = 56,     /* u32 mode of the running episode: 0 = the handle's creation mode (hk_create), m + 1 = mode m.
+                         hk_get_state writes 0 whenever the env plays the creation mode (so the records of single-mode
+                         handles do not depend on this word); hk_set_state reads 0 and any value above 3 as the creation
+                         mode.  Words 57-63 are unused (0). */
   HK_S_CONTACT = 64,  /* HK_N_PAIRS records of HK_CONTACT_WORDS words */
   HK_N_PAIRS = 27,
   HK_CONTACT_WORDS = 8,
@@ -147,6 +151,17 @@ int hk_step_host(hk_env* env, const float* action_host, int action_stride, int p
  * between steps, e.g. for the envs that just finished an episode).  EXTERNAL envs read columns 4..7 of action_dev
  * (a snapshot actor's output on obs_agent_two()); the others run their in-kernel controller.  NULL clears it. */
 int hk_set_opponent_policies(hk_env* env, const uint8_t* codes_dev);
+
+/* Per-env game mode (the reference's `mode` setter and reset(mode=...), hockey_env.py:345-364, 754-779: the mode of an
+ * env is read at each reset and sets the start layout, max_timesteps 250 / 80 and with it the reward scales).
+ * modes_dev: n_envs bytes of HK_MODE_NORMAL..HK_MODE_TRAIN_DEFENSE, caller-owned device memory that must stay valid while
+ * it is set.  Every later reset of an env -- hk_reset / hk_reset_seeded (masked) and the auto-reset of hk_step /
+ * hk_step_host / hk_rollout -- reads its byte and starts the next episode in that mode; the caller may rewrite it between
+ * calls (e.g. curriculum draws for the envs that just finished).  The contents are validated once, here.  NULL clears it:
+ * each env then keeps the mode it has (every env of a new handle plays the creation mode of hk_create). */
+int hk_set_reset_modes(hk_env* env, const uint8_t* modes_dev);
+/* The mode of each env's running episode: modes_dev [n] u8.  Asynchronous on `stream`; graph-capturable. */
+int hk_get_modes(hk_env* env, uint8_t* modes_dev, void* stream);
 
 /* k_steps ticks with in-kernel policies (no EXTERNAL), autoreset on, enqueued back to back without any
  * per-tick output: only the last tick's obs (nullable) is written; episode statistics accumulate in
