@@ -46,6 +46,22 @@ def load_td3_actor(path, device="cuda:0", name=None):
     return actor.to(device).eval()
 
 
+def _cuda_device(device, who):
+    from . import _lib
+    device = torch.device(device)
+    if device.type != "cuda" or not torch.cuda.is_available():
+        raise _lib.HockeyLibraryError(f"{who} needs a CUDA device: the actor kernel has no CPU fallback")
+    return device
+
+
+def _reference_state_dict(actor, who):
+    """The fp32 CPU state dict of an ActorNetwork-shaped module, checked against the reference architecture."""
+    sd = {k: v.detach().to("cpu", torch.float32) for k, v in actor.state_dict().items()}
+    if tuple(sd["fc1.weight"].shape) != (256, 18) or tuple(sd["fc2.weight"].shape) != (256, 256) or tuple(sd["fc3.weight"].shape) != (4, 256):
+        raise ValueError(f"{who} implements the reference architecture 18 -> 256 -> 256 -> 4")
+    return sd
+
+
 class FusedActor:
     """The same network as ONE fused sm_100a tensor-core kernel (csrc/hk_actor.cuh, hk_actor_forward): weights resident in
     shared memory (layer 1 TF32, layers 2-3 bf16), fp32 accumulation in tensor memory, hidden activations never leave the SM.  Callable like the
@@ -53,18 +69,15 @@ class FusedActor:
     pass `out=` to write into columns 0..3 of an existing [N,4] / [N,8] action tensor).  There is no fallback: without the
     CUDA library or a GPU this raises."""
 
+    PARAM_BYTES = 256 * 24 * 4 + 256 * 256 * 2 + 16 * 256 * 2 + 2 * 256 * 4 + 16 * 4  # hk_actor_param_bytes()
+
     def __init__(self, actor, device="cuda:0"):
         import ctypes as C
         from . import _lib
         self._C, self._lib = C, _lib
         self.L = _lib.load()
-        self.device = torch.device(device)
-        if self.device.type != "cuda" or not torch.cuda.is_available():
-            raise _lib.HockeyLibraryError("FusedActor needs a CUDA device: the actor kernel has no CPU fallback")
-        sd = {k: v.detach().to("cpu", torch.float32) for k, v in actor.state_dict().items()}
-        if tuple(sd["fc1.weight"].shape) != (256, 18) or tuple(sd["fc2.weight"].shape) != (256, 256) or tuple(sd["fc3.weight"].shape) != (4, 256):
-            raise ValueError("FusedActor implements the reference architecture 18 -> 256 -> 256 -> 4")
-        self.params = self.pack(sd).to(self.device)
+        self.device = _cuda_device(device, "FusedActor")
+        self.params = self.pack(_reference_state_dict(actor, "FusedActor")).to(self.device)
         assert self.params.numel() == int(self.L.hk_actor_param_bytes())
         self._out = None
 
@@ -104,6 +117,83 @@ class FusedActor:
             self._lib.check(self.L.hk_actor_forward(C.c_void_p(self.params.data_ptr()), C.c_void_p(obs.data_ptr()),
                                                     C.c_void_p(out.data_ptr()), int(out.stride(0)), n, obs.device.index or 0,
                                                     C.c_void_p(torch.cuda.current_stream(obs.device).cuda_stream)))
+        return out[:, :4] if out.shape[1] != 4 else out
+
+
+class FusedActorPool:
+    """K frozen actors (self-play snapshots, a league) evaluated per row in ONE tensor-core pass
+    (csrc/hk_actor.cuh k_actor_pool_mlp, hk_actor_forward_pool): row i goes through snapshot choice[i].  The rows are
+    grouped by snapshot on the device (no host sync; graph-capturable), and each written row equals
+    `FusedActor(snapshot choice[i])(obs)[i]` bit for bit.  The table is one [K, hk_actor_param_bytes()] uint8 device
+    tensor of `FusedActor.pack` blocks; `add` appends one (and re-allocates the table: re-capture graphs after it).
+    There is no fallback: without the CUDA library or a GPU this raises."""
+
+    MAX_K = 4096
+
+    def __init__(self, actors=(), device="cuda:0"):
+        import ctypes as C
+        from . import _lib
+        self._C, self._lib = C, _lib
+        self.L = _lib.load()
+        self.device = _cuda_device(device, "FusedActorPool")
+        self.table = self.pack(actors).to(self.device)
+        self._out = None
+        self._scratch = torch.empty(0, dtype=torch.uint8, device=self.device)
+
+    @staticmethod
+    def pack(actors):
+        """[K, param_bytes] uint8 (CPU): block s is `FusedActor.pack` of actors[s], at byte offset s * param_bytes of
+        the flattened table."""
+        blocks = [FusedActor.pack(_reference_state_dict(a, "FusedActorPool")) for a in actors]
+        return torch.stack(blocks) if blocks else torch.empty((0, FusedActor.PARAM_BYTES), dtype=torch.uint8)
+
+    def __len__(self):
+        return self.table.shape[0]
+
+    def add(self, actor):
+        """Append one snapshot; returns its index (the choice value that selects it)."""
+        if len(self) >= self.MAX_K:
+            raise ValueError(f"FusedActorPool holds at most {self.MAX_K} snapshots")
+        blk = self.pack([actor]).to(self.device)
+        self.table = torch.cat([self.table, blk])
+        return len(self) - 1
+
+    def __call__(self, obs, choice, out=None):
+        """obs [N,18] float32 CUDA, choice int32 / int64 CUDA [N] -> act[i] = actor_{choice[i]}(obs[i]) for choice[i] in
+        [0, K); other rows are not written.  out=None: a persistent [N,4] buffer (overwritten by the next call) whose
+        skipped rows are 0; or pass `out` = an [N, >= 4] float32 view with unit column stride (e.g. `a8[:, 4:]` of the
+        [N,8] action tensor): columns 0..3 of its written rows change, nothing else."""
+        if not (obs.is_cuda and obs.dtype == torch.float32 and obs.is_contiguous() and obs.dim() == 2 and obs.shape[1] == 18):
+            raise ValueError("FusedActorPool expects a contiguous float32 CUDA tensor [N, 18]")
+        n, k = obs.shape[0], len(self)
+        if k == 0:
+            raise ValueError("FusedActorPool is empty: add() a snapshot first")
+        if not (isinstance(choice, torch.Tensor) and choice.is_cuda and choice.dtype in (torch.int32, torch.int64)
+                and choice.shape == (n,) and choice.device == obs.device == self.table.device):
+            raise ValueError("choice must be an int32 or int64 CUDA tensor [N], on the pool's device like obs")
+        if choice.dtype == torch.int64:  # out-of-range values stay out of range after the narrowing
+            choice = torch.where((choice >= 0) & (choice < k), choice, -1).to(torch.int32)
+        choice = choice.contiguous()
+        if out is None:
+            if self._out is None or self._out.shape[0] != n or self._out.device != obs.device:
+                self._out = torch.empty((n, 4), dtype=torch.float32, device=obs.device)
+            out = self._out
+            out.zero_()
+        if not (out.is_cuda and out.dtype == torch.float32 and out.dim() == 2 and out.shape[0] == n and out.stride(1) == 1 and out.shape[1] >= 4):
+            raise ValueError("out must be a float32 CUDA tensor [N, >= 4] with unit column stride")
+        if n == 0:
+            return out[:, :4]
+        need = int(self.L.hk_actor_pool_scratch_bytes(n, k))
+        if need < 0:
+            self._lib.check(need)
+        if self._scratch.numel() < need:
+            self._scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
+        C = self._C
+        with torch.cuda.device(obs.device):
+            self._lib.check(self.L.hk_actor_forward_pool(C.c_void_p(self.table.data_ptr()), k, C.c_void_p(choice.data_ptr()),
+                                                         C.c_void_p(obs.data_ptr()), C.c_void_p(out.data_ptr()), int(out.stride(0)),
+                                                         n, C.c_void_p(self._scratch.data_ptr()), obs.device.index or 0,
+                                                         C.c_void_p(torch.cuda.current_stream(obs.device).cuda_stream)))
         return out[:, :4] if out.shape[1] != 4 else out
 
 

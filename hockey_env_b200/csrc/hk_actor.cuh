@@ -132,119 +132,309 @@ __device__ __forceinline__ void hiddenEpilogue(uint32_t taddr, const float* bias
   }
 }
 
-__global__ void __launch_bounds__(kThreads, 1) k_actor_mlp(const unsigned char* __restrict__ params, const float* __restrict__ obs,
-                                                           float* __restrict__ act, int actStride, long long n) {
-  extern __shared__ __align__(128) unsigned char smem[];
+// Per-CTA state of the tile loop: the TMEM accumulator base, this warp's lanes of it, the mbarrier the MMAs commit to and
+// the shared-memory addresses of the operands.
+struct TileCtx {
+  unsigned char* smem;
+  uint32_t tmem, myT, barA, sW1, sW2, sW3, sX, sAa;
+};
+
+// the parameter block (global, L2-resident after the first CTA) -> shared memory.  The tile body's
+// `fence.proxy.async.shared::cta`, executed by every thread after these writes, makes them visible to the tensor core.
+__device__ __forceinline__ void loadParams(unsigned char* smem, const unsigned char* __restrict__ params) {
+  for (int k = threadIdx.x; k < kParamBytes / 16; k += kThreads)
+    reinterpret_cast<uint4*>(smem)[k] = reinterpret_cast<const uint4*>(params)[k];
+}
+
+// mbarrier init and the 512-column TMEM allocation (one warp: layer-1 accumulator [0,256), layer-2 [256,512), layer-3
+// [0,16)); ends in a block barrier.  Free the columns with `actorTeardown`.
+__device__ __forceinline__ TileCtx actorSetup(unsigned char* smem) {
   const int t = threadIdx.x, warp = t >> 5;
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem + kOffBar);
   uint32_t* tmemSlot = reinterpret_cast<uint32_t*>(smem + kOffBar + 8);
-  // parameters: global (L2-resident after the first CTA) -> shared, once per CTA
-  for (int k = t; k < kParamBytes / 16; k += kThreads)
-    reinterpret_cast<uint4*>(smem)[k] = reinterpret_cast<const uint4*>(params)[k];
   if (t == 0) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smemAddr(bar)));
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (warp == 0) {  // one warp allocates all 512 TMEM columns: layer-1 accumulator [0,256), layer-2 [256,512), layer-3 [0,16)
+  if (warp == 0) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smemAddr(tmemSlot)), "r"(512));
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem = *tmemSlot;
-  const uint32_t myT = tmem + ((uint32_t)(warp * 32) << 16);  // this warp's 32 TMEM lanes
-  const uint32_t barA = smemAddr(bar);
-  const uint32_t sW1 = smemAddr(smem + kOffW1), sW2 = smemAddr(smem + kOffW2), sW3 = smemAddr(smem + kOffW3);
-  const uint32_t sX = smemAddr(smem + kOffX), sAa = smemAddr(smem + kOffA);
+  TileCtx c;
+  c.smem = smem;
+  c.tmem = *tmemSlot;
+  c.myT = c.tmem + ((uint32_t)(warp * 32) << 16);  // this warp's 32 TMEM lanes
+  c.barA = smemAddr(bar);
+  c.sW1 = smemAddr(smem + kOffW1);
+  c.sW2 = smemAddr(smem + kOffW2);
+  c.sW3 = smemAddr(smem + kOffW3);
+  c.sX = smemAddr(smem + kOffX);
+  c.sAa = smemAddr(smem + kOffA);
+  return c;
+}
+
+__device__ __forceinline__ void actorTeardown(const TileCtx& c) {
+  if ((threadIdx.x >> 5) == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(c.tmem), "r"(512));
+}
+
+// One tile of 128 rows through the three layers with the weights now in shared memory.  Thread t owns TMEM lane t; `row`
+// is the observation / action row it reads and writes, or -1 for a padding lane (zero input, nothing stored).  The only
+// thing the callers differ in is how a thread finds its row.  Ends in a block barrier: on return every MMA of the tile
+// has completed and every thread is done with the tile's shared memory (the weights may be replaced).
+__device__ __forceinline__ void actorTile(const TileCtx& c, uint32_t& phase, const float* __restrict__ obs,
+                                          float* __restrict__ act, int actStride, long long row) {
+  const int t = threadIdx.x;
+  unsigned char* smem = c.smem;
+  const uint32_t tmem = c.tmem, myT = c.myT, barA = c.barA;
   const float* b1 = reinterpret_cast<const float*>(smem + kOffB1);
   const float* b2 = reinterpret_cast<const float*>(smem + kOffB2);
   const float* b3 = reinterpret_cast<const float*>(smem + kOffB3);
   unsigned char* sA = smem + kOffA;
+  // ---- this thread's observation row -> tf32 -> layer-1 A operand (K padded 18 -> 24 with zeros) ----
+  float o[kK1];
+#pragma unroll
+  for (int k = 0; k < kK1; ++k) o[k] = 0.0f;
+  if (row >= 0) {
+    const float2* src = reinterpret_cast<const float2*>(obs + row * kObs);
+#pragma unroll
+    for (int k = 0; k < kObs / 2; ++k) {
+      const float2 v = src[k];
+      o[2 * k] = v.x;
+      o[2 * k + 1] = v.y;
+    }
+  }
+#pragma unroll
+  for (int q = 0; q < kK1 / 4; ++q)  // 16-byte K chunks of four tf32 values: chunk q at q * (kRows * 16) bytes, row t at + t * 16
+    *reinterpret_cast<uint4*>(smem + kOffX + q * (kRows * 16) + t * 16) =
+        make_uint4(toTf32(o[4 * q]), toTf32(o[4 * q + 1]), toTf32(o[4 * q + 2]), toTf32(o[4 * q + 3]));
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy smem writes -> visible to the tensor core
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  // ---- layer 1 (TF32): D1[128 x 256] = X[128 x 24] W1^T ----
+  if (t == 0) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+#pragma unroll
+    for (int ks = 0; ks < kK1 / 8; ++ks)
+      ummaTf32(tmem, umaDesc(c.sX + ks * 2 * (kRows * 16), kRows * 16, 128), umaDesc(c.sW1 + ks * 2 * (kHidden * 16), kHidden * 16, 128),
+               instrDesc(kRows, kHidden, 2), ks > 0);
+    ummaCommit(barA);
+  }
+  mbarWait(barA, phase);
+  phase ^= 1;
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  hiddenEpilogue(myT, b1, sA);
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  // ---- layer 2: D2[128 x 256] = H1[128 x 256] W2^T ----
+  if (t == 0) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+#pragma unroll
+    for (int ks = 0; ks < kHidden / 16; ++ks)
+      umma(tmem + kHidden, umaDesc(c.sAa + ks * 2 * (kRows * 16), kRows * 16, 128),
+           umaDesc(c.sW2 + ks * 2 * (kHidden * 16), kHidden * 16, 128), instrDesc(kRows, kHidden, 1), ks > 0);
+    ummaCommit(barA);
+  }
+  mbarWait(barA, phase);
+  phase ^= 1;
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  hiddenEpilogue(myT + kHidden, b2, sA);  // layer 2 has finished reading H1: its buffer takes H2
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  // ---- layer 3: D3[128 x 16] = H2[128 x 256] W3^T (4 real outputs) ----
+  if (t == 0) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+#pragma unroll
+    for (int ks = 0; ks < kHidden / 16; ++ks)
+      umma(tmem, umaDesc(c.sAa + ks * 2 * (kRows * 16), kRows * 16, 128), umaDesc(c.sW3 + ks * 2 * (kN3 * 16), kN3 * 16, 128),
+           instrDesc(kRows, kN3, 1), ks > 0);
+    ummaCommit(barA);
+  }
+  mbarWait(barA, phase);
+  phase ^= 1;
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  {
+    uint32_t r0, r1, r2, r3;
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(myT));
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+    if (row >= 0) {
+      float* dst = act + row * actStride;
+      dst[0] = tanhApprox(__uint_as_float(r0) + b3[0]);
+      dst[1] = tanhApprox(__uint_as_float(r1) + b3[1]);
+      dst[2] = tanhApprox(__uint_as_float(r2) + b3[2]);
+      dst[3] = tanhApprox(__uint_as_float(r3) + b3[3]);
+    }
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();  // the next tile's layer 1 overwrites the columns layer 3 was just read from
+}
+
+// one weight set, rows 0..n-1 in order: tile `tile` holds rows tile * 128 + t
+__global__ void __launch_bounds__(kThreads, 1) k_actor_mlp(const unsigned char* __restrict__ params, const float* __restrict__ obs,
+                                                           float* __restrict__ act, int actStride, long long n) {
+  extern __shared__ __align__(128) unsigned char smem[];
+  loadParams(smem, params);  // once per CTA
+  const TileCtx c = actorSetup(smem);
   uint32_t phase = 0;
   const long long tiles = (n + kRows - 1) / kRows;
   for (long long tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-    const long long row = tile * kRows + t;
-    // ---- this thread's observation row -> tf32 -> layer-1 A operand (K padded 18 -> 24 with zeros) ----
-    float o[kK1];
-#pragma unroll
-    for (int k = 0; k < kK1; ++k) o[k] = 0.0f;
-    if (row < n) {
-      const float2* src = reinterpret_cast<const float2*>(obs + row * kObs);
-#pragma unroll
-      for (int k = 0; k < kObs / 2; ++k) {
-        const float2 v = src[k];
-        o[2 * k] = v.x;
-        o[2 * k + 1] = v.y;
-      }
-    }
-#pragma unroll
-    for (int q = 0; q < kK1 / 4; ++q)  // 16-byte K chunks of four tf32 values: chunk q at q * (kRows * 16) bytes, row t at + t * 16
-      *reinterpret_cast<uint4*>(smem + kOffX + q * (kRows * 16) + t * 16) =
-          make_uint4(toTf32(o[4 * q]), toTf32(o[4 * q + 1]), toTf32(o[4 * q + 2]), toTf32(o[4 * q + 3]));
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy smem writes -> visible to the tensor core
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    // ---- layer 1 (TF32): D1[128 x 256] = X[128 x 24] W1^T ----
-    if (t == 0) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-      for (int ks = 0; ks < kK1 / 8; ++ks)
-        ummaTf32(tmem, umaDesc(sX + ks * 2 * (kRows * 16), kRows * 16, 128), umaDesc(sW1 + ks * 2 * (kHidden * 16), kHidden * 16, 128),
-                 instrDesc(kRows, kHidden, 2), ks > 0);
-      ummaCommit(barA);
-    }
-    mbarWait(barA, phase);
-    phase ^= 1;
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    hiddenEpilogue(myT, b1, sA);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    // ---- layer 2: D2[128 x 256] = H1[128 x 256] W2^T ----
-    if (t == 0) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-      for (int ks = 0; ks < kHidden / 16; ++ks)
-        umma(tmem + kHidden, umaDesc(sAa + ks * 2 * (kRows * 16), kRows * 16, 128),
-             umaDesc(sW2 + ks * 2 * (kHidden * 16), kHidden * 16, 128), instrDesc(kRows, kHidden, 1), ks > 0);
-      ummaCommit(barA);
-    }
-    mbarWait(barA, phase);
-    phase ^= 1;
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    hiddenEpilogue(myT + kHidden, b2, sA);  // layer 2 has finished reading H1: its buffer takes H2
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    // ---- layer 3: D3[128 x 16] = H2[128 x 256] W3^T (4 real outputs) ----
-    if (t == 0) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-      for (int ks = 0; ks < kHidden / 16; ++ks)
-        umma(tmem, umaDesc(sAa + ks * 2 * (kRows * 16), kRows * 16, 128), umaDesc(sW3 + ks * 2 * (kN3 * 16), kN3 * 16, 128),
-             instrDesc(kRows, kN3, 1), ks > 0);
-      ummaCommit(barA);
-    }
-    mbarWait(barA, phase);
-    phase ^= 1;
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    {
-      uint32_t r0, r1, r2, r3;
-      asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(myT));
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      if (row < n) {
-        float* dst = act + row * actStride;
-        dst[0] = tanhApprox(__uint_as_float(r0) + b3[0]);
-        dst[1] = tanhApprox(__uint_as_float(r1) + b3[1]);
-        dst[2] = tanhApprox(__uint_as_float(r2) + b3[2]);
-        dst[3] = tanhApprox(__uint_as_float(r3) + b3[3]);
-      }
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();  // the next tile's layer 1 overwrites the columns layer 3 was just read from
+    const long long row = tile * kRows + threadIdx.x;
+    actorTile(c, phase, obs, act, actStride, row < n ? row : -1);
   }
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
+  actorTeardown(c);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Snapshot pool: act[i] = actor_{choice[i]}(obs[i]) for K weight sets laid out back to back (K blocks of kParamBytes),
+// rows with choice[i] outside [0, K) untouched.  Rows are grouped by snapshot on the device, with no host sync:
+//   cudaMemsetAsync(counts) -> k_pool_count (histogram) -> k_pool_scan (group and tile offsets, one block)
+//   -> k_pool_scatter (row lists) -> k_actor_pool_mlp (persistent, tiles of one group share one weight set).
+// Scratch layout (int32 words, caller-owned, poolScratchWords(n, K) of them):
+//   counts[K] | groupOff[K + 1] | tileOff[K + 1] | cursor[K] | rows[n]
+// groupOff[s] is where group s starts in rows[], tileOff[s] its first tile; tileOff[K] is the total tile count.
+constexpr int kPoolMaxK = 4096;
+constexpr int kPoolThreads = 256;        // count / scatter blocks
+constexpr int kPoolItems = 8;            // rows per thread of one scatter block
+constexpr int kScanThreads = 1024;
+
+__host__ __device__ constexpr long long poolAlign4(long long words) { return (words + 3) & ~3LL; }  // 16-byte sections
+__host__ __device__ inline long long poolOffGroup(int k) { return poolAlign4(k); }
+__host__ __device__ inline long long poolOffTile(int k) { return poolOffGroup(k) + poolAlign4(k + 1); }
+__host__ __device__ inline long long poolOffCursor(int k) { return poolOffTile(k) + poolAlign4(k + 1); }
+__host__ __device__ inline long long poolOffRows(int k) { return poolOffCursor(k) + poolAlign4(k); }
+__host__ __device__ inline long long poolScratchWords(long long n, int k) { return poolOffRows(k) + poolAlign4(n); }
+
+// histogram of the valid choices: per-block counts in shared memory, then one global add per non-empty bin
+__global__ void __launch_bounds__(kPoolThreads) k_pool_count(const int32_t* __restrict__ choice, long long n, int k,
+                                                             int32_t* __restrict__ counts) {
+  extern __shared__ int32_t hist[];
+  for (int s = threadIdx.x; s < k; s += blockDim.x) hist[s] = 0;
+  __syncthreads();
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const int c = choice[i];
+    if (c >= 0 && c < k) atomicAdd(&hist[c], 1);
+  }
+  __syncthreads();
+  for (int s = threadIdx.x; s < k; s += blockDim.x)
+    if (hist[s]) atomicAdd(&counts[s], hist[s]);
+}
+
+// exclusive scans of the row counts and of the tile counts ceil(count / 128), one block; cursor[s] = groupOff[s]
+__global__ void __launch_bounds__(kScanThreads) k_pool_scan(int32_t* __restrict__ scratch, int k) {
+  __shared__ int2 warpSum[kScanThreads / 32];
+  const int32_t* counts = scratch;
+  int32_t* groupOff = scratch + poolOffGroup(k);
+  int32_t* tileOff = scratch + poolOffTile(k);
+  int32_t* cursor = scratch + poolOffCursor(k);
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const int per = (k + kScanThreads - 1) / kScanThreads;  // consecutive bins of this thread
+  const int s0 = min(t * per, k), s1 = min(s0 + per, k);
+  int2 mine = make_int2(0, 0);
+  for (int s = s0; s < s1; ++s) {
+    mine.x += counts[s];
+    mine.y += (counts[s] + kRows - 1) / kRows;
+  }
+  int2 inc = mine;  // inclusive scan over the warp, then over the warp totals
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const int x = __shfl_up_sync(0xffffffffu, inc.x, d), y = __shfl_up_sync(0xffffffffu, inc.y, d);
+    if (lane >= d) inc.x += x, inc.y += y;
+  }
+  if (lane == 31) warpSum[warp] = inc;
+  __syncthreads();
+  if (warp == 0) {
+    int2 w = warpSum[lane];
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const int x = __shfl_up_sync(0xffffffffu, w.x, d), y = __shfl_up_sync(0xffffffffu, w.y, d);
+      if (lane >= d) w.x += x, w.y += y;
+    }
+    warpSum[lane] = w;
+  }
+  __syncthreads();
+  int2 run = make_int2(inc.x - mine.x, inc.y - mine.y);
+  if (warp > 0) run.x += warpSum[warp - 1].x, run.y += warpSum[warp - 1].y;
+  for (int s = s0; s < s1; ++s) {
+    groupOff[s] = run.x;
+    cursor[s] = run.x;
+    tileOff[s] = run.y;
+    run.x += counts[s];
+    run.y += (counts[s] + kRows - 1) / kRows;
+  }
+  if (t == kScanThreads - 1) {
+    groupOff[k] = run.x;
+    tileOff[k] = run.y;
+  }
+}
+
+// row lists: a block takes kPoolThreads * kPoolItems consecutive rows, ranks them per group in shared memory, reserves
+// one range per non-empty group with a single atomic on that group's cursor and writes the row indices there
+__global__ void __launch_bounds__(kPoolThreads) k_pool_scatter(const int32_t* __restrict__ choice, long long n, int k,
+                                                               int32_t* __restrict__ scratch) {
+  extern __shared__ int32_t sh[];  // hist[k] | base[k]
+  int32_t* hist = sh;
+  int32_t* base = sh + k;
+  int32_t* cursor = scratch + poolOffCursor(k);
+  int32_t* rows = scratch + poolOffRows(k);
+  for (long long first = blockIdx.x * (long long)(kPoolThreads * kPoolItems); first < n;
+       first += (long long)gridDim.x * (kPoolThreads * kPoolItems)) {
+    for (int s = threadIdx.x; s < k; s += blockDim.x) hist[s] = 0;
+    __syncthreads();
+    int c[kPoolItems], rank[kPoolItems];
+#pragma unroll
+    for (int j = 0; j < kPoolItems; ++j) {
+      const long long i = first + j * kPoolThreads + threadIdx.x;
+      c[j] = i < n ? choice[i] : -1;
+      rank[j] = (c[j] >= 0 && c[j] < k) ? atomicAdd(&hist[c[j]], 1) : -1;
+    }
+    __syncthreads();
+    for (int s = threadIdx.x; s < k; s += blockDim.x)
+      if (hist[s]) base[s] = atomicAdd(&cursor[s], hist[s]);
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < kPoolItems; ++j)
+      if (rank[j] >= 0) rows[base[c[j]] + rank[j]] = (int32_t)(first + j * kPoolThreads + threadIdx.x);
+    __syncthreads();  // hist / base are reused by the next chunk
+  }
+}
+
+// Persistent: CTA b walks the contiguous tile range [b T / G, (b + 1) T / G) of the T = tileOff[K] tiles, so it crosses few
+// group boundaries; it copies a snapshot's weights into shared memory only when the group changes.  Tile j of group s holds
+// rows[groupOff[s] + j * 128 + t]; lanes past the group's end are padding.
+__global__ void __launch_bounds__(kThreads, 1) k_actor_pool_mlp(const unsigned char* __restrict__ params, int k,
+                                                                const int32_t* __restrict__ scratch, const float* __restrict__ obs,
+                                                                float* __restrict__ act, int actStride) {
+  extern __shared__ __align__(128) unsigned char smem[];
+  const int32_t* groupOff = scratch + poolOffGroup(k);
+  const int32_t* tileOff = scratch + poolOffTile(k);
+  const int32_t* rows = scratch + poolOffRows(k);
+  const long long total = tileOff[k];
+  const long long t0 = total * blockIdx.x / gridDim.x, t1 = total * (blockIdx.x + 1) / gridDim.x;
+  if (t0 >= t1) return;  // nothing to do: no TMEM allocated, no barrier entered
+  const TileCtx c = actorSetup(smem);
+  int lo = 0, hi = k - 1;  // the group of tile t0: the last s with tileOff[s] <= t0 (empty groups share their offset)
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (tileOff[mid] <= t0) lo = mid; else hi = mid - 1;
+  }
+  int s = lo, loaded = -1;
+  uint32_t phase = 0;
+  for (long long tile = t0; tile < t1; ++tile) {
+    while (tile >= tileOff[s + 1]) ++s;
+    if (s != loaded) {
+      // the previous tile (if any) ended with its layer-3 MMAs complete and a block barrier: the old weights are dead
+      loadParams(smem, params + (size_t)s * kParamBytes);
+      loaded = s;
+    }
+    const int local = (int)(tile - tileOff[s]) * kRows + threadIdx.x;
+    const int count = groupOff[s + 1] - groupOff[s];
+    actorTile(c, phase, obs, act, actStride, local < count ? (long long)rows[groupOff[s] + local] : -1LL);
+  }
+  actorTeardown(c);
 }
 
 }  // namespace hk_actor

@@ -1966,6 +1966,47 @@ int hk_actor_forward(const void* params_dev, const float* obs_dev, float* act_de
   return HK_OK;
 }
 
+int64_t hk_actor_pool_scratch_bytes(int64_t n, int k) {
+  if (n <= 0 || n > INT32_MAX || k < 1 || k > hk_actor::kPoolMaxK)
+    return fail(HK_E_INVALID, "hk_actor_pool_scratch_bytes: n must be in [1, 2^31 - 1] and k in [1, 4096]");
+  return 4 * hk_actor::poolScratchWords(n, k);
+}
+
+int hk_actor_forward_pool(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev,
+                          int act_stride, int64_t n, void* scratch_dev, int device, void* stream) {
+  using namespace hk_actor;
+  if (!params_dev || !choice_dev || !obs_dev || !act_dev || !scratch_dev) return fail(HK_E_INVALID, "hk_actor_forward_pool: NULL argument");
+  if (n <= 0 || n > INT32_MAX || act_stride < kAct)
+    return fail(HK_E_INVALID, "hk_actor_forward_pool: n must be in [1, 2^31 - 1] and act_stride >= 4");
+  if (k < 1 || k > kPoolMaxK) return fail(HK_E_INVALID, "hk_actor_forward_pool: k must be in [1, 4096]");
+  if ((((uintptr_t)params_dev) & 15u) || (((uintptr_t)obs_dev) & 7u) || (((uintptr_t)choice_dev) & 3u) || (((uintptr_t)scratch_dev) & 15u))
+    return fail(HK_E_INVALID, "hk_actor_forward_pool: params and scratch need 16-byte, obs 8-byte, choice 4-byte alignment");
+  int count = 0;
+  if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) return fail(HK_E_NODEVICE, "hk_actor_forward_pool: no CUDA device (there is no CPU fallback)");
+  if (device < 0 || device >= count) return fail(HK_E_INVALID, "hk_actor_forward_pool: bad device index");
+  DeviceGuard guard(device);
+  static bool configured[64] = {false};
+  if (!configured[device & 63]) {
+    HK_CUDA(cudaFuncSetAttribute(k_actor_pool_mlp, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    configured[device & 63] = true;
+  }
+  int sms = 148;
+  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sms < 1) sms = 148;
+  cudaStream_t st = (cudaStream_t)stream;
+  int32_t* scratch = (int32_t*)scratch_dev;
+  HK_CUDA(cudaMemsetAsync(scratch, 0, sizeof(int32_t) * (size_t)k, st));  // counts
+  const int64_t chunks = (n + kPoolThreads * kPoolItems - 1) / (kPoolThreads * kPoolItems);
+  const unsigned histBlocks = (unsigned)std::min<int64_t>(chunks, 4 * (int64_t)sms);
+  k_pool_count<<<histBlocks, kPoolThreads, sizeof(int32_t) * (size_t)k, st>>>(choice_dev, (long long)n, k, scratch);
+  k_pool_scan<<<1, kScanThreads, 0, st>>>(scratch, k);
+  k_pool_scatter<<<histBlocks, kPoolThreads, 2 * sizeof(int32_t) * (size_t)k, st>>>(choice_dev, (long long)n, k, scratch);
+  // the tile count is only known on the device: at most ceil(n / 128) + k - 1 tiles (one partial tile per group)
+  const int64_t grid = std::min<int64_t>(sms, (n + kRows - 1) / kRows + k);
+  k_actor_pool_mlp<<<(unsigned)grid, kThreads, kSmemBytes, st>>>((const unsigned char*)params_dev, k, scratch, obs_dev, act_dev, act_stride);
+  HK_CUDA(cudaGetLastError());
+  return HK_OK;
+}
+
 int hk_launches_per_step(const hk_env* h) { return h ? h->launches : 0; }
 
 int hk_kernel_timing(hk_env* h, int enable) {

@@ -12,20 +12,25 @@ The dense networks are plain torch modules (library matmuls): they are the ops n
                         rl/replay/uniform_buffer.py) -- `push` is one batched copy per tick instead of N Python calls
 * `evaluate`            the Evaluator protocol (rl/utils/evaluator.py:10-35): win / draw / loss rates and mean return
                         of a policy against a fixed opponent over n COMPLETE episodes (fixed quota per env)
+* `cross_play`          league table: K actors against each other (K x K ordered pairs) in one batch, one pooled
+                        tensor-core launch per player per tick, with `evaluate`'s complete-episode protocol
 * `evaluate_model`      the ModelEvaluator protocol (model_evaluation/model_evaluator.py:81-108): 300 episodes, seed
                         123, against the weak and the strong BasicOpponent
 """
 import torch
 
 from . import _lib
+from .actor import FusedActorPool
 from .env import HockeyVecEnv, Mode
 
 
 class OpponentPool:
     """Draws, per env and per episode, one opponent out of {weak, strong, snapshot_0..k-1} with the given
     probabilities (the reference draws one per episode for its single env; here every env of the batch holds its own
-    draw).  BasicOpponents run inside the step kernel; snapshot opponents are torch modules evaluated on
-    `obs_agent_two()` for all envs at once, their actions are only read by the envs that drew them."""
+    draw).  BasicOpponents run inside the step kernel.  Snapshot opponents are either a list of modules (each evaluated
+    on `obs_agent_two()` for all envs at once; their actions are only read by the envs that drew them) or a
+    `FusedActorPool`: then one pooled tensor-core launch evaluates, per env, only the snapshot it drew, straight into
+    columns 4..7 of a persistent [N, 8] action buffer."""
 
     WEAK, STRONG, SNAPSHOT0 = 0, 1, 2
 
@@ -33,7 +38,8 @@ class OpponentPool:
         if env.p2 != _lib.POLICY_PER_ENV:
             raise ValueError("OpponentPool needs HockeyVecEnv(..., p2='per_env')")
         self.env = env
-        self.snapshots = list(snapshots)
+        self.fused = isinstance(snapshots, FusedActorPool)
+        self.snapshots = snapshots if self.fused else list(snapshots)
         if p_snapshot > 0 and not self.snapshots:
             raise ValueError("p_snapshot > 0 without snapshots")
         k = len(self.snapshots)
@@ -45,11 +51,18 @@ class OpponentPool:
         self.choice = torch.zeros(env.num_envs, dtype=torch.long, device=env.device)
         self.codes = env.opponent_codes
         self._a2 = torch.zeros((env.num_envs, 4), dtype=torch.float32, device=env.device)
+        if self.fused:
+            self._a8 = torch.zeros((env.num_envs, 8), dtype=torch.float32, device=env.device)
+            self._pick = torch.empty(env.num_envs, dtype=torch.int32, device=env.device)
         self.resample(None)
 
     def add_snapshot(self, actor, p_snapshot=None):
-        """SelfPlayManager.add_snapshot (rl/training/self_play.py:30-45): later draws may pick `actor`."""
-        self.snapshots.append(actor)
+        """SelfPlayManager.add_snapshot (rl/training/self_play.py:30-45): later draws may pick `actor` (a module; with a
+        `FusedActorPool` it is packed into the pool)."""
+        if self.fused:
+            self.snapshots.add(actor)
+        else:
+            self.snapshots.append(actor)
         k = len(self.snapshots)
         ps = float(self.probs[2:].sum()) if p_snapshot is None else float(p_snapshot)
         base = self.probs[:2] / self.probs[:2].sum() * (1.0 - ps)
@@ -70,8 +83,14 @@ class OpponentPool:
     @torch.no_grad()
     def opponent_actions(self):
         """[N,4] actions of the snapshot opponents (zeros where an in-kernel BasicOpponent plays)."""
-        if not self.snapshots:
+        if not len(self.snapshots):
             return self._a2
+        if self.fused:
+            a2 = self._a8[:, 4:]
+            a2.zero_()
+            # snapshot index for the envs that drew one, -1 (not written) for the BasicOpponent envs
+            torch.sub(self.choice, self.SNAPSHOT0, out=self._pick).masked_fill_(self.choice < self.SNAPSHOT0, -1)
+            return self.snapshots(self.env.obs_agent_two(), self._pick, out=a2)
         obs2 = self.env.obs_agent_two()
         self._a2.zero_()
         for k, actor in enumerate(self.snapshots):
@@ -83,7 +102,12 @@ class OpponentPool:
     def step(self, a1):
         """One env tick with player-1 actions `a1` [N,4]; returns the env's step tuple.  Opponents of finished
         episodes are re-drawn afterwards."""
-        out = self.env.step(torch.cat([a1, self.opponent_actions()], dim=1).contiguous())
+        if self.fused:
+            self.opponent_actions()
+            self._a8[:, :4].copy_(a1)
+            out = self.env.step(self._a8)
+        else:
+            out = self.env.step(torch.cat([a1, self.opponent_actions()], dim=1).contiguous())
         self.resample(out[2])
         return out
 
@@ -207,6 +231,32 @@ def collect(pool_or_env, actor, buffer, steps):
     return buffer
 
 
+def _play_quota(env, act, k, max_ticks, credit):
+    """The complete-episode protocol of `evaluate`: sides alternate per env (even envs start with player 1), every env
+    plays a quota of `k` complete episodes and only those count.  Each tick: `act(obs)` gives the step's action tensor;
+    `credit(fin, winner, ret, length)` receives the float64 mask of the episodes that just finished within quota, the
+    winners, and the returns and lengths of those episodes.  Returns the per-env episode counts and the ticks played."""
+    n, dev = env.num_envs, env.device
+    obs, _ = env.reset(one_starting=(torch.arange(n, device=dev) % 2 == 0).to(torch.int8))
+    count = torch.zeros(n, dtype=torch.int64, device=dev)
+    ret = torch.zeros(n, dtype=torch.float64, device=dev)
+    length = torch.zeros(n, dtype=torch.int64, device=dev)
+    ticks = 0
+    while ticks < max_ticks:
+        obs, reward, done, _, info = env.step(act(obs))
+        ticks += 1
+        ret += reward.to(torch.float64)
+        length += 1
+        fin = done.to(torch.bool) & (count < k)
+        credit(fin.to(torch.float64), info["winner"], ret, length)
+        count += fin
+        ret = torch.where(done.to(torch.bool), torch.zeros_like(ret), ret)
+        length = torch.where(done.to(torch.bool), torch.zeros_like(length), length)
+        if ticks % 16 == 0 and bool((count >= k).all().item()):  # one small host read every 16 ticks
+            break
+    return count, ticks
+
+
 @torch.no_grad()
 def evaluate(actor, n_episodes=1000, opponent="strong", mode=Mode.NORMAL, num_envs=4096, device="cuda:0", seed=0,
              max_ticks=100000):
@@ -221,28 +271,13 @@ def evaluate(actor, n_episodes=1000, opponent="strong", mode=Mode.NORMAL, num_en
     env = HockeyVecEnv(num_envs, mode=mode, device=device, seed=seed, p2=opponent)
     n = env.num_envs
     k = -(-int(n_episodes) // n)
-    dev = env.device
-    obs, _ = env.reset(one_starting=(torch.arange(n, device=dev) % 2 == 0).to(torch.int8))
-    count = torch.zeros(n, dtype=torch.int64, device=dev)
-    ret = torch.zeros(n, dtype=torch.float64, device=dev)
-    length = torch.zeros(n, dtype=torch.int64, device=dev)
-    acc = torch.zeros(6, dtype=torch.float64, device=dev)  # wins, draws, losses, sum return, sum return^2, sum length
-    ticks = 0
-    while ticks < max_ticks:
-        obs, reward, done, _, info = env.step(actor(obs).contiguous())
-        ticks += 1
-        ret += reward.to(torch.float64)
-        length += 1
-        fin = done.to(torch.bool) & (count < k)
-        w = info["winner"]
-        f64 = fin.to(torch.float64)
-        acc += torch.stack([(f64 * (w == 1)).sum(), (f64 * (w == 0)).sum(), (f64 * (w == -1)).sum(), (f64 * ret).sum(),
-                            (f64 * ret * ret).sum(), (f64 * length).sum()])
-        count += fin
-        ret = torch.where(done.to(torch.bool), torch.zeros_like(ret), ret)
-        length = torch.where(done.to(torch.bool), torch.zeros_like(length), length)
-        if ticks % 16 == 0 and bool((count >= k).all().item()):  # one small host read every 16 ticks
-            break
+    acc = torch.zeros(6, dtype=torch.float64, device=env.device)  # wins, draws, losses, sum return, sum return^2, sum length
+
+    def credit(f64, w, ret, length):
+        acc.add_(torch.stack([(f64 * (w == 1)).sum(), (f64 * (w == 0)).sum(), (f64 * (w == -1)).sum(), (f64 * ret).sum(),
+                              (f64 * ret * ret).sum(), (f64 * length).sum()]))
+
+    count, ticks = _play_quota(env, lambda obs: actor(obs).contiguous(), k, max_ticks, credit)
     env.close()
     a = acc.cpu().tolist()
     m = max(int(count.sum().item()), 1)
@@ -250,6 +285,50 @@ def evaluate(actor, n_episodes=1000, opponent="strong", mode=Mode.NORMAL, num_en
     return {"episodes": m, "win_rate": a[0] / m, "draw_rate": a[1] / m, "loss_rate": a[2] / m, "mean_return": mean_ret,
             "std_return": max(a[4] / m - mean_ret * mean_ret, 0.0) ** 0.5, "mean_length": a[5] / m, "ticks": ticks,
             "episodes_per_env": k}
+
+
+@torch.no_grad()
+def cross_play(actors, episodes_per_pair, num_envs, mode=Mode.NORMAL, seed=0, device="cuda:0", max_ticks=100000):
+    """League table of K actors (modules of the reference architecture, or a `FusedActorPool`): every ordered pair
+    (i as player 1, j as player 2) plays `episodes_per_pair` or more COMPLETE episodes on an equal block of
+    B = num_envs // K^2 envs (rounded down to even, so both sides start equally often), with `evaluate`'s protocol:
+    a quota of ceil(episodes_per_pair / B) episodes per env, alternating sides.  Each tick is two pooled tensor-core
+    launches: player 1 on `obs` into action columns 0..3, player 2 on `obs_agent_two()` into columns 4..7.
+
+    Returns [K, K] float64 tensors (row i = player 1, column j = player 2, player 1's side): `win_rate`, `draw_rate`,
+    `loss_rate`, `mean_return`, and `episodes`; plus `ticks` and `episodes_per_env`."""
+    pool = actors if isinstance(actors, FusedActorPool) else FusedActorPool(actors, device=device)
+    kk = len(pool)
+    if kk < 1:
+        raise ValueError("cross_play needs at least one actor")
+    per_pair = num_envs // (kk * kk)
+    per_pair -= per_pair % 2
+    if per_pair < 2:
+        raise ValueError(f"cross_play needs num_envs >= 2 * K^2 = {2 * kk * kk}")
+    env = HockeyVecEnv(per_pair * kk * kk, mode=mode, device=pool.device, seed=seed, p1=None, p2=None)
+    n, dev = env.num_envs, env.device
+    pair = torch.arange(n, device=dev) // per_pair
+    c1, c2 = (pair // kk).to(torch.int32), (pair % kk).to(torch.int32)
+    a8 = torch.zeros((n, 8), dtype=torch.float32, device=dev)
+    acc = torch.zeros((kk * kk, 6), dtype=torch.float64, device=dev)  # per pair: as `evaluate`'s accumulator
+
+    def act(obs):
+        pool(obs, c1, out=a8[:, :4])
+        pool(env.obs_agent_two(), c2, out=a8[:, 4:])
+        return a8
+
+    def credit(f64, w, ret, length):
+        acc.index_add_(0, pair, torch.stack([f64 * (w == 1), f64 * (w == 0), f64 * (w == -1), f64 * ret, f64 * ret * ret,
+                                             f64 * length], 1))
+
+    k = -(-int(episodes_per_pair) // per_pair)
+    count, ticks = _play_quota(env, act, k, max_ticks, credit)
+    env.close()
+    episodes = torch.zeros(kk * kk, dtype=torch.float64, device=dev).index_add_(0, pair, count.to(torch.float64))
+    m = episodes.clamp(min=1).unsqueeze(1)
+    rates = (acc / m).view(kk, kk, 6)
+    return {"win_rate": rates[..., 0], "draw_rate": rates[..., 1], "loss_rate": rates[..., 2], "mean_return": rates[..., 3],
+            "episodes": episodes.view(kk, kk), "ticks": ticks, "episodes_per_env": k}
 
 
 @torch.no_grad()

@@ -218,6 +218,22 @@ int hk_actor_param_bytes(void);
 int hk_actor_forward(const void* params_dev, const float* obs_dev, float* act_dev, int act_stride, int64_t n, int device,
                      void* stream);
 
+/* Snapshot pool of the same actor (self-play opponents, league play): act[i, 0..3] = actor_{choice[i]}(obs[i, 0..17]) for
+ * every row with 0 <= choice[i] < k; rows with any other choice (negative included) are NOT written.  params_dev: k
+ * hk_actor_param_bytes()-byte blocks back to back (snapshot s at s * hk_actor_param_bytes(); 16-byte aligned).
+ * choice_dev: i32 [n] (4-byte aligned); obs_dev / act_dev / act_stride as for hk_actor_forward; 1 <= n <= 2^31 - 1,
+ * 1 <= k <= 4096.  scratch_dev: caller-owned device memory of hk_actor_pool_scratch_bytes(n, k) bytes (16-byte aligned,
+ * contents need not be initialised; one call at a time per buffer); the library allocates nothing per call.
+ * Each output row equals hk_actor_forward of its snapshot on that row, bit for bit.  The rows are grouped by snapshot
+ * on the device (a memset and three small kernels: histogram, offsets, row lists), then one persistent tensor-core
+ * kernel runs tiles of 128 rows of one snapshot each, copying a snapshot's weights into shared memory when its tiles
+ * start.  Enqueued on `stream` with no host synchronisation; graph-capturable.  Invalid arguments return HK_E_INVALID
+ * (before any device probe); valid ones without a GPU HK_E_NODEVICE.
+ * hk_actor_pool_scratch_bytes returns HK_E_INVALID for n or k out of range. */
+int64_t hk_actor_pool_scratch_bytes(int64_t n, int k);
+int hk_actor_forward_pool(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev,
+                          int act_stride, int64_t n, void* scratch_dev, int device, void* stream);
+
 /* Measurement: per-kernel device times of the ticks that follow.  hk_kernel_timing(env, 1) makes every hk_step /
  * hk_rollout tick record CUDA events on the launching stream around each kernel of the cascade (up to 2048 ticks; not
  * graph-capturable while enabled); hk_kernel_times synchronises the device, returns the summed milliseconds of
