@@ -54,6 +54,44 @@ def _cuda_device(device, who):
     return device
 
 
+_PARAM_SHAPES = (("fc1.weight", (256, 18)), ("fc1.bias", (256,)), ("fc2.weight", (256, 256)), ("fc2.bias", (256,)),
+                 ("fc3.weight", (4, 256)), ("fc3.bias", (4,)))
+
+
+def _live_params(actor, device, who):
+    """The module's six parameter tensors on `device` as contiguous fp32 (in place when they already are: no copy, no
+    host sync), in hk_actor_pack's order w1, b1, w2, b2, w3, b3."""
+    sd = actor.state_dict(keep_vars=True)
+    out = []
+    for name, shape in _PARAM_SHAPES:
+        t = sd[name].detach()
+        if tuple(t.shape) != shape:
+            raise ValueError(f"{who} implements the reference architecture 18 -> 256 -> 256 -> 4")
+        if t.device.type != "cuda" or (t.device.index or 0) != (device.index or 0):
+            raise ValueError(f"{who}: the module's parameters are on {t.device}, the packed block on {device}")
+        out.append(t.to(torch.float32).contiguous())
+    return out
+
+
+def _pack_on_device(L, lib, actor, dst, device, who):
+    """hk_actor_pack of `actor`'s live parameters into the 16-byte aligned block at `dst` (a uint8 CUDA tensor view)."""
+    import ctypes as C
+    ps = _live_params(actor, device, who)
+    with torch.cuda.device(device):
+        lib.check(L.hk_actor_pack(*[C.c_void_p(p.data_ptr()) for p in ps], C.c_void_p(dst.data_ptr()), device.index or 0,
+                                  C.c_void_p(torch.cuda.current_stream(device).cuda_stream)))
+
+
+def _noise_args(noise, noise_clip):
+    sigma = float(noise)
+    if not (sigma >= 0.0 and sigma != float("inf")):
+        raise ValueError("noise must be a finite standard deviation >= 0")
+    clip = 0.0 if noise_clip is None else float(noise_clip)
+    if clip != clip:
+        raise ValueError("noise_clip must not be NaN")
+    return sigma, clip
+
+
 def _reference_state_dict(actor, who):
     """The fp32 CPU state dict of an ActorNetwork-shaped module, checked against the reference architecture."""
     sd = {k: v.detach().to("cpu", torch.float32) for k, v in actor.state_dict().items()}
@@ -67,11 +105,17 @@ class FusedActor:
     shared memory (layer 1 TF32, layers 2-3 bf16), fp32 accumulation in tensor memory, hidden activations never leave the SM.  Callable like the
     module: obs [N,18] float32 CUDA tensor -> actions [N,4] (a persistent output buffer, overwritten by the next call;
     pass `out=` to write into columns 0..3 of an existing [N,4] / [N,8] action tensor).  There is no fallback: without the
-    CUDA library or a GPU this raises."""
+    CUDA library or a GPU this raises.
+
+    For a policy that is being trained: `refresh(module)` repacks the block on the device from the module's live
+    parameters (hk_actor_pack: no CPU copy, no host sync, graph-capturable), and `noise=sigma` adds TD3 exploration
+    noise in the kernel's epilogue, clamp(actor(obs) + clip(sigma * z, +-noise_clip), -1, 1) with z drawn by Philox from
+    (seed, row0 + row, counter).  The counter is a device int64 (`self.counter`) that every noisy call advances, so
+    consecutive calls -- and the replays of a captured graph -- draw fresh noise."""
 
     PARAM_BYTES = 256 * 24 * 4 + 256 * 256 * 2 + 16 * 256 * 2 + 2 * 256 * 4 + 16 * 4  # hk_actor_param_bytes()
 
-    def __init__(self, actor, device="cuda:0"):
+    def __init__(self, actor, device="cuda:0", seed=0):
         import ctypes as C
         from . import _lib
         self._C, self._lib = C, _lib
@@ -80,6 +124,14 @@ class FusedActor:
         self.params = self.pack(_reference_state_dict(actor, "FusedActor")).to(self.device)
         assert self.params.numel() == int(self.L.hk_actor_param_bytes())
         self._out = None
+        self.seed = int(seed) & (2**64 - 1)
+        self.counter = torch.zeros(1, dtype=torch.int64, device=self.device)
+
+    def refresh(self, actor):
+        """Repack the block in place from `actor`'s live parameters (fp32 tensors on this device), on the current
+        stream: no CPU copy, no host sync.  The result equals `FusedActor.pack` of the same weights byte for byte."""
+        _pack_on_device(self.L, self._lib, actor, self.params, self.device, "FusedActor.refresh")
+        return self
 
     @staticmethod
     def _core_matrix_order(w, n_pad, k_pad, dtype):
@@ -102,9 +154,13 @@ class FusedActor:
                  sd["fc2.bias"].contiguous().view(torch.uint8).flatten(), b3.view(torch.uint8).flatten()]
         return torch.cat(parts).contiguous()
 
-    def __call__(self, obs, out=None):
+    def __call__(self, obs, out=None, noise=0.0, noise_clip=None, row0=0):
+        """actions = actor(obs); with noise > 0, clamp(actor(obs) + clip(noise * z, +-noise_clip), -1, 1) (noise_clip None
+        or <= 0: no clip), then the counter advances.  `row0` is the global index of row 0 (shards of one batch pass
+        their offset to draw the same noise as one call over the whole batch)."""
         if not (obs.is_cuda and obs.dtype == torch.float32 and obs.is_contiguous() and obs.dim() == 2 and obs.shape[1] == 18):
             raise ValueError("FusedActor expects a contiguous float32 CUDA tensor [N, 18]")
+        sigma, clip = _noise_args(noise, noise_clip)
         n = obs.shape[0]
         if out is None:
             if self._out is None or self._out.shape[0] != n:
@@ -114,9 +170,15 @@ class FusedActor:
             raise ValueError("out must be a float32 CUDA tensor [N, >= 4] with unit column stride")
         C = self._C
         with torch.cuda.device(obs.device):
-            self._lib.check(self.L.hk_actor_forward(C.c_void_p(self.params.data_ptr()), C.c_void_p(obs.data_ptr()),
-                                                    C.c_void_p(out.data_ptr()), int(out.stride(0)), n, obs.device.index or 0,
-                                                    C.c_void_p(torch.cuda.current_stream(obs.device).cuda_stream)))
+            stream = C.c_void_p(torch.cuda.current_stream(obs.device).cuda_stream)
+            if sigma == 0.0:
+                self._lib.check(self.L.hk_actor_forward(C.c_void_p(self.params.data_ptr()), C.c_void_p(obs.data_ptr()),
+                                                        C.c_void_p(out.data_ptr()), int(out.stride(0)), n, obs.device.index or 0, stream))
+            else:
+                self._lib.check(self.L.hk_actor_forward_noisy(
+                    C.c_void_p(self.params.data_ptr()), C.c_void_p(obs.data_ptr()), C.c_void_p(out.data_ptr()), int(out.stride(0)), n,
+                    self.seed, C.c_void_p(self.counter.data_ptr()), sigma, clip, int(row0), obs.device.index or 0, stream))
+                self.counter.add_(1)
         return out[:, :4] if out.shape[1] != 4 else out
 
 
@@ -125,12 +187,13 @@ class FusedActorPool:
     (csrc/hk_actor.cuh k_actor_pool_mlp, hk_actor_forward_pool): row i goes through snapshot choice[i].  The rows are
     grouped by snapshot on the device (no host sync; graph-capturable), and each written row equals
     `FusedActor(snapshot choice[i])(obs)[i]` bit for bit.  The table is one [K, hk_actor_param_bytes()] uint8 device
-    tensor of `FusedActor.pack` blocks; `add` appends one (and re-allocates the table: re-capture graphs after it).
-    There is no fallback: without the CUDA library or a GPU this raises."""
+    tensor of `FusedActor.pack` blocks; `add` appends one (and re-allocates the table: re-capture graphs after it), `set`
+    repacks one slot in place on the device.  `noise=` / `noise_clip=` add the epilogue noise of `FusedActor` (keyed on
+    the row, not on the snapshot).  There is no fallback: without the CUDA library or a GPU this raises."""
 
     MAX_K = 4096
 
-    def __init__(self, actors=(), device="cuda:0"):
+    def __init__(self, actors=(), device="cuda:0", seed=0):
         import ctypes as C
         from . import _lib
         self._C, self._lib = C, _lib
@@ -139,6 +202,8 @@ class FusedActorPool:
         self.table = self.pack(actors).to(self.device)
         self._out = None
         self._scratch = torch.empty(0, dtype=torch.uint8, device=self.device)
+        self.seed = int(seed) & (2**64 - 1)
+        self.counter = torch.zeros(1, dtype=torch.int64, device=self.device)
 
     @staticmethod
     def pack(actors):
@@ -158,13 +223,23 @@ class FusedActorPool:
         self.table = torch.cat([self.table, blk])
         return len(self) - 1
 
-    def __call__(self, obs, choice, out=None):
+    def set(self, i, actor):
+        """Repack slot `i` in place from `actor`'s live parameters (hk_actor_pack into the table: no CPU copy, no host
+        sync); the other slots are not touched."""
+        i = int(i)
+        if not 0 <= i < len(self):
+            raise IndexError(f"FusedActorPool slot {i} out of range [0, {len(self)})")
+        _pack_on_device(self.L, self._lib, actor, self.table[i], self.device, "FusedActorPool.set")
+
+    def __call__(self, obs, choice, out=None, noise=0.0, noise_clip=None, row0=0):
         """obs [N,18] float32 CUDA, choice int32 / int64 CUDA [N] -> act[i] = actor_{choice[i]}(obs[i]) for choice[i] in
         [0, K); other rows are not written.  out=None: a persistent [N,4] buffer (overwritten by the next call) whose
         skipped rows are 0; or pass `out` = an [N, >= 4] float32 view with unit column stride (e.g. `a8[:, 4:]` of the
-        [N,8] action tensor): columns 0..3 of its written rows change, nothing else."""
+        [N,8] action tensor): columns 0..3 of its written rows change, nothing else.  noise / noise_clip / row0 as for
+        `FusedActor`; a noisy call advances the counter."""
         if not (obs.is_cuda and obs.dtype == torch.float32 and obs.is_contiguous() and obs.dim() == 2 and obs.shape[1] == 18):
             raise ValueError("FusedActorPool expects a contiguous float32 CUDA tensor [N, 18]")
+        sigma, clip = _noise_args(noise, noise_clip)
         n, k = obs.shape[0], len(self)
         if k == 0:
             raise ValueError("FusedActorPool is empty: add() a snapshot first")
@@ -190,10 +265,17 @@ class FusedActorPool:
             self._scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
         C = self._C
         with torch.cuda.device(obs.device):
-            self._lib.check(self.L.hk_actor_forward_pool(C.c_void_p(self.table.data_ptr()), k, C.c_void_p(choice.data_ptr()),
-                                                         C.c_void_p(obs.data_ptr()), C.c_void_p(out.data_ptr()), int(out.stride(0)),
-                                                         n, C.c_void_p(self._scratch.data_ptr()), obs.device.index or 0,
-                                                         C.c_void_p(torch.cuda.current_stream(obs.device).cuda_stream)))
+            stream = C.c_void_p(torch.cuda.current_stream(obs.device).cuda_stream)
+            if sigma == 0.0:
+                self._lib.check(self.L.hk_actor_forward_pool(C.c_void_p(self.table.data_ptr()), k, C.c_void_p(choice.data_ptr()),
+                                                             C.c_void_p(obs.data_ptr()), C.c_void_p(out.data_ptr()), int(out.stride(0)),
+                                                             n, C.c_void_p(self._scratch.data_ptr()), obs.device.index or 0, stream))
+            else:
+                self._lib.check(self.L.hk_actor_forward_pool_noisy(
+                    C.c_void_p(self.table.data_ptr()), k, C.c_void_p(choice.data_ptr()), C.c_void_p(obs.data_ptr()),
+                    C.c_void_p(out.data_ptr()), int(out.stride(0)), n, C.c_void_p(self._scratch.data_ptr()), self.seed,
+                    C.c_void_p(self.counter.data_ptr()), sigma, clip, int(row0), obs.device.index or 0, stream))
+                self.counter.add_(1)
         return out[:, :4] if out.shape[1] != 4 else out
 
 

@@ -29,7 +29,7 @@ constexpr int kN3 = 16;      // layer-3 N, padded from 4 to the smallest UMMA N 
 constexpr int kAct = 4;
 constexpr int kThreads = 128;
 
-// packed parameter block (prepared once by the host side, see actor.py FusedActor): byte offsets
+// packed parameter block (packed by the host side, actor.py FusedActor.pack, or on the device, k_actor_pack): byte offsets
 constexpr int kOffW1 = 0;                                // [kHidden x kK1]     tf32 (f32 bits), canonical K-major core-matrix order
 constexpr int kOffW2 = kOffW1 + kHidden * kK1 * 4;       // [kHidden x kHidden] bf16
 constexpr int kOffW3 = kOffW2 + kHidden * kHidden * 2;   // [kN3 x kHidden]     bf16 (rows 4..15 zero)
@@ -180,12 +180,58 @@ __device__ __forceinline__ void actorTeardown(const TileCtx& c) {
   if ((threadIdx.x >> 5) == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(c.tmem), "r"(512));
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Exploration / target-policy-smoothing noise in the layer-3 epilogue (the `kNoisy` instantiations):
+//   act = clamp(tanh(MLP(obs)) + clip(sigma * z, -clip, clip), -1, 1),   z = four standard normals per row.
+// Row i's normals come from ONE Philox4x32-10 call, hk::philox(seed, row0 + i, (uint32_t)ctr,
+// HK_STREAM_ACTOR_NOISE | (uint32_t)(ctr >> 32) << 8), ctr = the call's counter (read from device memory, so a replayed
+// graph draws fresh noise; the low 56 bits count), and Box-Muller on its words (x, y) -> z0, z1 and (z, w) -> z2, z3:
+//   u1 = ((a >> 8) + 1) * 2^-24  in (0, 1]  (log finite),   u2 = (b >> 8) * 2^-24  in [0, 1),
+//   r = sqrtf(-2 logf(u1)),   (z_even, z_odd) = (r cospif(2 u2), r sinpif(2 u2)).
+// A row's noise depends on its key only: not on n, the tile order or (in the pool) the grouping; `row0` lets shards of
+// one batch agree.  |z| <= sqrt(48 ln 2) ~ 5.77.
+struct NoiseKey {
+  uint64_t seed;
+  long long row0;
+  uint32_t c2, c3;   // Philox counter words 2 and 3 (counter low word, stream tag | counter high bits << 8)
+  float sigma, clip; // clip = +inf: no clip
+};
+
+__device__ __forceinline__ NoiseKey noiseKey(uint64_t seed, const uint64_t* counter, float sigma, float clip, long long row0) {
+  const uint64_t ctr = *counter;
+  NoiseKey k;
+  k.seed = seed;
+  k.row0 = row0;
+  k.c2 = (uint32_t)ctr;
+  k.c3 = (uint32_t)hk::HK_STREAM_ACTOR_NOISE | ((uint32_t)(ctr >> 32) << 8);
+  k.sigma = sigma;
+  k.clip = clip;
+  return k;
+}
+
+__device__ __forceinline__ void boxMuller(uint32_t a, uint32_t b, float& z0, float& z1) {
+  const float u1 = (float)((a >> 8) + 1u) * (1.0f / 16777216.0f);
+  const float u2 = (float)(b >> 8) * (1.0f / 16777216.0f);
+  const float r = sqrtf(-2.0f * logf(u1));
+  float s, c;
+  sincospif(2.0f * u2, &s, &c);
+  z0 = r * c;
+  z1 = r * s;
+}
+
+__device__ __forceinline__ float addNoise(float a, float z, const NoiseKey& k) {
+  const float e = fminf(fmaxf(k.sigma * z, -k.clip), k.clip);
+  return fminf(fmaxf(a + e, -1.0f), 1.0f);
+}
+
 // One tile of 128 rows through the three layers with the weights now in shared memory.  Thread t owns TMEM lane t; `row`
 // is the observation / action row it reads and writes, or -1 for a padding lane (zero input, nothing stored).  The only
 // thing the callers differ in is how a thread finds its row.  Ends in a block barrier: on return every MMA of the tile
-// has completed and every thread is done with the tile's shared memory (the weights may be replaced).
+// has completed and every thread is done with the tile's shared memory (the weights may be replaced).  kNoisy adds the
+// noise of `nk` to the four outputs (see NoiseKey); the plain instantiation ignores `nk`.
+template <bool kNoisy>
 __device__ __forceinline__ void actorTile(const TileCtx& c, uint32_t& phase, const float* __restrict__ obs,
-                                          float* __restrict__ act, int actStride, long long row) {
+                                          float* __restrict__ act, int actStride, long long row, const NoiseKey& nk) {
   const int t = threadIdx.x;
   unsigned char* smem = c.smem;
   const uint32_t tmem = c.tmem, myT = c.myT, barA = c.barA;
@@ -263,10 +309,21 @@ __device__ __forceinline__ void actorTile(const TileCtx& c, uint32_t& phase, con
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
     if (row >= 0) {
       float* dst = act + row * actStride;
-      dst[0] = tanhApprox(__uint_as_float(r0) + b3[0]);
-      dst[1] = tanhApprox(__uint_as_float(r1) + b3[1]);
-      dst[2] = tanhApprox(__uint_as_float(r2) + b3[2]);
-      dst[3] = tanhApprox(__uint_as_float(r3) + b3[3]);
+      if constexpr (kNoisy) {
+        const hk::U4 w = hk::philox(nk.seed, (uint64_t)(nk.row0 + row), nk.c2, nk.c3);
+        float z0, z1, z2, z3;
+        boxMuller(w.x, w.y, z0, z1);
+        boxMuller(w.z, w.w, z2, z3);
+        dst[0] = addNoise(tanhApprox(__uint_as_float(r0) + b3[0]), z0, nk);
+        dst[1] = addNoise(tanhApprox(__uint_as_float(r1) + b3[1]), z1, nk);
+        dst[2] = addNoise(tanhApprox(__uint_as_float(r2) + b3[2]), z2, nk);
+        dst[3] = addNoise(tanhApprox(__uint_as_float(r3) + b3[3]), z3, nk);
+      } else {
+        dst[0] = tanhApprox(__uint_as_float(r0) + b3[0]);
+        dst[1] = tanhApprox(__uint_as_float(r1) + b3[1]);
+        dst[2] = tanhApprox(__uint_as_float(r2) + b3[2]);
+        dst[3] = tanhApprox(__uint_as_float(r3) + b3[3]);
+      }
     }
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -274,8 +331,9 @@ __device__ __forceinline__ void actorTile(const TileCtx& c, uint32_t& phase, con
 }
 
 // one weight set, rows 0..n-1 in order: tile `tile` holds rows tile * 128 + t
-__global__ void __launch_bounds__(kThreads, 1) k_actor_mlp(const unsigned char* __restrict__ params, const float* __restrict__ obs,
-                                                           float* __restrict__ act, int actStride, long long n) {
+template <bool kNoisy>
+__device__ __forceinline__ void actorMlp(const unsigned char* __restrict__ params, const float* __restrict__ obs,
+                                         float* __restrict__ act, int actStride, long long n, const NoiseKey& nk) {
   extern __shared__ __align__(128) unsigned char smem[];
   loadParams(smem, params);  // once per CTA
   const TileCtx c = actorSetup(smem);
@@ -283,9 +341,21 @@ __global__ void __launch_bounds__(kThreads, 1) k_actor_mlp(const unsigned char* 
   const long long tiles = (n + kRows - 1) / kRows;
   for (long long tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
     const long long row = tile * kRows + threadIdx.x;
-    actorTile(c, phase, obs, act, actStride, row < n ? row : -1);
+    actorTile<kNoisy>(c, phase, obs, act, actStride, row < n ? row : -1, nk);
   }
   actorTeardown(c);
+}
+
+__global__ void __launch_bounds__(kThreads, 1) k_actor_mlp(const unsigned char* __restrict__ params, const float* __restrict__ obs,
+                                                           float* __restrict__ act, int actStride, long long n) {
+  actorMlp<false>(params, obs, act, actStride, n, NoiseKey{});
+}
+
+__global__ void __launch_bounds__(kThreads, 1) k_actor_mlp_noisy(const unsigned char* __restrict__ params, const float* __restrict__ obs,
+                                                                 float* __restrict__ act, int actStride, long long n, uint64_t seed,
+                                                                 const uint64_t* __restrict__ counter, float sigma, float clip,
+                                                                 long long row0) {
+  actorMlp<true>(params, obs, act, actStride, n, noiseKey(seed, counter, sigma, clip, row0));
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -405,9 +475,10 @@ __global__ void __launch_bounds__(kPoolThreads) k_pool_scatter(const int32_t* __
 // Persistent: CTA b walks the contiguous tile range [b T / G, (b + 1) T / G) of the T = tileOff[K] tiles, so it crosses few
 // group boundaries; it copies a snapshot's weights into shared memory only when the group changes.  Tile j of group s holds
 // rows[groupOff[s] + j * 128 + t]; lanes past the group's end are padding.
-__global__ void __launch_bounds__(kThreads, 1) k_actor_pool_mlp(const unsigned char* __restrict__ params, int k,
-                                                                const int32_t* __restrict__ scratch, const float* __restrict__ obs,
-                                                                float* __restrict__ act, int actStride) {
+template <bool kNoisy>
+__device__ __forceinline__ void actorPoolMlp(const unsigned char* __restrict__ params, int k, const int32_t* __restrict__ scratch,
+                                             const float* __restrict__ obs, float* __restrict__ act, int actStride,
+                                             const NoiseKey& nk) {
   extern __shared__ __align__(128) unsigned char smem[];
   const int32_t* groupOff = scratch + poolOffGroup(k);
   const int32_t* tileOff = scratch + poolOffTile(k);
@@ -432,9 +503,71 @@ __global__ void __launch_bounds__(kThreads, 1) k_actor_pool_mlp(const unsigned c
     }
     const int local = (int)(tile - tileOff[s]) * kRows + threadIdx.x;
     const int count = groupOff[s + 1] - groupOff[s];
-    actorTile(c, phase, obs, act, actStride, local < count ? (long long)rows[groupOff[s] + local] : -1LL);
+    actorTile<kNoisy>(c, phase, obs, act, actStride, local < count ? (long long)rows[groupOff[s] + local] : -1LL, nk);
   }
   actorTeardown(c);
+}
+
+__global__ void __launch_bounds__(kThreads, 1) k_actor_pool_mlp(const unsigned char* __restrict__ params, int k,
+                                                                const int32_t* __restrict__ scratch, const float* __restrict__ obs,
+                                                                float* __restrict__ act, int actStride) {
+  actorPoolMlp<false>(params, k, scratch, obs, act, actStride, NoiseKey{});
+}
+
+__global__ void __launch_bounds__(kThreads, 1) k_actor_pool_mlp_noisy(const unsigned char* __restrict__ params, int k,
+                                                                      const int32_t* __restrict__ scratch, const float* __restrict__ obs,
+                                                                      float* __restrict__ act, int actStride, uint64_t seed,
+                                                                      const uint64_t* __restrict__ counter, float sigma, float clip,
+                                                                      long long row0) {
+  actorPoolMlp<true>(params, k, scratch, obs, act, actStride, noiseKey(seed, counter, sigma, clip, row0));
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Device-side pack: an ActorNetwork's fp32 parameters (fc1 [256, 18], fc2 [256, 256], fc3 [4, 256] row-major, biases)
+// -> one kParamBytes block, byte-identical to actor.py FusedActor.pack.  Thread j writes 32-bit word j of the block:
+// layer 1 as raw f32 bits, layers 2-3 as two bf16 (round to nearest even) of consecutive k, in K-major core-matrix order
+// (element (n, k) of a [N, K] operand with e elements per 16-byte chunk at (k / e) * (N * 16) + n * 16 + (k % e) * size
+// bytes), zeros in the padding (K 18 -> 24, fc3 rows 4 -> 16, b3 4 -> 16).
+constexpr int kPackThreads = 256;
+constexpr int kParamWords = kParamBytes / 4;
+
+__device__ __forceinline__ uint32_t bf16Bits(float x) {
+  const __nv_bfloat16 h = __float2bfloat16_rn(x);
+  return (uint32_t)*reinterpret_cast<const uint16_t*>(&h);
+}
+
+// word `j` of a bf16 [nPad x kDim] operand (8 elements per chunk): elements (n, k), (n, k + 1) of w [nReal x kDim]
+__device__ __forceinline__ uint32_t packBf16Word(const float* __restrict__ w, int j, int nPad, int nReal, int kDim) {
+  const int chunk = j / (nPad * 4), rem = j % (nPad * 4);
+  const int n = rem / 4, k = chunk * 8 + (rem % 4) * 2;
+  if (n >= nReal) return 0u;
+  return bf16Bits(w[n * kDim + k]) | (bf16Bits(w[n * kDim + k + 1]) << 16);
+}
+
+__global__ void __launch_bounds__(kPackThreads) k_actor_pack(const float* __restrict__ w1, const float* __restrict__ b1,
+                                                             const float* __restrict__ w2, const float* __restrict__ b2,
+                                                             const float* __restrict__ w3, const float* __restrict__ b3,
+                                                             uint32_t* __restrict__ out) {
+  const int j = blockIdx.x * kPackThreads + threadIdx.x;
+  if (j >= kParamWords) return;
+  uint32_t v;
+  if (j < kOffW2 / 4) {  // layer 1: 4 f32 per chunk
+    const int chunk = j / (kHidden * 4), rem = j % (kHidden * 4);
+    const int n = rem / 4, k = chunk * 4 + rem % 4;
+    v = k < kObs ? __float_as_uint(w1[n * kObs + k]) : 0u;
+  } else if (j < kOffW3 / 4) {
+    v = packBf16Word(w2, j - kOffW2 / 4, kHidden, kHidden, kHidden);
+  } else if (j < kOffB1 / 4) {
+    v = packBf16Word(w3, j - kOffW3 / 4, kN3, kAct, kHidden);
+  } else if (j < kOffB2 / 4) {
+    v = __float_as_uint(b1[j - kOffB1 / 4]);
+  } else if (j < kOffB3 / 4) {
+    v = __float_as_uint(b2[j - kOffB2 / 4]);
+  } else {
+    const int i = j - kOffB3 / 4;
+    v = i < kAct ? __float_as_uint(b3[i]) : 0u;
+  }
+  out[j] = v;
 }
 
 }  // namespace hk_actor

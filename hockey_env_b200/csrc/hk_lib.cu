@@ -13,6 +13,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <algorithm>
+#include <cmath>
 #include <string>
 
 #include "../../include/hockey_b200.h"
@@ -1944,26 +1945,83 @@ int hk_debug_lane_trace(hk_env* h, uint32_t* out_host, int64_t n_words) {
 
 int hk_actor_param_bytes(void) { return hk_actor::kParamBytes; }
 
-int hk_actor_forward(const void* params_dev, const float* obs_dev, float* act_dev, int act_stride, int64_t n, int device, void* stream) {
-  if (!params_dev || !obs_dev || !act_dev) return fail(HK_E_INVALID, "hk_actor_forward: NULL argument");
-  if (n <= 0 || act_stride < hk_actor::kAct) return fail(HK_E_INVALID, "hk_actor_forward: n must be positive and act_stride >= 4");
-  if ((((uintptr_t)params_dev) & 15u) || (((uintptr_t)obs_dev) & 7u)) return fail(HK_E_INVALID, "hk_actor_forward: params need 16-byte, obs 8-byte alignment");
+// validation shared by the plain and the noisy entry points (error messages name `who`); HK_OK or an error code
+static int actorCheck(const char* who, const void* params_dev, const float* obs_dev, const float* act_dev, int act_stride, int64_t n) {
+  if (!params_dev || !obs_dev || !act_dev) return fail(HK_E_INVALID, std::string(who) + ": NULL argument");
+  if (n <= 0 || act_stride < hk_actor::kAct) return fail(HK_E_INVALID, std::string(who) + ": n must be positive and act_stride >= 4");
+  if ((((uintptr_t)params_dev) & 15u) || (((uintptr_t)obs_dev) & 7u)) return fail(HK_E_INVALID, std::string(who) + ": params need 16-byte, obs 8-byte alignment");
+  return HK_OK;
+}
+
+static int noiseCheck(const char* who, const uint64_t* counter_dev, float sigma, float clip, int64_t row0) {
+  if (!counter_dev) return fail(HK_E_INVALID, std::string(who) + ": NULL argument");
+  if (((uintptr_t)counter_dev) & 7u) return fail(HK_E_INVALID, std::string(who) + ": counter needs 8-byte alignment");
+  if (!(sigma >= 0.0f) || std::isinf(sigma)) return fail(HK_E_INVALID, std::string(who) + ": sigma must be finite and >= 0");
+  if (std::isnan(clip)) return fail(HK_E_INVALID, std::string(who) + ": clip must not be NaN");
+  if (row0 < 0) return fail(HK_E_INVALID, std::string(who) + ": row0 must be >= 0");
+  return HK_OK;
+}
+
+static int deviceCheck(const char* who, int device) {
   int count = 0;
-  if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) return fail(HK_E_NODEVICE, "hk_actor_forward: no CUDA device (there is no CPU fallback)");
-  if (device < 0 || device >= count) return fail(HK_E_INVALID, "hk_actor_forward: bad device index");
-  DeviceGuard guard(device);
-  static bool configured[64] = {false};
+  if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) return fail(HK_E_NODEVICE, std::string(who) + ": no CUDA device (there is no CPU fallback)");
+  if (device < 0 || device >= count) return fail(HK_E_INVALID, std::string(who) + ": bad device index");
+  return HK_OK;
+}
+
+// clip <= 0 or +inf: no clip (the kernel clamps to +-inf)
+static float effectiveClip(float clip) { return clip > 0.0f ? clip : INFINITY; }
+
+static int actorConfigure(const void* kernel, bool* configured, int device) {
   if (!configured[device & 63]) {
-    HK_CUDA(cudaFuncSetAttribute(hk_actor::k_actor_mlp, cudaFuncAttributeMaxDynamicSharedMemorySize, hk_actor::kSmemBytes));
+    HK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, hk_actor::kSmemBytes));
     configured[device & 63] = true;
   }
+  return HK_OK;
+}
+
+static int actorSms(int device) {
   int sms = 148;
   if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sms < 1) sms = 148;
+  return sms;
+}
+
+// One launch of the single-weight-set kernel; sigma == 0 runs the plain kernel (bit-identical to hk_actor_forward).
+static int actorLaunch(const void* params_dev, const float* obs_dev, float* act_dev, int act_stride, int64_t n, bool noisy,
+                       uint64_t seed, const uint64_t* counter_dev, float sigma, float clip, int64_t row0, int device, void* stream) {
+  DeviceGuard guard(device);
   const int64_t tiles = (n + hk_actor::kRows - 1) / hk_actor::kRows;
-  hk_actor::k_actor_mlp<<<(unsigned)std::min<int64_t>(tiles, sms), hk_actor::kThreads, hk_actor::kSmemBytes, (cudaStream_t)stream>>>(
-      (const unsigned char*)params_dev, obs_dev, act_dev, act_stride, (long long)n);
+  const unsigned grid = (unsigned)std::min<int64_t>(tiles, actorSms(device));
+  if (noisy && sigma != 0.0f) {
+    static bool configured[64] = {false};
+    if (int rc = actorConfigure((const void*)hk_actor::k_actor_mlp_noisy, configured, device)) return rc;
+    hk_actor::k_actor_mlp_noisy<<<grid, hk_actor::kThreads, hk_actor::kSmemBytes, (cudaStream_t)stream>>>(
+        (const unsigned char*)params_dev, obs_dev, act_dev, act_stride, (long long)n, seed, counter_dev, sigma, effectiveClip(clip),
+        (long long)row0);
+  } else {
+    static bool configured[64] = {false};
+    if (int rc = actorConfigure((const void*)hk_actor::k_actor_mlp, configured, device)) return rc;
+    hk_actor::k_actor_mlp<<<grid, hk_actor::kThreads, hk_actor::kSmemBytes, (cudaStream_t)stream>>>(
+        (const unsigned char*)params_dev, obs_dev, act_dev, act_stride, (long long)n);
+  }
   HK_CUDA(cudaGetLastError());
   return HK_OK;
+}
+
+int hk_actor_forward(const void* params_dev, const float* obs_dev, float* act_dev, int act_stride, int64_t n, int device, void* stream) {
+  const char* who = "hk_actor_forward";
+  if (int rc = actorCheck(who, params_dev, obs_dev, act_dev, act_stride, n)) return rc;
+  if (int rc = deviceCheck(who, device)) return rc;
+  return actorLaunch(params_dev, obs_dev, act_dev, act_stride, n, false, 0, nullptr, 0.0f, 0.0f, 0, device, stream);
+}
+
+int hk_actor_forward_noisy(const void* params_dev, const float* obs_dev, float* act_dev, int act_stride, int64_t n, uint64_t seed,
+                           const uint64_t* counter_dev, float sigma, float clip, int64_t row0, int device, void* stream) {
+  const char* who = "hk_actor_forward_noisy";
+  if (int rc = actorCheck(who, params_dev, obs_dev, act_dev, act_stride, n)) return rc;
+  if (int rc = noiseCheck(who, counter_dev, sigma, clip, row0)) return rc;
+  if (int rc = deviceCheck(who, device)) return rc;
+  return actorLaunch(params_dev, obs_dev, act_dev, act_stride, n, true, seed, counter_dev, sigma, clip, row0, device, stream);
 }
 
 int64_t hk_actor_pool_scratch_bytes(int64_t n, int k) {
@@ -1972,26 +2030,30 @@ int64_t hk_actor_pool_scratch_bytes(int64_t n, int k) {
   return 4 * hk_actor::poolScratchWords(n, k);
 }
 
-int hk_actor_forward_pool(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev,
-                          int act_stride, int64_t n, void* scratch_dev, int device, void* stream) {
+static int poolCheck(const char* who, const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev,
+                     int act_stride, int64_t n, void* scratch_dev) {
   using namespace hk_actor;
-  if (!params_dev || !choice_dev || !obs_dev || !act_dev || !scratch_dev) return fail(HK_E_INVALID, "hk_actor_forward_pool: NULL argument");
+  if (!params_dev || !choice_dev || !obs_dev || !act_dev || !scratch_dev) return fail(HK_E_INVALID, std::string(who) + ": NULL argument");
   if (n <= 0 || n > INT32_MAX || act_stride < kAct)
-    return fail(HK_E_INVALID, "hk_actor_forward_pool: n must be in [1, 2^31 - 1] and act_stride >= 4");
-  if (k < 1 || k > kPoolMaxK) return fail(HK_E_INVALID, "hk_actor_forward_pool: k must be in [1, 4096]");
+    return fail(HK_E_INVALID, std::string(who) + ": n must be in [1, 2^31 - 1] and act_stride >= 4");
+  if (k < 1 || k > kPoolMaxK) return fail(HK_E_INVALID, std::string(who) + ": k must be in [1, 4096]");
   if ((((uintptr_t)params_dev) & 15u) || (((uintptr_t)obs_dev) & 7u) || (((uintptr_t)choice_dev) & 3u) || (((uintptr_t)scratch_dev) & 15u))
-    return fail(HK_E_INVALID, "hk_actor_forward_pool: params and scratch need 16-byte, obs 8-byte, choice 4-byte alignment");
-  int count = 0;
-  if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) return fail(HK_E_NODEVICE, "hk_actor_forward_pool: no CUDA device (there is no CPU fallback)");
-  if (device < 0 || device >= count) return fail(HK_E_INVALID, "hk_actor_forward_pool: bad device index");
+    return fail(HK_E_INVALID, std::string(who) + ": params and scratch need 16-byte, obs 8-byte, choice 4-byte alignment");
+  return HK_OK;
+}
+
+// The grouping kernels, then the pooled tensor-core kernel; sigma == 0 runs the plain one (bit-identical to
+// hk_actor_forward_pool).
+static int poolLaunch(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev, int act_stride,
+                      int64_t n, void* scratch_dev, bool noisy, uint64_t seed, const uint64_t* counter_dev, float sigma, float clip,
+                      int64_t row0, int device, void* stream) {
+  using namespace hk_actor;
   DeviceGuard guard(device);
-  static bool configured[64] = {false};
-  if (!configured[device & 63]) {
-    HK_CUDA(cudaFuncSetAttribute(k_actor_pool_mlp, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    configured[device & 63] = true;
-  }
-  int sms = 148;
-  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sms < 1) sms = 148;
+  const bool withNoise = noisy && sigma != 0.0f;
+  static bool configured[64] = {false}, configuredNoisy[64] = {false};
+  if (int rc = withNoise ? actorConfigure((const void*)k_actor_pool_mlp_noisy, configuredNoisy, device) : actorConfigure((const void*)k_actor_pool_mlp, configured, device))
+    return rc;
+  const int sms = actorSms(device);
   cudaStream_t st = (cudaStream_t)stream;
   int32_t* scratch = (int32_t*)scratch_dev;
   HK_CUDA(cudaMemsetAsync(scratch, 0, sizeof(int32_t) * (size_t)k, st));  // counts
@@ -2002,7 +2064,46 @@ int hk_actor_forward_pool(const void* params_dev, int k, const int32_t* choice_d
   k_pool_scatter<<<histBlocks, kPoolThreads, 2 * sizeof(int32_t) * (size_t)k, st>>>(choice_dev, (long long)n, k, scratch);
   // the tile count is only known on the device: at most ceil(n / 128) + k - 1 tiles (one partial tile per group)
   const int64_t grid = std::min<int64_t>(sms, (n + kRows - 1) / kRows + k);
-  k_actor_pool_mlp<<<(unsigned)grid, kThreads, kSmemBytes, st>>>((const unsigned char*)params_dev, k, scratch, obs_dev, act_dev, act_stride);
+  if (withNoise)
+    k_actor_pool_mlp_noisy<<<(unsigned)grid, kThreads, kSmemBytes, st>>>((const unsigned char*)params_dev, k, scratch, obs_dev, act_dev,
+                                                                         act_stride, seed, counter_dev, sigma, effectiveClip(clip), (long long)row0);
+  else
+    k_actor_pool_mlp<<<(unsigned)grid, kThreads, kSmemBytes, st>>>((const unsigned char*)params_dev, k, scratch, obs_dev, act_dev, act_stride);
+  HK_CUDA(cudaGetLastError());
+  return HK_OK;
+}
+
+int hk_actor_forward_pool(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev,
+                          int act_stride, int64_t n, void* scratch_dev, int device, void* stream) {
+  const char* who = "hk_actor_forward_pool";
+  if (int rc = poolCheck(who, params_dev, k, choice_dev, obs_dev, act_dev, act_stride, n, scratch_dev)) return rc;
+  if (int rc = deviceCheck(who, device)) return rc;
+  return poolLaunch(params_dev, k, choice_dev, obs_dev, act_dev, act_stride, n, scratch_dev, false, 0, nullptr, 0.0f, 0.0f, 0, device, stream);
+}
+
+int hk_actor_forward_pool_noisy(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev,
+                                int act_stride, int64_t n, void* scratch_dev, uint64_t seed, const uint64_t* counter_dev, float sigma,
+                                float clip, int64_t row0, int device, void* stream) {
+  const char* who = "hk_actor_forward_pool_noisy";
+  if (int rc = poolCheck(who, params_dev, k, choice_dev, obs_dev, act_dev, act_stride, n, scratch_dev)) return rc;
+  if (int rc = noiseCheck(who, counter_dev, sigma, clip, row0)) return rc;
+  if (int rc = deviceCheck(who, device)) return rc;
+  return poolLaunch(params_dev, k, choice_dev, obs_dev, act_dev, act_stride, n, scratch_dev, true, seed, counter_dev, sigma, clip, row0,
+                    device, stream);
+}
+
+int hk_actor_pack(const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3, void* params_dev,
+                  int device, void* stream) {
+  const char* who = "hk_actor_pack";
+  if (!w1 || !b1 || !w2 || !b2 || !w3 || !b3 || !params_dev) return fail(HK_E_INVALID, std::string(who) + ": NULL argument");
+  if (((uintptr_t)params_dev) & 15u) return fail(HK_E_INVALID, std::string(who) + ": params need 16-byte alignment");
+  if ((((uintptr_t)w1) | ((uintptr_t)b1) | ((uintptr_t)w2) | ((uintptr_t)b2) | ((uintptr_t)w3) | ((uintptr_t)b3)) & 3u)
+    return fail(HK_E_INVALID, std::string(who) + ": weights and biases need 4-byte alignment");
+  if (int rc = deviceCheck(who, device)) return rc;
+  DeviceGuard guard(device);
+  using namespace hk_actor;
+  k_actor_pack<<<(kParamWords + kPackThreads - 1) / kPackThreads, kPackThreads, 0, (cudaStream_t)stream>>>(w1, b1, w2, b2, w3, b3,
+                                                                                                          (uint32_t*)params_dev);
   HK_CUDA(cudaGetLastError());
   return HK_OK;
 }

@@ -319,6 +319,6 @@ HK_HD double u53(uint32_t hi, uint32_t lo) {
   return ((double)(hi >> 5) * 67108864.0 + (double)(lo >> 6)) * (1.0 / 9007199254740992.0);
 }
 HK_HD float u_pm1(uint32_t x) { return (float)(x >> 8) * (1.0f / 8388608.0f) - 1.0f; }
-enum { HK_STREAM_RESET = 0, HK_STREAM_OPP = 1, HK_STREAM_ACT = 2, HK_STREAM_PHASE0 = 3 };
+enum { HK_STREAM_RESET = 0, HK_STREAM_OPP = 1, HK_STREAM_ACT = 2, HK_STREAM_PHASE0 = 3, HK_STREAM_ACTOR_NOISE = 4 };  // 4: hk_actor.cuh NoiseKey
 
 }  // namespace hk

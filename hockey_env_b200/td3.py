@@ -129,6 +129,8 @@ class DeviceTD3Learner:
         self.train_step = 0
         self.gen = torch.Generator(device=self.device)
         self.gen.manual_seed(seed)
+        self.seed = seed
+        self.fused_actor = None  # train(..., fused=True): the FusedActor mirror of `actor` that acts in the env
 
     @torch.no_grad()
     def compute_target(self, next_state, reward, done):
@@ -199,24 +201,43 @@ def _explore(actor, obs, noise_scale, gen):
     return (a + torch.randn(a.shape, device=a.device, generator=gen) * noise_scale).clamp(-1, 1)
 
 
-def train(env_or_pool, learner, ticks, updates_per_tick=1, noise_scale=None, warmup_ticks=8):
+def train(env_or_pool, learner, ticks, updates_per_tick=1, noise_scale=None, warmup_ticks=8, fused=False):
     """Batched form of TD3Trainer's loop (rl/training/train.py:135-172): every tick all envs act with Gaussian
     exploration noise, their transitions (terminal observation as next_obs on done) go to the learner's device replay
-    buffer, and `updates_per_tick` learner steps follow.  Returns the mean critic loss of the last tick (device scalar)."""
+    buffer, and `updates_per_tick` learner steps follow.  Returns the mean critic loss of the last tick (device scalar).
+
+    fused=True: the envs act through `learner.fused_actor`, a `FusedActor` mirror of `learner.actor` (created on first
+    use, seeded with the learner's seed), with the exploration noise drawn in the kernel: one launch per tick.  The
+    mirror is repacked on the device (`FusedActor.refresh`: no host sync) at the start of the call and after every tick
+    whose updates changed the actor, so every tick acts with the current weights.  The learner itself still trains the
+    fp32 module; only the behaviour policy runs in bf16 / TF32 (TD3 is off-policy)."""
+    from .actor import FusedActor
     from .training import OpponentPool
     pool = env_or_pool if isinstance(env_or_pool, OpponentPool) else None
     env = pool.env if pool else env_or_pool
     buf = learner.replay_buffer
     scale = learner.cfg.action_noise_scale if noise_scale is None else noise_scale
+    mirror = None
+    if fused:
+        if learner.fused_actor is None:
+            learner.fused_actor = FusedActor(learner.actor, device=learner.device, seed=learner.seed)
+        mirror = learner.fused_actor.refresh(learner.actor)
     obs = env.obs.clone()
     loss = None
     for t in range(ticks):
-        a = _explore(learner.actor, obs, scale, learner.gen)
+        if mirror is not None:
+            a = mirror(obs, noise=scale)
+        else:
+            a = _explore(learner.actor, obs, scale, learner.gen)
         nobs, reward, done, _, _ = pool.step(a) if pool else env.step(a.contiguous())
         nxt = torch.where(done.to(torch.bool).unsqueeze(1), env.final_obs, nobs) if env.final_obs is not None else nobs
         buf.push(obs, a, reward, nxt, done)
         obs = nobs.clone()
         if t >= warmup_ticks:
+            changed = False
             for _ in range(updates_per_tick):
-                _, loss = learner.update_from_buffer()
+                actor_loss, loss = learner.update_from_buffer()
+                changed |= actor_loss is not None
+            if changed and mirror is not None:
+                mirror.refresh(learner.actor)
     return loss

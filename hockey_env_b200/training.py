@@ -20,7 +20,7 @@ The dense networks are plain torch modules (library matmuls): they are the ops n
 import torch
 
 from . import _lib
-from .actor import FusedActorPool
+from .actor import FusedActor, FusedActorPool
 from .env import HockeyVecEnv, Mode
 
 
@@ -215,15 +215,28 @@ class DeviceReplayBuffer:
         return self.obs[idx], self.action[idx], self.reward[idx], self.next_obs[idx], self.done[idx]
 
 
+def behaviour_actions(actor, obs, noise=0.0):
+    """The behaviour policy of one tick: actor(obs), plus Gaussian exploration noise of std `noise` clamped to [-1, 1]
+    when noise > 0.  A `FusedActor` draws the noise in its kernel epilogue (one launch); any other module runs, then
+    torch's randn / add / clamp."""
+    if not noise:
+        return actor(obs)
+    if isinstance(actor, FusedActor):
+        return actor(obs, noise=noise)
+    a = actor(obs)
+    return (a + torch.randn(a.shape, device=a.device) * noise).clamp(-1, 1)
+
+
 @torch.no_grad()
-def collect(pool_or_env, actor, buffer, steps):
-    """`steps` ticks of experience collection: actor -> env -> buffer, all on the device.  With auto-reset the
-    transition of a finished episode stores the TERMINAL observation (`final_obs`) as next_obs, as the reference's
+def collect(pool_or_env, actor, buffer, steps, noise=0.0):
+    """`steps` ticks of experience collection: actor -> env -> buffer, all on the device.  `actor` is a module or a
+    `FusedActor`; `noise` > 0 adds Gaussian exploration noise of that std (see `behaviour_actions`).  With auto-reset
+    the transition of a finished episode stores the TERMINAL observation (`final_obs`) as next_obs, as the reference's
     loop does (rl/training/train.py:136-160)."""
     env = pool_or_env.env if isinstance(pool_or_env, OpponentPool) else pool_or_env
     obs = env.obs.clone()
     for _ in range(steps):
-        a1 = actor(obs)
+        a1 = behaviour_actions(actor, obs, noise)
         nobs, reward, done, _, _ = pool_or_env.step(a1) if isinstance(pool_or_env, OpponentPool) else env.step(a1.contiguous())
         nxt = torch.where(done.to(torch.bool).unsqueeze(1), env.final_obs, nobs) if env.final_obs is not None else nobs
         buffer.push(obs, a1, reward, nxt, done)

@@ -234,6 +234,29 @@ int64_t hk_actor_pool_scratch_bytes(int64_t n, int k);
 int hk_actor_forward_pool(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev,
                           int act_stride, int64_t n, void* scratch_dev, int device, void* stream);
 
+/* The same two kernels with Gaussian noise in the output epilogue (TD3 exploration, target-policy smoothing):
+ * act[i] = clamp(tanh(MLP(obs[i])) + c(sigma * z_i), -1, 1), c = clip to [-clip, clip] (clip <= 0 or +inf: no clip).
+ * z_i: four standard normals from one Philox4x32-10 call keyed on (seed, row0 + i, *counter_dev) and Box-Muller; the
+ * exact key and uniform mapping are in csrc/hk_actor.cuh (NoiseKey).  Row i's noise depends only on that key (not on n,
+ * tile order or pool grouping); row0 lets the shards of one batch agree.  counter_dev: one u64 in device memory (8-byte
+ * aligned) read by the kernel, so a captured graph draws fresh noise on each replay if the caller advances it.
+ * sigma must be finite and >= 0; sigma == 0 gives output bit-identical to hk_actor_forward / hk_actor_forward_pool.
+ * Other arguments and error rules as for those two; row0 >= 0.  Enqueued on `stream`; graph-capturable. */
+int hk_actor_forward_noisy(const void* params_dev, const float* obs_dev, float* act_dev, int act_stride, int64_t n, uint64_t seed,
+                           const uint64_t* counter_dev, float sigma, float clip, int64_t row0, int device, void* stream);
+int hk_actor_forward_pool_noisy(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev,
+                                int act_stride, int64_t n, void* scratch_dev, uint64_t seed, const uint64_t* counter_dev, float sigma,
+                                float clip, int64_t row0, int device, void* stream);
+
+/* Pack an ActorNetwork's fp32 parameters on the device into one hk_actor_param_bytes() block, byte-identical to
+ * hockey_env_b200.actor.FusedActor.pack: w1 [256, 18], b1 [256], w2 [256, 256], b2 [256], w3 [4, 256], b3 [4], contiguous
+ * f32 device arrays (4-byte aligned).  params_dev: 16-byte aligned; may point into a pool table (slot s at
+ * s * hk_actor_param_bytes()) to refresh one snapshot in place.  One small kernel on `stream`, no host synchronisation;
+ * graph-capturable.  Invalid arguments return HK_E_INVALID (before any device probe); valid ones without a GPU
+ * HK_E_NODEVICE. */
+int hk_actor_pack(const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
+                  void* params_dev, int device, void* stream);
+
 /* Measurement: per-kernel device times of the ticks that follow.  hk_kernel_timing(env, 1) makes every hk_step /
  * hk_rollout tick record CUDA events on the launching stream around each kernel of the cascade (up to 2048 ticks; not
  * graph-capturable while enabled); hk_kernel_times synchronises the device, returns the summed milliseconds of
