@@ -20,6 +20,7 @@
 #include "hk_tick.cuh"
 #if !defined(HK_TU_INLINE)
 #include "hk_actor.cuh"
+#include "hk_td3.cuh"
 #endif
 
 using namespace hk;
@@ -2105,6 +2106,111 @@ int hk_actor_pack(const float* w1, const float* b1, const float* w2, const float
   k_actor_pack<<<(kParamWords + kPackThreads - 1) / kPackThreads, kPackThreads, 0, (cudaStream_t)stream>>>(w1, b1, w2, b2, w3, b3,
                                                                                                           (uint32_t*)params_dev);
   HK_CUDA(cudaGetLastError());
+  return HK_OK;
+}
+
+int64_t hk_td3_arena_bytes(void) { return 4 * hk_td3::kArenaFloats; }
+
+int64_t hk_td3_scratch_bytes(int batch) {
+  if (batch < 1 || batch > hk_td3::kMaxBatch) return fail(HK_E_INVALID, "hk_td3_scratch_bytes: batch must be in [1, 1024]");
+  return 4 * hk_td3::carve(nullptr, batch).floats;
+}
+
+// The cluster size of k_td3_update on `device`: 16 CTAs (non-portable) when the device can co-schedule such a cluster,
+// else the portable 8.  The result does not depend on it (csrc/hk_td3.cuh).
+static int td3Cluster(int device) {
+  static int size[64] = {0};
+  int& s = size[device & 63];
+  if (s == 0) {
+    const void* k = (const void*)hk_td3::k_td3_update;
+    s = 8;
+    if (cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess) {
+      cudaLaunchConfig_t cfg = {};
+      cudaLaunchAttribute attr;
+      attr.id = cudaLaunchAttributeClusterDimension;
+      attr.val.clusterDim.x = hk_td3::kClusterMax;
+      attr.val.clusterDim.y = attr.val.clusterDim.z = 1;
+      cfg.gridDim = dim3(hk_td3::kClusterMax);
+      cfg.blockDim = dim3(hk_td3::kThreads);
+      cfg.attrs = &attr;
+      cfg.numAttrs = 1;
+      int clusters = 0;
+      if (cudaOccupancyMaxActiveClusters(&clusters, k, &cfg) == cudaSuccess && clusters >= 1) s = hk_td3::kClusterMax;
+    }
+    cudaGetLastError();  // a refused probe leaves no sticky error
+  }
+  return s;
+}
+
+static bool finiteNonNeg(float x) { return x >= 0.0f && !std::isinf(x); }
+
+int hk_td3_update(void* arena_dev, void* scratch_dev, const hk_td3_batch* batch, int batch_size, const hk_td3_hparams* hp,
+                  const float* action_low_dev, const float* action_range_dev, uint64_t seed, int do_actor, float* losses_dev,
+                  int device, void* stream) {
+  const std::string who = "hk_td3_update";
+  if (!arena_dev || !scratch_dev || !batch || !hp || !action_low_dev || !action_range_dev || !losses_dev)
+    return fail(HK_E_INVALID, who + ": NULL argument");
+  if (!batch->obs || !batch->action || !batch->reward || !batch->next_obs || !batch->done || !batch->idx)
+    return fail(HK_E_INVALID, who + ": NULL batch array");
+  if (batch->prio_weights && !batch->prio_idx) return fail(HK_E_INVALID, who + ": NULL prio_idx with prio_weights");
+  if ((((uintptr_t)arena_dev) & 15u) || (((uintptr_t)scratch_dev) & 15u))
+    return fail(HK_E_INVALID, who + ": arena and scratch need 16-byte alignment");
+  if ((((uintptr_t)batch->idx) & 7u) || (batch->prio_weights && (((uintptr_t)batch->prio_idx) & 7u)))
+    return fail(HK_E_INVALID, who + ": idx and prio_idx need 8-byte alignment");
+  if ((((uintptr_t)batch->obs) | ((uintptr_t)batch->action) | ((uintptr_t)batch->reward) | ((uintptr_t)batch->next_obs) |
+       ((uintptr_t)batch->done) | ((uintptr_t)batch->prio_weights) | ((uintptr_t)action_low_dev) | ((uintptr_t)action_range_dev) |
+       ((uintptr_t)losses_dev)) & 3u)
+    return fail(HK_E_INVALID, who + ": float arrays need 4-byte alignment");
+  if (batch_size < 1 || batch_size > hk_td3::kMaxBatch) return fail(HK_E_INVALID, who + ": batch must be in [1, 1024]");
+  const float hv[10] = {hp->gamma, hp->tau_actor, hp->tau_critic, hp->lr_actor, hp->lr_critic, hp->wd_actor, hp->wd_critic,
+                        hp->beta, hp->target_noise, hp->target_noise_clip};
+  const char* hn[10] = {"gamma", "tau_actor", "tau_critic", "lr_actor", "lr_critic", "wd_actor", "wd_critic", "beta",
+                        "target_noise", "target_noise_clip"};
+  for (int i = 0; i < 10; ++i)
+    if (!finiteNonNeg(hv[i])) return fail(HK_E_INVALID, who + ": " + hn[i] + " must be finite and >= 0");
+  if (batch->prio_weights && batch->prio_n < 1) return fail(HK_E_INVALID, who + ": prio_n must be >= 1");
+  if (int rc = deviceCheck(who.c_str(), device)) return rc;
+  DeviceGuard guard(device);
+  hk_td3::Args a;
+  a.arena = (float*)arena_dev;
+  a.scratch = (float*)scratch_dev;
+  a.obs = batch->obs;
+  a.act = batch->action;
+  a.rew = batch->reward;
+  a.nobs = batch->next_obs;
+  a.done = batch->done;
+  a.idx = (const long long*)batch->idx;
+  a.pw = batch->prio_weights;
+  a.pidx = (const long long*)batch->prio_idx;
+  a.pn = (long long)batch->prio_n;
+  a.alow = action_low_dev;
+  a.arange = action_range_dev;
+  a.losses = losses_dev;
+  a.seed = seed;
+  a.B = batch_size;
+  a.doActor = do_actor ? 1 : 0;
+  a.gamma = hp->gamma;
+  a.tauA = hp->tau_actor;
+  a.tauC = hp->tau_critic;
+  a.lrA = hp->lr_actor;
+  a.lrC = hp->lr_critic;
+  a.wdA = hp->wd_actor;
+  a.wdC = hp->wd_critic;
+  a.beta = hp->beta;
+  a.sigma = hp->target_noise;
+  a.clip = hp->target_noise_clip;
+  const int cluster = td3Cluster(device);
+  cudaLaunchConfig_t cfg = {};
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeClusterDimension;
+  attr.val.clusterDim.x = (unsigned)cluster;
+  attr.val.clusterDim.y = attr.val.clusterDim.z = 1;
+  cfg.gridDim = dim3((unsigned)cluster);
+  cfg.blockDim = dim3(hk_td3::kThreads);
+  cfg.stream = (cudaStream_t)stream;
+  cfg.attrs = &attr;
+  cfg.numAttrs = 1;
+  HK_CUDA(cudaLaunchKernelEx(&cfg, hk_td3::k_td3_update, a));
   return HK_OK;
 }
 

@@ -7,6 +7,7 @@ learner consumes the sampled tensors in place.  Same algorithm, same hyper-param
 are plain torch modules (library GEMMs + autograd): they are the dense ops next to the env path, not the path.
 """
 import copy
+import math
 from dataclasses import dataclass
 
 import torch
@@ -92,11 +93,16 @@ class DevicePrioritizedReplayBuffer(DeviceReplayBuffer):
         idx = (start + torch.arange(n, device=self.device)) % self.capacity
         self.weights[idx] = top
 
-    def sample(self, batch_size):
+    def sample_indices(self, batch_size):
+        """Draw min(batch_size, len) indices proportionally to the weights; they become `last_batch_inds`."""
         batch_size = min(int(batch_size), self.size)
         w = torch.nan_to_num(self.weights[:self.size], nan=0.0, posinf=0.0, neginf=0.0).clamp_min(1e-6)
         idx = torch.multinomial(w / w.sum(), batch_size, replacement=True, generator=self.gen)
         self.last_batch_inds = idx
+        return idx
+
+    def sample(self, batch_size):
+        idx = self.sample_indices(batch_size)
         return self.obs[idx], self.action[idx], self.reward[idx], self.next_obs[idx], self.done[idx]
 
     def get_last_probs(self):
@@ -193,6 +199,150 @@ class DeviceTD3Learner:
         self.critic.load_state_dict(ckpt["critic"])
         self.target_actor.load_state_dict(ckpt["target_policy"])
         self.target_critic.load_state_dict(ckpt["target_critic"])
+
+
+_ACTOR_SHAPES = {"fc1.weight": (256, 18), "fc1.bias": (256,), "fc2.weight": (256, 256), "fc2.bias": (256,),
+                 "fc3.weight": (4, 256), "fc3.bias": (4,)}
+_HEAD_SHAPES = {"fc1.weight": (256, 22), "fc1.bias": (256,), "fc2.weight": (256, 256), "fc2.bias": (256,),
+                "fc3.weight": (1, 256), "fc3.bias": (1,)}
+_CRITIC_SHAPES = {f"{h}.{k}": v for h in ("q1", "q2") for k, v in _HEAD_SHAPES.items()}
+
+
+def _pad64(n):
+    return (n + 63) // 64 * 64
+
+
+class FusedTD3Learner(DeviceTD3Learner):
+    """`DeviceTD3Learner.update` as ONE sm_100a kernel launch per update (csrc/hk_td3.cuh, hk_td3_update): the batch
+    gather, the target policy with clipped smoothing noise, the twin-critic step with Adam, prioritized importance
+    weights and priority write-back, and on actor steps the actor step and the Polyak updates.  No host sync, no
+    allocation in the kernel call; graph-capturable.  fp32 throughout with fixed summation orders: bit-reproducible run
+    to run, and equal to the torch learner up to fp32 rounding (not bit for bit).
+
+    Every parameter of actor, critic, target_actor and target_critic is re-homed into a view of one device arena, so the
+    modules, `state_dict()` / `load_state_dict()` (the reference's checkpoint format, interchangeable with
+    `DeviceTD3Learner`) and `FusedActor.refresh(learner.actor)` work on the live weights.  The Adam state lives in the
+    arena as well, with its step counts as device int64: `actor_optimizer` / `critic_optimizer` exist but are never
+    stepped, and checkpoints carry no optimizer state, as in the reference.  The target-policy noise is Philox keyed on
+    (seed, batch row, a device counter that every update advances), not torch's generator; the replay indices still come
+    from the buffer's generator (`sample_indices`), so a fused and a torch learner on equal buffers train on the same
+    batches.  Only the reference architecture is supported (actor 18-256-256-4, critic 22-256-256-1), on CUDA."""
+
+    MAX_BATCH = 1024
+
+    def __init__(self, actor=None, critic=None, config=None, replay_buffer=None, device="cuda:0", seed=0):
+        import ctypes as C
+        from . import _lib
+        from .actor import _cuda_device
+        super().__init__(actor, critic, config, replay_buffer, device, seed)
+        self.device = _cuda_device(self.device, "FusedTD3Learner")
+        self._C, self._lib = C, _lib
+        self.L = _lib.load()
+        for net, shapes, who in ((self.actor, _ACTOR_SHAPES, "actor"), (self.critic, _CRITIC_SHAPES, "critic")):
+            got = {k: tuple(v.shape) for k, v in net.named_parameters()}
+            if got != shapes:
+                raise ValueError(f"FusedTD3Learner implements the reference architecture only (actor 18-256-256-4, twin "
+                                 f"critic 22-256-256-1); the {who} has parameters {got}")
+        blocks, ctr_off, nbytes = self.arena_layout()
+        if nbytes != int(self.L.hk_td3_arena_bytes()):
+            raise _lib.HockeyLibraryError("FusedTD3Learner: the library's arena size does not match this package")
+        self.arena = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
+        f = self.arena.view(torch.float32)
+        self.blocks = {name: f[o:o + n] for name, (o, n) in blocks.items()}  # flat fp32 views, parameters in state_dict order
+        self.counters = self.arena[4 * ctr_off:4 * ctr_off + 24].view(torch.int64)  # critic step, actor step, noise counter
+        for name, net in (("actor", self.actor), ("critic", self.critic), ("target_actor", self.target_actor),
+                          ("target_critic", self.target_critic)):
+            blk, o = self.blocks[name], 0
+            with torch.no_grad():
+                for p in net.parameters():  # state_dict order without the critic's buffers
+                    view = blk[o:o + p.numel()].view(p.shape)
+                    view.copy_(p.detach().to(torch.float32))
+                    p.data = view
+                    o += p.numel()
+        self._losses = None
+        self._scratch, self._scratch_b = None, 0
+        self._arange = None
+        self._hp = _lib.TD3HParams()
+
+    @staticmethod
+    def arena_layout():
+        """The arena of include/hockey_b200.h (hk_td3_update): ({block: (float offset, floats)}, float offset of the three
+        int64 counters, bytes).  Blocks start at multiples of 64 floats."""
+        pa = sum(math.prod(s) for s in _ACTOR_SHAPES.values())
+        pc = sum(math.prod(s) for s in _CRITIC_SHAPES.values())
+        blocks, off = {}, 0
+        for name, n in (("actor", pa), ("critic", pc), ("target_actor", pa), ("target_critic", pc), ("m_actor", pa),
+                        ("v_actor", pa), ("m_critic", pc), ("v_critic", pc)):
+            blocks[name] = (off, n)
+            off += _pad64(n)
+        return blocks, off, 4 * (off + 64)
+
+    def _hparams(self):
+        c, hp = self.cfg, self._hp
+        for k, v in (("gamma", c.gamma), ("tau_actor", c.tau_actor), ("tau_critic", c.tau_critic), ("lr_actor", c.lr_pol),
+                     ("lr_critic", c.lr_q), ("wd_actor", c.wd_pol), ("wd_critic", c.wd_q), ("beta", c.beta),
+                     ("target_noise", c.target_action_noise_scale), ("target_noise_clip", c.target_action_noise_clip)):
+            setattr(hp, k, float(v))
+        return hp
+
+    def _launch(self, arrays, idx, prio):
+        """One hk_td3_update on the current stream; arrays = (obs, action, reward, next_obs, done) base tensors, idx their
+        int64 rows, prio = (weights, weight indices, N) or None."""
+        C = self._C
+        b = idx.shape[0]
+        if not 1 <= b <= self.MAX_BATCH:
+            raise ValueError(f"FusedTD3Learner: batch size must be in [1, {self.MAX_BATCH}], got {b}")
+        if self._scratch is None or self._scratch_b < b:
+            self._scratch = torch.empty(int(self.L.hk_td3_scratch_bytes(b)), dtype=torch.uint8, device=self.device)
+            self._scratch_b = b
+        self.train_step += 1
+        do_actor = self.train_step % self.cfg.policy_update_freq == 0
+        losses = torch.empty(2, dtype=torch.float32, device=self.device)
+        batch = self._lib.TD3Batch(*[t.data_ptr() for t in arrays], idx.data_ptr())
+        if prio is not None:
+            batch.prio_weights, batch.prio_idx, batch.prio_n = prio[0].data_ptr(), prio[1].data_ptr(), int(prio[2])
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            self._lib.check(self.L.hk_td3_update(
+                C.c_void_p(self.arena.data_ptr()), C.c_void_p(self._scratch.data_ptr()), C.byref(batch), b, C.byref(self._hparams()),
+                C.c_void_p(self.critic.action_low.data_ptr()), C.c_void_p(self.critic.action_range.data_ptr()),
+                self.seed & (2**64 - 1), int(do_actor), C.c_void_p(losses.data_ptr()), self.device.index or 0, C.c_void_p(stream)))
+        self._last_batch = b
+        return (losses[0] if do_actor else None), losses[1]
+
+    def last_importance_weights(self):
+        """[B] importance weights the last update used (ones for a uniform batch), computed in the kernel."""
+        return self._scratch.view(torch.float32)[:self._last_batch]
+
+    @staticmethod
+    def _f32(t):
+        return t.detach().to(torch.float32).contiguous()
+
+    def update(self, state, action, reward, next_state, done):
+        """One learner step on a given batch, in one launch; returns (actor_loss or None, critic_loss) as device scalars.
+        With a prioritized buffer whose `last_batch_inds` are set (the batch came from its `sample`), the importance
+        weights and the priority write-back use those indices, as `DeviceTD3Learner.update` does."""
+        arrays = [self._f32(t) for t in (state, action, reward, next_state, done)]
+        b = arrays[0].shape[0]
+        if self._arange is None or self._arange.shape[0] < b:
+            self._arange = torch.arange(max(b, 1), dtype=torch.int64, device=self.device)
+        prio = None
+        if self.prioritized and self.replay_buffer.last_batch_inds is not None:
+            buf = self.replay_buffer
+            prio = (buf.weights, buf.last_batch_inds.to(torch.int64).contiguous(), buf.size)
+            buf.last_batch_inds = None
+        return self._launch(arrays, self._arange[:b], prio)
+
+    def update_from_buffer(self, batch_size=None):
+        """Draw the batch's indices from the replay buffer (`sample_indices`: the same draws as `sample`) and run one
+        update that gathers the rows in the kernel."""
+        buf = self.replay_buffer
+        idx = buf.sample_indices(batch_size or self.cfg.batch_size)
+        prio = None
+        if self.prioritized:
+            prio = (buf.weights, idx, buf.size)
+            buf.last_batch_inds = None
+        return self._launch((buf.obs, buf.action, buf.reward, buf.next_obs, buf.done), idx, prio)
 
 
 @torch.no_grad()

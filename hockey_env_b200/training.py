@@ -210,8 +210,12 @@ class DeviceReplayBuffer:
         self.pos = (self.pos + n) % self.capacity
         self.size = min(self.capacity, self.size + n)
 
+    def sample_indices(self, batch_size):
+        """The int64 row indices `sample` gathers (drawn from the buffer's generator): uniform over the stored rows."""
+        return torch.randint(0, self.size, (batch_size,), device=self.device, generator=self.gen)
+
     def sample(self, batch_size):
-        idx = torch.randint(0, self.size, (batch_size,), device=self.device, generator=self.gen)
+        idx = self.sample_indices(batch_size)
         return self.obs[idx], self.action[idx], self.reward[idx], self.next_obs[idx], self.done[idx]
 
 

@@ -257,6 +257,48 @@ int hk_actor_forward_pool_noisy(const void* params_dev, int k, const int32_t* ch
 int hk_actor_pack(const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3,
                   void* params_dev, int device, void* stream);
 
+/* One TD3 learner update (hockey_env_b200.td3.FusedTD3Learner) in ONE kernel launch: gather, target policy smoothing,
+ * twin-critic forward / backward / Adam, prioritized importance weights and priority write-back, and with do_actor the
+ * actor forward through the stepped Q1, actor backward / Adam and Polyak of both target nets.  Reference architecture
+ * only: actor 18-256-256-4, twin critic 22-256-256-1.  The numerics contract is stated in csrc/hk_td3.cuh.
+ *
+ * arena_dev: hk_td3_arena_bytes() bytes, 16-byte aligned, fp32 offsets (in floats):
+ *   actor params        0        (71,684: fc1.weight [256,18], fc1.bias, fc2.weight [256,256], fc2.bias, fc3.weight [4,256], fc3.bias)
+ *   critic params       71,744   (143,874: q1.fc1.weight [256,22], q1.fc1.bias, q1.fc2.*, q1.fc3.weight [1,256], q1.fc3.bias, q2.*)
+ *   target actor        215,680, target critic 287,424, Adam m / v of the actor 431,360 / 503,104,
+ *   Adam m / v of the critic 574,848 / 718,784,
+ *   counters            862,720  (int64: critic step, actor step, target-noise counter)
+ * Every net is in state_dict order, row-major as torch stores it; each block starts at a multiple of 64 floats.
+ * scratch_dev: hk_td3_scratch_bytes(batch) bytes, 16-byte aligned, contents need not be initialised; its first `batch`
+ * floats hold the batch's importance weights after the call.  One call at a time per arena and per scratch buffer.
+ * batch->idx: [batch] int64 rows of the replay arrays (each in [0, capacity): not checked).  batch->prio_weights: NULL for
+ * a uniform batch; otherwise the buffer's weights, indexed by batch->prio_idx, with N = prio_n >= 1.
+ * losses_dev: [2] floats, actor loss (written on actor steps only) and critic loss.
+ * Enqueued on `stream` with no host synchronisation and no allocation; graph-capturable.  Invalid arguments (NULL
+ * pointers, misalignment, batch outside [1, 1024], non-finite or negative lr / tau / gamma / sigma / clip / wd / beta,
+ * prio_n < 1) return HK_E_INVALID before any device probe; valid ones without a GPU HK_E_NODEVICE.
+ * hk_td3_scratch_bytes returns HK_E_INVALID for batch out of range. */
+typedef struct {
+  const float* obs;          /* [capacity, 18] */
+  const float* action;       /* [capacity, 4] */
+  const float* reward;       /* [capacity] */
+  const float* next_obs;     /* [capacity, 18] */
+  const float* done;         /* [capacity], 0 or 1 */
+  const int64_t* idx;        /* [batch], 8-byte aligned */
+  float* prio_weights;       /* NULL: uniform batch */
+  const int64_t* prio_idx;   /* [batch] (prioritized only) */
+  int64_t prio_n;            /* number of stored transitions (prioritized only) */
+} hk_td3_batch;
+typedef struct {
+  float gamma, tau_actor, tau_critic, lr_actor, lr_critic, wd_actor, wd_critic, beta;
+  float target_noise, target_noise_clip;
+} hk_td3_hparams;
+int64_t hk_td3_arena_bytes(void);
+int64_t hk_td3_scratch_bytes(int batch);
+int hk_td3_update(void* arena_dev, void* scratch_dev, const hk_td3_batch* batch, int batch_size, const hk_td3_hparams* hp,
+                  const float* action_low_dev, const float* action_range_dev, uint64_t seed, int do_actor, float* losses_dev,
+                  int device, void* stream);
+
 /* Measurement: per-kernel device times of the ticks that follow.  hk_kernel_timing(env, 1) makes every hk_step /
  * hk_rollout tick record CUDA events on the launching stream around each kernel of the cascade (up to 2048 ticks; not
  * graph-capturable while enabled); hk_kernel_times synchronises the device, returns the summed milliseconds of
