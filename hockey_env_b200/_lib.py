@@ -19,7 +19,7 @@ STEP_AUTORESET = 1
 EXPORTS = [
     "hk_create", "hk_destroy", "hk_num_envs", "hk_reset", "hk_reset_seeded", "hk_step", "hk_step_host", "hk_host_record_bytes", "hk_rollout", "hk_get_obs", "hk_get_info", "hk_get_state",
     "hk_set_state", "hk_set_obs_state", "hk_set_opponent_policies", "hk_set_reset_modes", "hk_get_modes", "hk_get_stats", "hk_clear_stats", "hk_stats_device_ptr", "hk_copy_stats", "hk_debug_phase_cycles", "hk_debug_finish_cycles", "hk_launches_per_step", "hk_debug_lane_trace", "hk_kernel_timing", "hk_kernel_times", "hk_actor_param_bytes", "hk_actor_forward", "hk_actor_pool_scratch_bytes", "hk_actor_forward_pool", "hk_actor_forward_noisy",
-    "hk_actor_forward_pool_noisy", "hk_actor_pack", "hk_td3_arena_bytes", "hk_td3_scratch_bytes", "hk_td3_update", "hk_last_error",
+    "hk_actor_forward_pool_noisy", "hk_actor_pack", "hk_td3_arena_bytes", "hk_td3_scratch_bytes", "hk_td3_update", "hk_td3_cluster_size", "hk_last_error",
     "hk_version",
 ]
 
@@ -116,6 +116,8 @@ def load():
     L.hk_td3_scratch_bytes.restype = i64
     L.hk_td3_update.argtypes = [vp, vp, C.POINTER(TD3Batch), i32, C.POINTER(TD3HParams), vp, vp, u64, i32, vp, i32, vp]
     L.hk_td3_update.restype = i32
+    L.hk_td3_cluster_size.argtypes = [i32]
+    L.hk_td3_cluster_size.restype = i32
     L.hk_launches_per_step.argtypes = [vp]
     L.hk_launches_per_step.restype = i32
     L.hk_get_state.argtypes = [vp, vp, vp]

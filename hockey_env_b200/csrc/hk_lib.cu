@@ -2117,9 +2117,14 @@ int64_t hk_td3_scratch_bytes(int batch) {
 }
 
 // The cluster size of k_td3_update on `device`: 16 CTAs (non-portable) when the device can co-schedule such a cluster,
-// else the portable 8.  The result does not depend on it (csrc/hk_td3.cuh).
+// else the portable 8.  The result does not depend on it (csrc/hk_td3.cuh).  HK_TD3_CLUSTER=n (read once) lowers the
+// size to n >= 1, so that the tests can run the update at other sizes; it never raises the probed size.
 static int td3Cluster(int device) {
   static int size[64] = {0};
+  static const int cap = [] {
+    const char* e = getenv("HK_TD3_CLUSTER");
+    return e ? atoi(e) : 0;
+  }();
   int& s = size[device & 63];
   if (s == 0) {
     const void* k = (const void*)hk_td3::k_td3_update;
@@ -2138,8 +2143,15 @@ static int td3Cluster(int device) {
       if (cudaOccupancyMaxActiveClusters(&clusters, k, &cfg) == cudaSuccess && clusters >= 1) s = hk_td3::kClusterMax;
     }
     cudaGetLastError();  // a refused probe leaves no sticky error
+    if (cap >= 1 && cap < s) s = cap;
   }
   return s;
+}
+
+int hk_td3_cluster_size(int device) {
+  if (int rc = deviceCheck("hk_td3_cluster_size", device)) return rc;
+  DeviceGuard guard(device);
+  return td3Cluster(device);
 }
 
 static bool finiteNonNeg(float x) { return x >= 0.0f && !std::isinf(x); }

@@ -28,7 +28,9 @@
 //    torch to fp32 rounding, not bit for bit.
 //  * Action normalisation: every critic forward applies TwinQNetwork's ((a - low) / range) * 2 - 1 from the critic's
 //    action_low / action_range buffers (skipped, like torch, when a range entry is infinite); the actor's backward pass
-//    multiplies the action gradient by 2 and divides it by range.
+//    multiplies the action gradient by 2 and divides it by range.  The target critic's forward uses the same (online)
+//    buffers, so the target critic must carry equal bounds: FusedTD3Learner rejects a critic / target critic pair whose
+//    buffers differ.
 //  * Target noise: a' = clamp(target_actor(s') + clip(sigma * z, -clip, clip), -1, 1), z = four normals per row from one
 //    Philox4x32-10 call hk::philox(seed, row, (uint32_t)ctr, HK_STREAM_TD3_TARGET | (uint32_t)(ctr >> 32) << 8) and
 //    Box-Muller exactly as hk_actor.cuh's NoiseKey (u1 = ((a >> 8) + 1) 2^-24, u2 = (b >> 8) 2^-24); ctr is the arena's

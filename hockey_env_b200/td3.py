@@ -226,7 +226,9 @@ class FusedTD3Learner(DeviceTD3Learner):
     stepped, and checkpoints carry no optimizer state, as in the reference.  The target-policy noise is Philox keyed on
     (seed, batch row, a device counter that every update advances), not torch's generator; the replay indices still come
     from the buffer's generator (`sample_indices`), so a fused and a torch learner on equal buffers train on the same
-    batches.  Only the reference architecture is supported (actor 18-256-256-4, critic 22-256-256-1), on CUDA."""
+    batches.  Only the reference architecture is supported (actor 18-256-256-4, critic 22-256-256-1), on CUDA.  The
+    kernel normalises both critics' actions with the critic's action bounds, so a checkpoint whose target critic carries
+    other action_low / action_range buffers is rejected with ValueError."""
 
     MAX_BATCH = 1024
 
@@ -243,6 +245,7 @@ class FusedTD3Learner(DeviceTD3Learner):
             if got != shapes:
                 raise ValueError(f"FusedTD3Learner implements the reference architecture only (actor 18-256-256-4, twin "
                                  f"critic 22-256-256-1); the {who} has parameters {got}")
+        self._check_action_bounds(self.critic.state_dict(), self.target_critic.state_dict())
         blocks, ctr_off, nbytes = self.arena_layout()
         if nbytes != int(self.L.hk_td3_arena_bytes()):
             raise _lib.HockeyLibraryError("FusedTD3Learner: the library's arena size does not match this package")
@@ -276,6 +279,19 @@ class FusedTD3Learner(DeviceTD3Learner):
             blocks[name] = (off, n)
             off += _pad64(n)
         return blocks, off, 4 * (off + 64)
+
+    @staticmethod
+    def _check_action_bounds(critic_sd, target_sd):
+        """The kernel normalises the target critic's actions with the critic's action_low / action_range buffers, so the
+        two critics must carry equal ones (DeviceTD3Learner would use the target critic's own)."""
+        for k in ("action_low", "action_range"):
+            if not torch.equal(critic_sd[k].detach().cpu(), target_sd[k].detach().cpu()):
+                raise ValueError(f"FusedTD3Learner: the critic's and the target critic's {k} differ "
+                                 f"({critic_sd[k].tolist()} vs {target_sd[k].tolist()}); the fused update uses the critic's")
+
+    def load_state_dict(self, ckpt):
+        self._check_action_bounds(ckpt["critic"], ckpt["target_critic"])
+        super().load_state_dict(ckpt)
 
     def _hparams(self):
         c, hp = self.cfg, self._hp

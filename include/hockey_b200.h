@@ -298,6 +298,10 @@ int64_t hk_td3_scratch_bytes(int batch);
 int hk_td3_update(void* arena_dev, void* scratch_dev, const hk_td3_batch* batch, int batch_size, const hk_td3_hparams* hp,
                   const float* action_low_dev, const float* action_range_dev, uint64_t seed, int do_actor, float* losses_dev,
                   int device, void* stream);
+/* The cluster size (CTAs) that hk_td3_update launches with on `device`: 16 when the device can co-schedule such a
+ * cluster, else 8, or lower when the environment variable HK_TD3_CLUSTER (read once per process) asks for a smaller
+ * size >= 1.  Results do not depend on it.  HK_E_NODEVICE without a GPU, HK_E_INVALID for a bad device index. */
+int hk_td3_cluster_size(int device);
 
 /* Measurement: per-kernel device times of the ticks that follow.  hk_kernel_timing(env, 1) makes every hk_step /
  * hk_rollout tick record CUDA events on the launching stream around each kernel of the cascade (up to 2048 ticks; not
