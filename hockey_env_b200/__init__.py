@@ -14,7 +14,10 @@ from .env import (  # noqa: F401
 from .vector import HockeyGymVectorEnv  # noqa: F401
 from .actor import ActorNetwork, FusedActor, FusedActorPool, actor_rollout, load_td3_actor  # noqa: F401
 from .training import DeviceReplayBuffer, OpponentPool, collect, cross_play, evaluate, evaluate_model  # noqa: F401
-from .td3 import DevicePrioritizedReplayBuffer, DeviceTD3Learner, FusedTD3Learner, TD3Config, TwinQNetwork  # noqa: F401
+from .td3 import (  # noqa: F401
+    DevicePrioritizedReplayBuffer, DeviceTD3Learner, FusedTD3Learner, FusedTD3Population, PopulationReplayBuffer, TD3Config,
+    TwinQNetwork, train_population,
+)
 
-__all__ = ["make", "make_vec", "spec", "REGISTRY", "OpponentPool", "DeviceReplayBuffer", "collect", "cross_play", "evaluate", "evaluate_model", "DevicePrioritizedReplayBuffer", "DeviceTD3Learner", "FusedTD3Learner", "TD3Config", "TwinQNetwork", "HockeyGymVectorEnv", "ActorNetwork", "FusedActor", "FusedActorPool", "actor_rollout", "load_td3_actor", "HockeyVecEnv", "HockeyEnv", "HockeyEnv_BasicOpponent", "BasicOpponent", "PolicyOpponent", "Mode",
+__all__ = ["make", "make_vec", "spec", "REGISTRY", "OpponentPool", "DeviceReplayBuffer", "collect", "cross_play", "evaluate", "evaluate_model", "DevicePrioritizedReplayBuffer", "DeviceTD3Learner", "FusedTD3Learner", "FusedTD3Population", "PopulationReplayBuffer", "train_population", "TD3Config", "TwinQNetwork", "HockeyGymVectorEnv", "ActorNetwork", "FusedActor", "FusedActorPool", "actor_rollout", "load_td3_actor", "HockeyVecEnv", "HockeyEnv", "HockeyEnv_BasicOpponent", "BasicOpponent", "PolicyOpponent", "Mode",
            "HockeyLibraryError", "load_library"]

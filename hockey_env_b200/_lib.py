@@ -13,13 +13,15 @@ OBS_DIM, ACT_DIM, INFO_DIM, STATS_DIM = 18, 4, 4, 16
 N_PAIRS, CONTACT_WORDS = 27, 8
 STATE_WORDS = 64 + N_PAIRS * CONTACT_WORDS
 HK_OK, HK_E_INVALID, HK_E_CUDA, HK_E_NODEVICE = 0, -1, -2, -3
+TD3_MAX_POPULATION = 64
 POLICY_EXTERNAL, POLICY_BASIC_WEAK, POLICY_BASIC_STRONG, POLICY_RANDOM, POLICY_ZERO, POLICY_PER_ENV = 0, 1, 2, 3, 4, 5
 STEP_AUTORESET = 1
 
 EXPORTS = [
     "hk_create", "hk_destroy", "hk_num_envs", "hk_reset", "hk_reset_seeded", "hk_step", "hk_step_host", "hk_host_record_bytes", "hk_rollout", "hk_get_obs", "hk_get_info", "hk_get_state",
     "hk_set_state", "hk_set_obs_state", "hk_set_opponent_policies", "hk_set_reset_modes", "hk_get_modes", "hk_get_stats", "hk_clear_stats", "hk_stats_device_ptr", "hk_copy_stats", "hk_debug_phase_cycles", "hk_debug_finish_cycles", "hk_launches_per_step", "hk_debug_lane_trace", "hk_kernel_timing", "hk_kernel_times", "hk_actor_param_bytes", "hk_actor_forward", "hk_actor_pool_scratch_bytes", "hk_actor_forward_pool", "hk_actor_forward_noisy",
-    "hk_actor_forward_pool_noisy", "hk_actor_pack", "hk_td3_arena_bytes", "hk_td3_scratch_bytes", "hk_td3_update", "hk_td3_cluster_size", "hk_last_error",
+    "hk_actor_forward_pool_noisy", "hk_actor_pack", "hk_td3_arena_bytes", "hk_td3_scratch_bytes", "hk_td3_update", "hk_td3_cluster_size",
+    "hk_td3_update_population", "hk_td3_population_cluster_size", "hk_actor_pack_many", "hk_last_error",
     "hk_version",
 ]
 
@@ -118,6 +120,12 @@ def load():
     L.hk_td3_update.restype = i32
     L.hk_td3_cluster_size.argtypes = [i32]
     L.hk_td3_cluster_size.restype = i32
+    L.hk_td3_update_population.argtypes = [vp, vp, C.POINTER(TD3Batch), i32, i32, C.POINTER(TD3HParams), vp, vp, vp, vp, vp, i32, vp]
+    L.hk_td3_update_population.restype = i32
+    L.hk_td3_population_cluster_size.argtypes = [i32, i32]
+    L.hk_td3_population_cluster_size.restype = i32
+    L.hk_actor_pack_many.argtypes = [vp, i64, i32, vp, i32, vp]
+    L.hk_actor_pack_many.restype = i32
     L.hk_launches_per_step.argtypes = [vp]
     L.hk_launches_per_step.restype = i32
     L.hk_get_state.argtypes = [vp, vp, vp]

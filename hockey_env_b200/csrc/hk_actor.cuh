@@ -544,12 +544,10 @@ __device__ __forceinline__ uint32_t packBf16Word(const float* __restrict__ w, in
   return bf16Bits(w[n * kDim + k]) | (bf16Bits(w[n * kDim + k + 1]) << 16);
 }
 
-__global__ void __launch_bounds__(kPackThreads) k_actor_pack(const float* __restrict__ w1, const float* __restrict__ b1,
-                                                             const float* __restrict__ w2, const float* __restrict__ b2,
-                                                             const float* __restrict__ w3, const float* __restrict__ b3,
-                                                             uint32_t* __restrict__ out) {
-  const int j = blockIdx.x * kPackThreads + threadIdx.x;
-  if (j >= kParamWords) return;
+// word j < kParamWords of the packed block of one actor
+__device__ __forceinline__ uint32_t packWord(const float* __restrict__ w1, const float* __restrict__ b1, const float* __restrict__ w2,
+                                             const float* __restrict__ b2, const float* __restrict__ w3, const float* __restrict__ b3,
+                                             int j) {
   uint32_t v;
   if (j < kOffW2 / 4) {  // layer 1: 4 f32 per chunk
     const int chunk = j / (kHidden * 4), rem = j % (kHidden * 4);
@@ -567,7 +565,33 @@ __global__ void __launch_bounds__(kPackThreads) k_actor_pack(const float* __rest
     const int i = j - kOffB3 / 4;
     v = i < kAct ? __float_as_uint(b3[i]) : 0u;
   }
-  out[j] = v;
+  return v;
+}
+
+__global__ void __launch_bounds__(kPackThreads) k_actor_pack(const float* __restrict__ w1, const float* __restrict__ b1,
+                                                             const float* __restrict__ w2, const float* __restrict__ b2,
+                                                             const float* __restrict__ w3, const float* __restrict__ b3,
+                                                             uint32_t* __restrict__ out) {
+  const int j = blockIdx.x * kPackThreads + threadIdx.x;
+  if (j >= kParamWords) return;
+  out[j] = packWord(w1, b1, w2, b2, w3, b3, j);
+}
+
+// K actors at once: slot s (blockIdx.y) of the pool table from the fp32 actor block at actors + s * stride, whose
+// parameters lie back to back in state_dict order (fc1.weight, fc1.bias, fc2.weight, fc2.bias, fc3.weight, fc3.bias):
+// exactly the actor block of a TD3 arena (hk_td3.cuh), so stride = the arena's size in floats packs a population.
+constexpr int kActorFloats = kHidden * kObs + kHidden + kHidden * kHidden + kHidden + kAct * kHidden + kAct;
+__global__ void __launch_bounds__(kPackThreads) k_actor_pack_many(const float* __restrict__ actors, long long stride,
+                                                                  uint32_t* __restrict__ table) {
+  const int j = blockIdx.x * kPackThreads + threadIdx.x;
+  if (j >= kParamWords) return;
+  const float* w1 = actors + (long long)blockIdx.y * stride;
+  const float* b1 = w1 + kHidden * kObs;
+  const float* w2 = b1 + kHidden;
+  const float* b2 = w2 + kHidden * kHidden;
+  const float* w3 = b2 + kHidden;
+  const float* b3 = w3 + kAct * kHidden;
+  table[(long long)blockIdx.y * kParamWords + j] = packWord(w1, b1, w2, b2, w3, b3, j);
 }
 
 }  // namespace hk_actor

@@ -2109,6 +2109,22 @@ int hk_actor_pack(const float* w1, const float* b1, const float* w2, const float
   return HK_OK;
 }
 
+int hk_actor_pack_many(const float* actors_dev, int64_t stride_floats, int k, void* table_dev, int device, void* stream) {
+  const char* who = "hk_actor_pack_many";
+  if (!actors_dev || !table_dev) return fail(HK_E_INVALID, std::string(who) + ": NULL argument");
+  if (k < 1 || k > hk_actor::kPoolMaxK) return fail(HK_E_INVALID, std::string(who) + ": k must be in [1, 4096]");
+  if (stride_floats < hk_actor::kActorFloats) return fail(HK_E_INVALID, std::string(who) + ": stride_floats must be >= 71684");
+  if (((uintptr_t)table_dev) & 15u) return fail(HK_E_INVALID, std::string(who) + ": table needs 16-byte alignment");
+  if (((uintptr_t)actors_dev) & 3u) return fail(HK_E_INVALID, std::string(who) + ": actors need 4-byte alignment");
+  if (int rc = deviceCheck(who, device)) return rc;
+  DeviceGuard guard(device);
+  using namespace hk_actor;
+  const dim3 grid((kParamWords + kPackThreads - 1) / kPackThreads, (unsigned)k);
+  k_actor_pack_many<<<grid, kPackThreads, 0, (cudaStream_t)stream>>>(actors_dev, (long long)stride_floats, (uint32_t*)table_dev);
+  HK_CUDA(cudaGetLastError());
+  return HK_OK;
+}
+
 int64_t hk_td3_arena_bytes(void) { return 4 * hk_td3::kArenaFloats; }
 
 int64_t hk_td3_scratch_bytes(int batch) {
@@ -2156,33 +2172,20 @@ int hk_td3_cluster_size(int device) {
 
 static bool finiteNonNeg(float x) { return x >= 0.0f && !std::isinf(x); }
 
-int hk_td3_update(void* arena_dev, void* scratch_dev, const hk_td3_batch* batch, int batch_size, const hk_td3_hparams* hp,
-                  const float* action_low_dev, const float* action_range_dev, uint64_t seed, int do_actor, float* losses_dev,
-                  int device, void* stream) {
-  const std::string who = "hk_td3_update";
-  if (!arena_dev || !scratch_dev || !batch || !hp || !action_low_dev || !action_range_dev || !losses_dev)
-    return fail(HK_E_INVALID, who + ": NULL argument");
-  if (!batch->obs || !batch->action || !batch->reward || !batch->next_obs || !batch->done || !batch->idx)
-    return fail(HK_E_INVALID, who + ": NULL batch array");
-  if (batch->prio_weights && !batch->prio_idx) return fail(HK_E_INVALID, who + ": NULL prio_idx with prio_weights");
-  if ((((uintptr_t)arena_dev) & 15u) || (((uintptr_t)scratch_dev) & 15u))
-    return fail(HK_E_INVALID, who + ": arena and scratch need 16-byte alignment");
-  if ((((uintptr_t)batch->idx) & 7u) || (batch->prio_weights && (((uintptr_t)batch->prio_idx) & 7u)))
-    return fail(HK_E_INVALID, who + ": idx and prio_idx need 8-byte alignment");
-  if ((((uintptr_t)batch->obs) | ((uintptr_t)batch->action) | ((uintptr_t)batch->reward) | ((uintptr_t)batch->next_obs) |
-       ((uintptr_t)batch->done) | ((uintptr_t)batch->prio_weights) | ((uintptr_t)action_low_dev) | ((uintptr_t)action_range_dev) |
-       ((uintptr_t)losses_dev)) & 3u)
-    return fail(HK_E_INVALID, who + ": float arrays need 4-byte alignment");
-  if (batch_size < 1 || batch_size > hk_td3::kMaxBatch) return fail(HK_E_INVALID, who + ": batch must be in [1, 1024]");
+// The ten hyper-parameters; `who` prefixes the message ("hk_td3_update" or "hk_td3_update_population: member m").
+static int td3HparamsCheck(const std::string& who, const hk_td3_hparams* hp) {
   const float hv[10] = {hp->gamma, hp->tau_actor, hp->tau_critic, hp->lr_actor, hp->lr_critic, hp->wd_actor, hp->wd_critic,
                         hp->beta, hp->target_noise, hp->target_noise_clip};
   const char* hn[10] = {"gamma", "tau_actor", "tau_critic", "lr_actor", "lr_critic", "wd_actor", "wd_critic", "beta",
                         "target_noise", "target_noise_clip"};
   for (int i = 0; i < 10; ++i)
     if (!finiteNonNeg(hv[i])) return fail(HK_E_INVALID, who + ": " + hn[i] + " must be finite and >= 0");
-  if (batch->prio_weights && batch->prio_n < 1) return fail(HK_E_INVALID, who + ": prio_n must be >= 1");
-  if (int rc = deviceCheck(who.c_str(), device)) return rc;
-  DeviceGuard guard(device);
+  return HK_OK;
+}
+
+// The kernel arguments of one learner's update; the batch's idx / prio_idx are taken from `batch` as given.
+static hk_td3::Args td3Args(void* arena_dev, void* scratch_dev, const hk_td3_batch* batch, int batch_size, const hk_td3_hparams* hp,
+                            const float* action_low_dev, const float* action_range_dev, uint64_t seed, int do_actor, float* losses_dev) {
   hk_td3::Args a;
   a.arena = (float*)arena_dev;
   a.scratch = (float*)scratch_dev;
@@ -2211,18 +2214,132 @@ int hk_td3_update(void* arena_dev, void* scratch_dev, const hk_td3_batch* batch,
   a.beta = hp->beta;
   a.sigma = hp->target_noise;
   a.clip = hp->target_noise_clip;
-  const int cluster = td3Cluster(device);
+  return a;
+}
+
+static cudaLaunchConfig_t td3LaunchConfig(cudaLaunchAttribute* attr, int cluster, int clusters, void* stream) {
   cudaLaunchConfig_t cfg = {};
-  cudaLaunchAttribute attr;
-  attr.id = cudaLaunchAttributeClusterDimension;
-  attr.val.clusterDim.x = (unsigned)cluster;
-  attr.val.clusterDim.y = attr.val.clusterDim.z = 1;
-  cfg.gridDim = dim3((unsigned)cluster);
+  attr->id = cudaLaunchAttributeClusterDimension;
+  attr->val.clusterDim.x = (unsigned)cluster;
+  attr->val.clusterDim.y = attr->val.clusterDim.z = 1;
+  cfg.gridDim = dim3((unsigned)(cluster * clusters));
   cfg.blockDim = dim3(hk_td3::kThreads);
   cfg.stream = (cudaStream_t)stream;
-  cfg.attrs = &attr;
+  cfg.attrs = attr;
   cfg.numAttrs = 1;
+  return cfg;
+}
+
+int hk_td3_update(void* arena_dev, void* scratch_dev, const hk_td3_batch* batch, int batch_size, const hk_td3_hparams* hp,
+                  const float* action_low_dev, const float* action_range_dev, uint64_t seed, int do_actor, float* losses_dev,
+                  int device, void* stream) {
+  const std::string who = "hk_td3_update";
+  if (!arena_dev || !scratch_dev || !batch || !hp || !action_low_dev || !action_range_dev || !losses_dev)
+    return fail(HK_E_INVALID, who + ": NULL argument");
+  if (!batch->obs || !batch->action || !batch->reward || !batch->next_obs || !batch->done || !batch->idx)
+    return fail(HK_E_INVALID, who + ": NULL batch array");
+  if (batch->prio_weights && !batch->prio_idx) return fail(HK_E_INVALID, who + ": NULL prio_idx with prio_weights");
+  if ((((uintptr_t)arena_dev) & 15u) || (((uintptr_t)scratch_dev) & 15u))
+    return fail(HK_E_INVALID, who + ": arena and scratch need 16-byte alignment");
+  if ((((uintptr_t)batch->idx) & 7u) || (batch->prio_weights && (((uintptr_t)batch->prio_idx) & 7u)))
+    return fail(HK_E_INVALID, who + ": idx and prio_idx need 8-byte alignment");
+  if ((((uintptr_t)batch->obs) | ((uintptr_t)batch->action) | ((uintptr_t)batch->reward) | ((uintptr_t)batch->next_obs) |
+       ((uintptr_t)batch->done) | ((uintptr_t)batch->prio_weights) | ((uintptr_t)action_low_dev) | ((uintptr_t)action_range_dev) |
+       ((uintptr_t)losses_dev)) & 3u)
+    return fail(HK_E_INVALID, who + ": float arrays need 4-byte alignment");
+  if (batch_size < 1 || batch_size > hk_td3::kMaxBatch) return fail(HK_E_INVALID, who + ": batch must be in [1, 1024]");
+  if (int rc = td3HparamsCheck(who, hp)) return rc;
+  if (batch->prio_weights && batch->prio_n < 1) return fail(HK_E_INVALID, who + ": prio_n must be >= 1");
+  if (int rc = deviceCheck(who.c_str(), device)) return rc;
+  DeviceGuard guard(device);
+  const hk_td3::Args a = td3Args(arena_dev, scratch_dev, batch, batch_size, hp, action_low_dev, action_range_dev, seed, do_actor, losses_dev);
+  cudaLaunchAttribute attr;
+  const cudaLaunchConfig_t cfg = td3LaunchConfig(&attr, td3Cluster(device), 1, stream);
   HK_CUDA(cudaLaunchKernelEx(&cfg, hk_td3::k_td3_update, a));
+  return HK_OK;
+}
+
+// How many clusters of 16 and of 8 CTAs of k_td3_update_population the device keeps resident at once (probed once per
+// device; 0 where the probe is refused).
+static void td3PopulationOccupancy(int device, int* occ16, int* occ8) {
+  static int probed[64][2] = {{0}};
+  static bool done[64] = {false};
+  int* p = probed[device & 63];
+  if (!done[device & 63]) {
+    const void* k = (const void*)hk_td3::k_td3_update_population;
+    const bool nonPortable = cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
+    for (int i = 0; i < 2; ++i) {
+      const int size = i == 0 ? 16 : 8;
+      if (size > 8 && !nonPortable) continue;
+      cudaLaunchAttribute attr;
+      const cudaLaunchConfig_t cfg = td3LaunchConfig(&attr, size, 1, nullptr);
+      int clusters = 0;
+      if (cudaOccupancyMaxActiveClusters(&clusters, k, &cfg) == cudaSuccess) p[i] = clusters;
+    }
+    cudaGetLastError();  // a refused probe leaves no sticky error
+    done[device & 63] = true;
+  }
+  *occ16 = p[0];
+  *occ8 = p[1];
+}
+
+// The cluster size of a population launch of k members: the largest of {16, 8} at which all k clusters are resident at
+// once, else 16 (the clusters then run in waves, and 16-CTA clusters finish each wave sooner).  The result does not depend
+// on it.  HK_TD3_CLUSTER (td3Cluster) caps it, for the tests.
+static int td3PopulationCluster(int k, int device) {
+  int occ16 = 0, occ8 = 0;
+  td3PopulationOccupancy(device, &occ16, &occ8);
+  return std::min(occ16 >= k ? 16 : occ8 >= k ? 8 : 16, td3Cluster(device));
+}
+
+int hk_td3_population_cluster_size(int k, int device) {
+  if (k < 1 || k > hk_td3::kMaxPopulation) return fail(HK_E_INVALID, "hk_td3_population_cluster_size: k must be in [1, 64]");
+  if (int rc = deviceCheck("hk_td3_population_cluster_size", device)) return rc;
+  DeviceGuard guard(device);
+  return td3PopulationCluster(k, device);
+}
+
+int hk_td3_update_population(void* arenas_dev, void* scratch_dev, const hk_td3_batch* batch, int batch_size, int k,
+                             const hk_td3_hparams* hp, const float* const* action_low, const float* const* action_range,
+                             const uint64_t* seeds, const uint8_t* do_actor, float* losses_dev, int device, void* stream) {
+  const std::string who = "hk_td3_update_population";
+  if (!arenas_dev || !scratch_dev || !batch || !hp || !action_low || !action_range || !seeds || !do_actor || !losses_dev)
+    return fail(HK_E_INVALID, who + ": NULL argument");
+  if (!batch->obs || !batch->action || !batch->reward || !batch->next_obs || !batch->done || !batch->idx)
+    return fail(HK_E_INVALID, who + ": NULL batch array");
+  if (batch->prio_weights && !batch->prio_idx) return fail(HK_E_INVALID, who + ": NULL prio_idx with prio_weights");
+  if ((((uintptr_t)arenas_dev) & 15u) || (((uintptr_t)scratch_dev) & 15u))
+    return fail(HK_E_INVALID, who + ": arenas and scratch need 16-byte alignment");
+  if ((((uintptr_t)batch->idx) & 7u) || (batch->prio_weights && (((uintptr_t)batch->prio_idx) & 7u)))
+    return fail(HK_E_INVALID, who + ": idx and prio_idx need 8-byte alignment");
+  if ((((uintptr_t)batch->obs) | ((uintptr_t)batch->action) | ((uintptr_t)batch->reward) | ((uintptr_t)batch->next_obs) |
+       ((uintptr_t)batch->done) | ((uintptr_t)batch->prio_weights) | ((uintptr_t)losses_dev)) & 3u)
+    return fail(HK_E_INVALID, who + ": float arrays need 4-byte alignment");
+  if (k < 1 || k > hk_td3::kMaxPopulation) return fail(HK_E_INVALID, who + ": k must be in [1, 64]");
+  if (batch_size < 1 || batch_size > hk_td3::kMaxBatch) return fail(HK_E_INVALID, who + ": batch must be in [1, 1024]");
+  if (batch->prio_weights && batch->prio_n < 1) return fail(HK_E_INVALID, who + ": prio_n must be >= 1");
+  for (int m = 0; m < k; ++m) {
+    const std::string wm = who + ": member " + std::to_string(m);
+    if (!action_low[m] || !action_range[m]) return fail(HK_E_INVALID, wm + ": NULL action_low / action_range");
+    if ((((uintptr_t)action_low[m]) | ((uintptr_t)action_range[m])) & 3u)
+      return fail(HK_E_INVALID, wm + ": action_low / action_range need 4-byte alignment");
+    if (int rc = td3HparamsCheck(wm, hp + m)) return rc;
+  }
+  if (int rc = deviceCheck(who.c_str(), device)) return rc;
+  DeviceGuard guard(device);
+  const int64_t arenaFloats = hk_td3::kArenaFloats, scratchFloats = hk_td3::carve(nullptr, batch_size).floats;
+  hk_td3::PopulationArgs p;
+  memset(&p, 0, sizeof(p));
+  for (int m = 0; m < k; ++m) {
+    hk_td3_batch bm = *batch;
+    bm.idx = batch->idx + (int64_t)m * batch_size;
+    if (batch->prio_weights) bm.prio_idx = batch->prio_idx + (int64_t)m * batch_size;
+    p.m[m] = td3Args((float*)arenas_dev + m * arenaFloats, (float*)scratch_dev + m * scratchFloats, &bm, batch_size, hp + m,
+                     action_low[m], action_range[m], seeds[m], do_actor[m], losses_dev + 2 * m);
+  }
+  cudaLaunchAttribute attr;
+  const cudaLaunchConfig_t cfg = td3LaunchConfig(&attr, td3PopulationCluster(k, device), k, stream);
+  HK_CUDA(cudaLaunchKernelEx(&cfg, hk_td3::k_td3_update_population, p));
   return HK_OK;
 }
 

@@ -18,7 +18,8 @@
 //     the actor's backward pass) and the loss are a warp per row, dot products reduced by a fixed xor-shuffle tree.
 //   * flat: Adam and Polyak are elementwise over the parameter vectors.
 // So every output element is computed by exactly one thread in a fixed order whatever the cluster size, and the result
-// does not depend on it.  A single cluster is bounded by latency, not by FMA throughput; the fp32 SIMT path keeps the
+// does not depend on it.  k_td3_update_population runs K such updates (K independent learners)
+// in one grid of K clusters, cluster m on member m's arguments; each member's result is that of its own k_td3_update.  A single cluster is bounded by latency, not by FMA throughput; the fp32 SIMT path keeps the
 // learner equivalent to torch's fp32 learner (tensor cores are out of scope, DESIGN.md section 4.2).
 //
 // Numerics contract:
@@ -331,8 +332,8 @@ __device__ __forceinline__ void polyak(float* tp, const float* p, int n, float t
   for (int i = gtid; i < n; i += gstride) tp[i] = ld(tp + i) * keep + tau * ld(p + i);
 }
 
-// ---- the kernel -----------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kThreads, 1) k_td3_update(const Args a) {
+// ---- the update body: one learner's update on the calling cluster ----------------------------------------------------------
+__device__ __forceinline__ void td3Update(const Args& a) {
   __shared__ __align__(16) Smem sm;
   const int nc = (int)cg::this_cluster().num_blocks(), c = (int)cg::this_cluster().block_rank();
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
@@ -654,6 +655,23 @@ __global__ void __launch_bounds__(kThreads, 1) k_td3_update(const Args a) {
     if (a.doActor) ctr[1] = tA;
     ctr[2] = noiseCtr + 1;
   }
+}
+
+// ---- the kernels ----------------------------------------------------------------------------------------------------------
+// One learner: one cluster.
+__global__ void __launch_bounds__(kThreads, 1) k_td3_update(const Args a) { td3Update(a); }
+
+// A population of K independent learners: K clusters in one grid; cluster m (blockIdx.x / cluster size) runs member m's
+// update.  The members share nothing the update writes (arena, scratch, losses and, for prioritized batches, the rows of
+// the weights their prio_idx point at are per member), so the clusters never synchronise with each other.  The table is a
+// __grid_constant__ parameter: the dynamically indexed member is read from parameter space, never copied to local memory.
+constexpr int kMaxPopulation = 64;  // HK_TD3_MAX_POPULATION
+static_assert(sizeof(Args) * kMaxPopulation < 32764 - 64, "the member table must fit the kernel parameter space");
+struct PopulationArgs {
+  Args m[kMaxPopulation];
+};
+__global__ void __launch_bounds__(kThreads, 1) k_td3_update_population(const __grid_constant__ PopulationArgs p) {
+  td3Update(p.m[blockIdx.x / cg::this_cluster().num_blocks()]);
 }
 
 }  // namespace hk_td3

@@ -115,6 +115,101 @@ class DevicePrioritizedReplayBuffer(DeviceReplayBuffer):
         self.last_batch_inds = None
 
 
+class PopulationReplayBuffer:
+    """One device replay buffer for a population of K learners (`FusedTD3Population`): arrays of K * capacity rows, of
+    which member m owns rows [m * capacity, (m + 1) * capacity), each a ring buffer like `DeviceReplayBuffer` (or, with
+    prioritized=True, like `DevicePrioritizedReplayBuffer`).  All members share the ring position and the size.
+
+    `push` takes the transitions of N = K * n envs: env block m (rows [m * n, (m + 1) * n)) goes to member m, one strided
+    copy per array.  `sample_indices(b)` returns [K, b] int64 GLOBAL rows, member m's inside its own rows, so that one
+    population update reads all members' batches from the shared arrays (and, prioritized, writes each member's
+    priorities into its own rows only)."""
+
+    def __init__(self, k, capacity, obs_dim=18, action_dim=4, device="cuda:0", seed=0, prioritized=False, init_weight=1e8):
+        self.k, self.capacity, self.device = int(k), int(capacity), torch.device(device)
+        if self.k < 1 or self.capacity < 1:
+            raise ValueError("PopulationReplayBuffer needs k >= 1 and capacity >= 1")
+        rows = self.k * self.capacity
+        self.obs = torch.empty((rows, obs_dim), dtype=torch.float32, device=self.device)
+        self.action = torch.empty((rows, action_dim), dtype=torch.float32, device=self.device)
+        self.reward = torch.empty(rows, dtype=torch.float32, device=self.device)
+        self.next_obs = torch.empty((rows, obs_dim), dtype=torch.float32, device=self.device)
+        self.done = torch.empty(rows, dtype=torch.float32, device=self.device)
+        self.prioritized = bool(prioritized)
+        self.init_weight = float(init_weight)
+        self.weights = torch.full((rows,), self.init_weight, dtype=torch.float32, device=self.device) if self.prioritized else None
+        self.pos, self.size = 0, 0
+        self.seed = seed
+        self.gen = torch.Generator(device=self.device)
+        self.gen.manual_seed(seed)
+        self.offsets = torch.arange(self.k, dtype=torch.int64, device=self.device).unsqueeze(1) * self.capacity  # [K, 1]
+
+    def __len__(self):
+        return self.size
+
+    def _rows(self, t):
+        """[K, capacity, ...] view of a [K * capacity, ...] array."""
+        return t.view(self.k, self.capacity, *t.shape[1:])
+
+    def push(self, obs, action, reward, next_obs, done):
+        """N = K * n transitions (n <= capacity); block m of the batch goes to member m's ring."""
+        n_all = obs.shape[0]
+        if n_all % self.k:
+            raise ValueError(f"PopulationReplayBuffer.push: {n_all} rows do not split into {self.k} equal blocks")
+        n = n_all // self.k
+        if n > self.capacity:
+            raise ValueError("batch larger than the buffer")
+        top = None
+        if self.prioritized:
+            w = self._rows(self.weights)
+            top = w[:, :self.size].amax(1) if self.size > 0 else torch.full((self.k,), self.init_weight, device=self.device)
+        first = min(n, self.capacity - self.pos)
+        for dst, src in ((self.obs, obs), (self.action, action), (self.reward, reward), (self.next_obs, next_obs),
+                         (self.done, done.to(torch.float32))):
+            d, sv = self._rows(dst), src.reshape(self.k, n, *src.shape[1:])
+            d[:, self.pos:self.pos + first].copy_(sv[:, :first])
+            if first < n:
+                d[:, :n - first].copy_(sv[:, first:])
+        if top is not None:
+            w = self._rows(self.weights)
+            w[:, self.pos:self.pos + first] = top.unsqueeze(1)
+            if first < n:
+                w[:, :n - first] = top.unsqueeze(1)
+        self.pos = (self.pos + n) % self.capacity
+        self.size = min(self.capacity, self.size + n)
+
+    def sample_indices(self, batch_size):
+        """[K, b] int64 global rows, b = min(batch_size, len): uniform over each member's stored rows (one randint), or
+        proportional to each member's weights (one row-wise multinomial)."""
+        b = min(int(batch_size), self.size)
+        if not self.prioritized:
+            local = torch.randint(0, self.size, (self.k, b), device=self.device, generator=self.gen)
+        else:
+            w = torch.nan_to_num(self._rows(self.weights)[:, :self.size], nan=0.0, posinf=0.0, neginf=0.0).clamp_min(1e-6)
+            local = torch.multinomial(w / w.sum(1, keepdim=True), b, replacement=True, generator=self.gen)
+        return local + self.offsets
+
+    def member(self, m):
+        """Member m's rows as a `DeviceReplayBuffer` (prioritized: `DevicePrioritizedReplayBuffer`) over VIEWS of this
+        buffer's arrays, with this buffer's current size and position and a generator of its own (seeded seed + 1 + m).
+        Writes through either alias the same memory; size and position are copied, not shared."""
+        m = int(m)
+        if not 0 <= m < self.k:
+            raise IndexError(f"member {m} out of range [0, {self.k})")
+        cls = DevicePrioritizedReplayBuffer if self.prioritized else DeviceReplayBuffer
+        out = cls.__new__(cls)
+        out.capacity, out.device = self.capacity, self.device
+        lo, hi = m * self.capacity, (m + 1) * self.capacity
+        out.obs, out.action, out.reward = self.obs[lo:hi], self.action[lo:hi], self.reward[lo:hi]
+        out.next_obs, out.done = self.next_obs[lo:hi], self.done[lo:hi]
+        out.pos, out.size = self.pos, self.size
+        out.gen = torch.Generator(device=self.device)
+        out.gen.manual_seed(self.seed + 1 + m)
+        if self.prioritized:
+            out.init_weight, out.weights, out.last_batch_inds = self.init_weight, self.weights[lo:hi], None
+        return out
+
+
 class DeviceTD3Learner:
     """TD3Learner.update (rl/td3/learner.py:55-219) on device batches: clipped-noise target actions, min of the twin target
     critics, weighted smooth-L1 critic loss (mean of both heads), actor and Polyak target updates every
@@ -232,7 +327,9 @@ class FusedTD3Learner(DeviceTD3Learner):
 
     MAX_BATCH = 1024
 
-    def __init__(self, actor=None, critic=None, config=None, replay_buffer=None, device="cuda:0", seed=0):
+    def __init__(self, actor=None, critic=None, config=None, replay_buffer=None, device="cuda:0", seed=0, arena=None):
+        """arena: None (allocate one), or a zeroed contiguous uint8 CUDA tensor of hk_td3_arena_bytes() bytes on `device`
+        to home the parameters in (FusedTD3Population passes rows of its [K, bytes] arena table)."""
         import ctypes as C
         from . import _lib
         from .actor import _cuda_device
@@ -249,7 +346,12 @@ class FusedTD3Learner(DeviceTD3Learner):
         blocks, ctr_off, nbytes = self.arena_layout()
         if nbytes != int(self.L.hk_td3_arena_bytes()):
             raise _lib.HockeyLibraryError("FusedTD3Learner: the library's arena size does not match this package")
-        self.arena = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
+        if arena is None:
+            arena = torch.zeros(nbytes, dtype=torch.uint8, device=self.device)
+        elif not (arena.dtype == torch.uint8 and arena.is_contiguous() and tuple(arena.shape) == (nbytes,)
+                  and arena.device == self.device and arena.data_ptr() % 16 == 0):
+            raise ValueError(f"FusedTD3Learner: arena must be a contiguous 16-byte aligned uint8 tensor [{nbytes}] on {self.device}")
+        self.arena = arena
         f = self.arena.view(torch.float32)
         self.blocks = {name: f[o:o + n] for name, (o, n) in blocks.items()}  # flat fp32 views, parameters in state_dict order
         self.counters = self.arena[4 * ctr_off:4 * ctr_off + 24].view(torch.int64)  # critic step, actor step, noise counter
@@ -361,6 +463,146 @@ class FusedTD3Learner(DeviceTD3Learner):
         return self._launch((buf.obs, buf.action, buf.reward, buf.next_obs, buf.done), idx, prio)
 
 
+class FusedTD3Population:
+    """K independent TD3 learners (a seed or hyper-parameter sweep, population-based training) updated in ONE launch of K
+    thread-block clusters (hk_td3_update_population): member m's update is byte-for-byte the one `FusedTD3Learner` would
+    make with the same batch, so the population runs K learners at once on SMs a single learner leaves idle.
+
+    `members[m]` is a full `FusedTD3Learner` whose arena is row m of `arenas` ([K, hk_td3_arena_bytes()] uint8): its
+    modules, `state_dict` / `load_state_dict`, `FusedActor.refresh(member.actor)` and a single-member `update` work on
+    the live weights.  `configs[m]` is member m's `TD3Config`; every field may differ per member except batch_size,
+    buffer_size and prioritized_replay, which the shared `PopulationReplayBuffer` fixes.  Hyper-parameters are read at
+    every update, so editing `configs[m]` between calls is PBT's explore step; `copy_member(dst, src)` is its exploit step.
+
+    configs: None (defaults), one TD3Config (copied for each member) or a list of K.  actors / critics: lists of K modules
+    or None (fresh ones).  seeds: K target-noise seeds (default 0 .. K-1).  replay_buffer: a PopulationReplayBuffer of
+    this K (default: a new one of the configs' buffer_size and prioritized_replay, seed 0)."""
+
+    MAX_K = 64  # HK_TD3_MAX_POPULATION
+
+    def __init__(self, k, configs=None, actors=None, critics=None, seeds=None, replay_buffer=None, device="cuda:0"):
+        import ctypes as C
+        from . import _lib
+        self.k = int(k)
+        if not 1 <= self.k <= self.MAX_K:
+            raise ValueError(f"FusedTD3Population: k must be in [1, {self.MAX_K}], got {k}")
+        self.configs = self._configs(self.k, configs)
+        for name, xs in (("actors", actors), ("critics", critics), ("seeds", seeds)):
+            if xs is not None and len(xs) != self.k:
+                raise ValueError(f"FusedTD3Population: {name} must have k = {self.k} entries, got {len(xs)}")
+        cfg0 = self.configs[0]
+        if replay_buffer is not None and (replay_buffer.k != self.k or replay_buffer.prioritized != cfg0.prioritized_replay):
+            raise ValueError(f"FusedTD3Population: the replay buffer must be a PopulationReplayBuffer of k = {self.k} with "
+                             f"prioritized={cfg0.prioritized_replay}")
+        from .actor import _cuda_device
+        self.device = _cuda_device(device, "FusedTD3Population")
+        if self.device.index is None:
+            self.device = torch.device("cuda", torch.cuda.current_device())
+        self._C, self._lib = C, _lib
+        self.L = _lib.load()
+        self.seeds = [int(s) & (2**64 - 1) for s in (seeds if seeds is not None else range(self.k))]
+        self.replay_buffer = replay_buffer if replay_buffer is not None else PopulationReplayBuffer(
+            self.k, cfg0.buffer_size, device=self.device, prioritized=cfg0.prioritized_replay)
+        self.arena_bytes = int(self.L.hk_td3_arena_bytes())
+        self.arenas = torch.zeros((self.k, self.arena_bytes), dtype=torch.uint8, device=self.device)
+        self.members = [FusedTD3Learner(actor=None if actors is None else actors[m], critic=None if critics is None else critics[m],
+                                        config=self.configs[m], device=self.device, seed=self.seeds[m], arena=self.arenas[m])
+                        for m in range(self.k)]
+        self._scratch, self._scratch_b = None, 0
+        self._last_batch = 0
+        self.fused_pool = None  # train_population: the FusedActorPool the members act through
+        n = self.k
+        self._hp = (_lib.TD3HParams * n)()
+        self._low, self._range = (C.c_void_p * n)(), (C.c_void_p * n)()
+        self._seeds = (C.c_uint64 * n)(*self.seeds)
+        self._do_actor = (C.c_uint8 * n)()
+
+    @staticmethod
+    def _configs(k, configs):
+        if configs is None:
+            configs = TD3Config()
+        if isinstance(configs, TD3Config):
+            configs = [copy.copy(configs) for _ in range(k)]
+        configs = list(configs)
+        if len(configs) != k:
+            raise ValueError(f"FusedTD3Population: configs must have k = {k} entries, got {len(configs)}")
+        for f in ("batch_size", "buffer_size", "prioritized_replay"):
+            vals = {getattr(c, f) for c in configs}
+            if len(vals) != 1:
+                raise ValueError(f"FusedTD3Population: {f} must be equal across the members (they share one replay buffer "
+                                 f"and one launch), got {sorted(vals)}")
+        return configs
+
+    def __len__(self):
+        return self.k
+
+    def copy_member(self, dst, src):
+        """Make member dst a copy of member src: the whole arena row (weights, targets, Adam moments, step counts and
+        noise counter), the critics' action bounds and the actor-step schedule.  configs and seeds stay per member."""
+        d, s = self.members[dst], self.members[src]
+        self.arenas[dst].copy_(self.arenas[src])
+        for net_d, net_s in ((d.critic, s.critic), (d.target_critic, s.target_critic)):
+            for k in ("action_low", "action_high", "action_range"):
+                getattr(net_d, k).copy_(getattr(net_s, k))
+        d.train_step = s.train_step
+
+    def update_from_buffer(self, batch_size=None):
+        """One index draw ([K, b] from the population buffer) and one population launch (`update`)."""
+        return self.update(self.replay_buffer.sample_indices(batch_size or self.configs[0].batch_size))
+
+    def update(self, idx):
+        """One population launch on the batches idx ([K, b] int64 CUDA: global rows of the population buffer, member m's
+        inside its own rows; not checked).  Returns ([K] actor losses, NaN for members that made no actor step; [K] critic
+        losses) as device tensors; no host sync, graph-capturable."""
+        C, lib, buf = self._C, self._lib, self.replay_buffer
+        if not (idx.dtype == torch.int64 and idx.dim() == 2 and idx.shape[0] == self.k and idx.is_contiguous()
+                and idx.device == self.device):
+            raise ValueError(f"FusedTD3Population.update: idx must be a contiguous int64 tensor [{self.k}, b] on {self.device}")
+        b = idx.shape[1]
+        if not 1 <= b <= FusedTD3Learner.MAX_BATCH:
+            raise ValueError(f"FusedTD3Population: batch size must be in [1, {FusedTD3Learner.MAX_BATCH}], got {b}")
+        per = int(self.L.hk_td3_scratch_bytes(b))
+        if self._scratch is None or self._scratch_b != b:
+            self._scratch = torch.empty((self.k, per), dtype=torch.uint8, device=self.device)
+            self._scratch_b = b
+        for m, mem in enumerate(self.members):
+            mem.cfg = self.configs[m]
+            mem.train_step += 1
+            self._do_actor[m] = int(mem.train_step % mem.cfg.policy_update_freq == 0)
+            self._hp[m] = mem._hparams()
+            self._low[m], self._range[m] = mem.critic.action_low.data_ptr(), mem.critic.action_range.data_ptr()
+        losses = torch.full((self.k, 2), float("nan"), dtype=torch.float32, device=self.device)
+        batch = lib.TD3Batch(buf.obs.data_ptr(), buf.action.data_ptr(), buf.reward.data_ptr(), buf.next_obs.data_ptr(),
+                             buf.done.data_ptr(), idx.data_ptr())
+        if buf.prioritized:
+            batch.prio_weights, batch.prio_idx, batch.prio_n = buf.weights.data_ptr(), idx.data_ptr(), buf.size
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            lib.check(self.L.hk_td3_update_population(
+                C.c_void_p(self.arenas.data_ptr()), C.c_void_p(self._scratch.data_ptr()), C.byref(batch), b, self.k, self._hp,
+                self._low, self._range, self._seeds, self._do_actor, C.c_void_p(losses.data_ptr()), self.device.index,
+                C.c_void_p(stream)))
+        self._last_batch = b
+        self.last_do_actor = [bool(v) for v in self._do_actor]
+        return losses[:, 0], losses[:, 1]
+
+    def last_importance_weights(self):
+        """[K, B] importance weights of the last update (ones for uniform batches), computed in the kernel."""
+        return self._scratch.view(torch.float32)[:, :self._last_batch]
+
+    def refresh_pool(self, pool):
+        """Repack slots 0 .. K-1 of `pool` (a FusedActorPool) from the members' live actors in one hk_actor_pack_many
+        launch (no host sync); other slots are not touched."""
+        C = self._C
+        if len(pool) < self.k or pool.device != self.device:
+            raise ValueError(f"refresh_pool needs a FusedActorPool of >= {self.k} slots on {self.device}")
+        with torch.cuda.device(self.device):
+            self._lib.check(self.L.hk_actor_pack_many(
+                C.c_void_p(self.arenas.data_ptr()), self.arena_bytes // 4, self.k, C.c_void_p(pool.table.data_ptr()),
+                self.device.index, C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
+        return pool
+
+
 @torch.no_grad()
 def _explore(actor, obs, noise_scale, gen):
     a = actor(obs)
@@ -406,4 +648,49 @@ def train(env_or_pool, learner, ticks, updates_per_tick=1, noise_scale=None, war
                 changed |= actor_loss is not None
             if changed and mirror is not None:
                 mirror.refresh(learner.actor)
+    return loss
+
+
+def train_population(env_or_pool, population, ticks, updates_per_tick=1, noise_scale=None, warmup_ticks=8):
+    """`train(..., fused=True)` for a `FusedTD3Population`: the env's N rows are split into K equal contiguous blocks, and
+    block m acts through member m -- one noisy `FusedActorPool` launch per tick with the constant choice row // (N / K),
+    exploration noise keyed on the global row.  The transitions go to the population's buffer (block m to member m),
+    `updates_per_tick` population launches follow each tick after `warmup_ticks`, and after a tick whose updates stepped
+    any actor one hk_actor_pack_many launch repacks all K slots.  The exploration sigma is one scalar for the population
+    (noise_scale, or the members' action_noise_scale, which must then be equal).  An `OpponentPool` works as with
+    `train` (player-1 columns only).  Returns the [K] critic losses of the last update (device tensor; None if none ran)."""
+    from .actor import FusedActorPool
+    from .training import OpponentPool
+    pool = env_or_pool if isinstance(env_or_pool, OpponentPool) else None
+    env = pool.env if pool else env_or_pool
+    k, n = population.k, env.num_envs
+    if n % k:
+        raise ValueError(f"train_population: {n} envs do not split into {k} equal blocks")
+    if noise_scale is None:
+        scales = {c.action_noise_scale for c in population.configs}
+        if len(scales) != 1:
+            raise ValueError(f"train_population: the members' action_noise_scale differ ({sorted(scales)}); the pooled actor "
+                             f"launch takes one sigma, so pass noise_scale=")
+        noise_scale = scales.pop()
+    buf = population.replay_buffer
+    if population.fused_pool is None:
+        population.fused_pool = FusedActorPool([m.actor for m in population.members], device=population.device,
+                                               seed=population.seeds[0])
+    acting = population.refresh_pool(population.fused_pool)
+    choice = (torch.arange(n, device=env.device) // (n // k)).to(torch.int32)
+    obs = env.obs.clone()
+    loss = None
+    for t in range(ticks):
+        a = acting(obs, choice, noise=noise_scale)
+        nobs, reward, done, _, _ = pool.step(a) if pool else env.step(a.contiguous())
+        nxt = torch.where(done.to(torch.bool).unsqueeze(1), env.final_obs, nobs) if env.final_obs is not None else nobs
+        buf.push(obs, a, reward, nxt, done)
+        obs = nobs.clone()
+        if t >= warmup_ticks:
+            changed = False
+            for _ in range(updates_per_tick):
+                _, loss = population.update_from_buffer()
+                changed |= any(population.last_do_actor)
+            if changed:
+                population.refresh_pool(acting)
     return loss

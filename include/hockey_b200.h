@@ -303,6 +303,46 @@ int hk_td3_update(void* arena_dev, void* scratch_dev, const hk_td3_batch* batch,
  * size >= 1.  Results do not depend on it.  HK_E_NODEVICE without a GPU, HK_E_INVALID for a bad device index. */
 int hk_td3_cluster_size(int device);
 
+/* K independent TD3 learners (a seed or hyper-parameter sweep, population-based training) updated in ONE launch of K
+ * clusters: cluster m runs exactly hk_td3_update's update for member m, so the result of every member is byte-identical
+ * to an hk_td3_update call with member m's arguments (the single-member oracle).  1 <= k <= HK_TD3_MAX_POPULATION.
+ * Per member m:
+ *   arena      arenas_dev + m * hk_td3_arena_bytes() (K arenas back to back);
+ *   scratch    scratch_dev + m * hk_td3_scratch_bytes(batch_size) (its first batch_size floats: member m's importance
+ *              weights after the call);
+ *   indices    batch->idx + m * batch_size, and for a prioritized batch batch->prio_idx + m * batch_size ([k][batch] int64
+ *              each, rows of the replay arrays that all members share);
+ *   hp[m], seeds[m], do_actor[m] (nonzero: an actor step), action_low[m] / action_range[m] (device pointers to the member
+ *   critic's [4] buffers; the two pointer tables are host arrays), losses_dev + 2 * m (actor loss on actor steps only,
+ *   critic loss).
+ * Shared: the replay arrays, batch_size (1..1024), batch->prio_weights and batch->prio_n (every member's N).  For a
+ * prioritized batch, member m's prio_idx must point at rows only member m uses (its own part of the buffer), so that the
+ * priority write-backs of different members never overlap; the members' updates are otherwise independent.
+ * Everything travels in the launch's parameters (no device-side table, no host-to-device copy, no allocation, no host
+ * synchronisation): graph-capturable like hk_td3_update.  Invalid arguments (as for hk_td3_update, plus k outside [1, 64]
+ * and NULL or misaligned per-member pointers) return HK_E_INVALID before any device probe, with the member index and the
+ * field in the message (e.g. "hk_td3_update_population: member 3: lr_critic must be finite and >= 0"); valid ones
+ * without a GPU HK_E_NODEVICE. */
+#define HK_TD3_MAX_POPULATION 64
+int hk_td3_update_population(void* arenas_dev, void* scratch_dev, const hk_td3_batch* batch, int batch_size, int k,
+                             const hk_td3_hparams* hp /* [k] */, const float* const* action_low /* [k] */,
+                             const float* const* action_range /* [k] */, const uint64_t* seeds /* [k] */,
+                             const uint8_t* do_actor /* [k] */, float* losses_dev /* [k][2] */, int device, void* stream);
+/* The cluster size (CTAs per member) of a population launch of k members on `device`: the largest of {16, 8} at which the
+ * device keeps all k clusters resident at once (cudaOccupancyMaxActiveClusters >= k), else 16; never above
+ * hk_td3_cluster_size(device).  Results do not depend on it.  HK_E_INVALID for k outside [1, 64] or a bad device index,
+ * HK_E_NODEVICE without a GPU. */
+int hk_td3_population_cluster_size(int k, int device);
+
+/* Repack K actors into K slots of a pool table (hk_actor_forward_pool) in one launch: slot s (at table_dev +
+ * s * hk_actor_param_bytes(), 16-byte aligned) is packed from the actor whose fp32 parameters lie back to back in
+ * state_dict order (fc1.weight [256,18], fc1.bias, fc2.weight [256,256], fc2.bias, fc3.weight [4,256], fc3.bias) at
+ * actors_dev + s * stride_floats (4-byte aligned; stride_floats >= 71,684).  That is the actor block of a TD3 arena, so
+ * actors_dev = the first arena and stride_floats = hk_td3_arena_bytes() / 4 repack a whole population.  Each slot is
+ * byte-identical to hk_actor_pack of the same actor; slots >= k are not touched.  1 <= k <= 4096.  Error rules and
+ * stream semantics as for hk_actor_pack. */
+int hk_actor_pack_many(const float* actors_dev, int64_t stride_floats, int k, void* table_dev, int device, void* stream);
+
 /* Measurement: per-kernel device times of the ticks that follow.  hk_kernel_timing(env, 1) makes every hk_step /
  * hk_rollout tick record CUDA events on the launching stream around each kernel of the cascade (up to 2048 ticks; not
  * graph-capturable while enabled); hk_kernel_times synchronises the device, returns the summed milliseconds of
