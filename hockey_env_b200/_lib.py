@@ -21,7 +21,8 @@ EXPORTS = [
     "hk_create", "hk_destroy", "hk_num_envs", "hk_reset", "hk_reset_seeded", "hk_step", "hk_step_host", "hk_host_record_bytes", "hk_rollout", "hk_get_obs", "hk_get_info", "hk_get_state",
     "hk_set_state", "hk_set_obs_state", "hk_set_opponent_policies", "hk_set_reset_modes", "hk_get_modes", "hk_get_stats", "hk_clear_stats", "hk_stats_device_ptr", "hk_copy_stats", "hk_debug_phase_cycles", "hk_debug_finish_cycles", "hk_launches_per_step", "hk_debug_lane_trace", "hk_kernel_timing", "hk_kernel_times", "hk_actor_param_bytes", "hk_actor_forward", "hk_actor_pool_scratch_bytes", "hk_actor_forward_pool", "hk_actor_forward_noisy",
     "hk_actor_forward_pool_noisy", "hk_actor_pack", "hk_td3_arena_bytes", "hk_td3_scratch_bytes", "hk_td3_update", "hk_td3_cluster_size",
-    "hk_td3_update_population", "hk_td3_population_cluster_size", "hk_actor_pack_many", "hk_last_error",
+    "hk_td3_update_population", "hk_td3_population_cluster_size", "hk_actor_pack_many", "hk_actor_forward_explore",
+    "hk_actor_forward_pool_explore", "hk_last_error",
     "hk_version",
 ]
 
@@ -110,6 +111,10 @@ def load():
     L.hk_actor_forward_noisy.restype = i32
     L.hk_actor_forward_pool_noisy.argtypes = [vp, i32, vp, vp, vp, i32, i64, vp, u64, vp, f32, f32, i64, i32, vp]
     L.hk_actor_forward_pool_noisy.restype = i32
+    L.hk_actor_forward_explore.argtypes = [vp, vp, vp, i32, i64, u64, vp, vp, vp, vp, i64, i32, vp]
+    L.hk_actor_forward_explore.restype = i32
+    L.hk_actor_forward_pool_explore.argtypes = [vp, i32, vp, vp, vp, i32, i64, vp, u64, vp, vp, vp, vp, i64, i32, vp]
+    L.hk_actor_forward_pool_explore.restype = i32
     L.hk_actor_pack.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, vp]
     L.hk_actor_pack.restype = i32
     L.hk_td3_arena_bytes.argtypes = []

@@ -82,6 +82,17 @@ def _pack_on_device(L, lib, actor, dst, device, who):
                                   C.c_void_p(torch.cuda.current_stream(device).cuda_stream)))
 
 
+def _explore_args(noise, noise_clip, reset):
+    """True for noise=ExplorationNoise (which carries its own clip); reset= is only meaningful with one."""
+    if isinstance(noise, ExplorationNoise):
+        if noise_clip is not None:
+            raise ValueError("noise_clip does not apply to an ExplorationNoise: its slots carry the clip")
+        return True
+    if reset is not None:
+        raise ValueError("reset= needs noise=ExplorationNoise")
+    return False
+
+
 def _noise_args(noise, noise_clip):
     sigma = float(noise)
     if not (sigma >= 0.0 and sigma != float("inf")):
@@ -90,6 +101,117 @@ def _noise_args(noise, noise_clip):
     if clip != clip:
         raise ValueError("noise_clip must not be NaN")
     return sigma, clip
+
+
+_UNCHANGED = object()
+
+
+class ExplorationNoise:
+    """Exploration noise for the fused actors (`FusedActor` / `FusedActorPool` with `noise=`): a per-slot AR(1) process
+    with per-row state on the device, drawn in the kernel's epilogue (hk_actor_forward_explore and _pool_explore):
+        x' = rho_s * x + scale_s * z,   act = clamp(actor(obs) + clip(x', +-clip_s), -1, 1),   x = 0 where `reset` is set
+    with z the normals of the Gaussian noisy call.  A Gaussian slot (theta=None) is rho = 0, scale = sigma: i.i.d.
+    noise, bit-identical to `noise=sigma`.  An Ornstein-Uhlenbeck slot dx = -theta x dt + sigma sqrt(dt) dW is
+    rho = 1 - theta dt, scale = sigma sqrt(dt).  A `FusedActor` uses slot 0; a pool uses slot s for the rows of
+    snapshot s (so a population explores with one slot per member).
+
+    `table` is the [slots, 4] float32 device table {rho, scale, clip, 0} (clip +inf: no clip) that the kernel reads at
+    every launch, so `set` (annealing, a PBT explore step) takes effect in a captured graph without re-capture.
+    `state` is the [n, 4] float32 process state, zeros at construction; `reset(mask)` zeroes rows.  The training loops
+    (`collect`, `td3.train`, `td3.train_population`) pass the previous step's done tensor as `reset=` and, before they
+    return, zero the rows whose episode ended on their last tick, so every episode starts from x = 0, across calls too.
+
+    Per-slot arguments are scalars or sequences of length `slots` (None entries allowed for clip and theta).
+
+    clip is a bound, not a switch: clip=None (or +inf) means no clip, and clip=0 clamps the added noise to zero, so the
+    actions are the policy's own while the state still evolves.  This differs from `noise=sigma, noise_clip=0` on the
+    Gaussian path, where noise_clip <= 0 means no clip: to carry such a setting over, pass clip=None."""
+
+    def __init__(self, n, slots=1, sigma=0.2, clip=None, theta=None, dt=1e-2, device="cuda:0"):
+        n, slots = int(n), int(slots)
+        if n < 1 or slots < 1:
+            raise ValueError("ExplorationNoise needs n >= 1 rows and slots >= 1")
+
+        def per_slot(name, v):
+            if isinstance(v, (list, tuple)) or (isinstance(v, torch.Tensor) and v.dim() > 0):
+                v = list(v)
+                if len(v) != slots:
+                    raise ValueError(f"ExplorationNoise: {name} has {len(v)} entries for {slots} slots")
+                return v
+            return [v] * slots
+
+        cols = [per_slot(nm, v) for nm, v in (("sigma", sigma), ("clip", clip), ("theta", theta), ("dt", dt))]
+        self._params = [dict(sigma=s, clip=c, theta=t, dt=d) for s, c, t, d in zip(*cols)]
+        rows = [self.slot_row(**p) for p in self._params]  # validated on the host before any device work
+        self.n, self.slots = n, slots
+        self.device = _cuda_device(device, "ExplorationNoise")
+        self.table = torch.tensor([r + (0.0,) for r in rows], dtype=torch.float32).to(self.device)
+        self.state = torch.zeros((n, 4), dtype=torch.float32, device=self.device)
+
+    @staticmethod
+    def slot_row(sigma, clip=None, theta=None, dt=1e-2):
+        """(rho, scale, clip) of one slot, computed in float64 and rounded once to float32 (returned as Python floats that
+        are exact float32 values).  Raises ValueError for sigma not finite or < 0, theta < 0, dt <= 0, theta * dt > 1 or
+        clip < 0 (None: no clip; 0: the added noise is clamped to zero)."""
+        import math
+        import numpy as np
+        sigma, dt = float(sigma), float(dt)
+        if not (math.isfinite(sigma) and sigma >= 0.0):
+            raise ValueError("ExplorationNoise: sigma must be finite and >= 0")
+        if not (math.isfinite(dt) and dt > 0.0):
+            raise ValueError("ExplorationNoise: dt must be finite and > 0")
+        if clip is not None and not float(clip) >= 0.0:
+            raise ValueError("ExplorationNoise: clip must be None or >= 0")
+        if theta is None:
+            rho, scale = 0.0, sigma
+        else:
+            theta = float(theta)
+            if not (math.isfinite(theta) and theta >= 0.0):
+                raise ValueError("ExplorationNoise: theta must be finite and >= 0")
+            if theta * dt > 1.0:
+                raise ValueError("ExplorationNoise: theta * dt must be <= 1")
+            rho, scale = 1.0 - theta * dt, sigma * math.sqrt(dt)
+        c = math.inf if clip is None else float(clip)
+        return tuple(float(np.float32(v)) for v in (rho, scale, c))
+
+    def set(self, slot, sigma=_UNCHANGED, clip=_UNCHANGED, theta=_UNCHANGED, dt=_UNCHANGED):
+        """Rewrite slot `slot` of the device table in place (three fills on the current stream: no host sync).  Omitted
+        arguments keep the slot's current value; clip=None means no clip, theta=None Gaussian.  The state is kept."""
+        slot = int(slot)
+        if not 0 <= slot < self.slots:
+            raise IndexError(f"ExplorationNoise slot {slot} out of range [0, {self.slots})")
+        p = dict(self._params[slot])
+        for name, v in (("sigma", sigma), ("clip", clip), ("theta", theta), ("dt", dt)):
+            if v is not _UNCHANGED:
+                p[name] = v
+        row = self.slot_row(**p)
+        self._params[slot] = p
+        with torch.cuda.device(self.device):
+            for j, v in enumerate(row):
+                self.table[slot, j].fill_(v)
+
+    def reset(self, mask=None):
+        """Zero the state of every row (mask None) or of the rows where `mask` ([n] bool / uint8 on the device) is set."""
+        if mask is None:
+            self.state.zero_()
+        else:
+            self.state.masked_fill_(mask.to(device=self.device, dtype=torch.bool).view(self.n, 1), 0.0)
+
+    def _launch_args(self, n, slots, device, reset, who):
+        """c_void_p of the table, the state and the reset mask (None or NULL) of a call over n rows that reads `slots`
+        slots; the reset tensor is returned too, to keep a converted copy alive across the launch."""
+        import ctypes as C
+        if self.n != n or self.device.type != device.type or (self.device.index or 0) != (device.index or 0):
+            raise ValueError(f"{who}: the ExplorationNoise holds {self.n} rows on {self.device}, the call has {n} on {device}")
+        if self.slots < slots:
+            raise ValueError(f"{who}: the ExplorationNoise has {self.slots} slots, the pool {slots} snapshots")
+        if reset is not None:
+            if not (isinstance(reset, torch.Tensor) and reset.device == device and reset.dtype in (torch.bool, torch.uint8)
+                    and reset.shape == (n,)):
+                raise ValueError(f"{who}: reset must be a bool or uint8 tensor [N] on the call's device (the previous done)")
+            reset = reset.contiguous().view(torch.uint8)
+        ptr = C.c_void_p(reset.data_ptr()) if reset is not None else None
+        return C.c_void_p(self.table.data_ptr()), C.c_void_p(self.state.data_ptr()), ptr, reset
 
 
 def _reference_state_dict(actor, who):
@@ -154,13 +276,16 @@ class FusedActor:
                  sd["fc2.bias"].contiguous().view(torch.uint8).flatten(), b3.view(torch.uint8).flatten()]
         return torch.cat(parts).contiguous()
 
-    def __call__(self, obs, out=None, noise=0.0, noise_clip=None, row0=0):
+    def __call__(self, obs, out=None, noise=0.0, noise_clip=None, row0=0, reset=None):
         """actions = actor(obs); with noise > 0, clamp(actor(obs) + clip(noise * z, +-noise_clip), -1, 1) (noise_clip None
         or <= 0: no clip), then the counter advances.  `row0` is the global index of row 0 (shards of one batch pass
-        their offset to draw the same noise as one call over the whole batch)."""
+        their offset to draw the same noise as one call over the whole batch).  noise=ExplorationNoise (of N rows):
+        exploration through its slot 0 and its state, with `reset` ([N] bool / uint8, e.g. the previous step's done,
+        or None) zeroing the state of the rows where it is set first; the clip is the slot's, the counter advances."""
         if not (obs.is_cuda and obs.dtype == torch.float32 and obs.is_contiguous() and obs.dim() == 2 and obs.shape[1] == 18):
             raise ValueError("FusedActor expects a contiguous float32 CUDA tensor [N, 18]")
-        sigma, clip = _noise_args(noise, noise_clip)
+        explore = _explore_args(noise, noise_clip, reset)
+        sigma, clip = (None, None) if explore else _noise_args(noise, noise_clip)
         n = obs.shape[0]
         if out is None:
             if self._out is None or self._out.shape[0] != n:
@@ -171,7 +296,13 @@ class FusedActor:
         C = self._C
         with torch.cuda.device(obs.device):
             stream = C.c_void_p(torch.cuda.current_stream(obs.device).cuda_stream)
-            if sigma == 0.0:
+            if explore:
+                table, state, rst, _keep = noise._launch_args(n, 1, obs.device, reset, "FusedActor")
+                self._lib.check(self.L.hk_actor_forward_explore(
+                    C.c_void_p(self.params.data_ptr()), C.c_void_p(obs.data_ptr()), C.c_void_p(out.data_ptr()), int(out.stride(0)), n,
+                    self.seed, C.c_void_p(self.counter.data_ptr()), table, state, rst, int(row0), obs.device.index or 0, stream))
+                self.counter.add_(1)
+            elif sigma == 0.0:
                 self._lib.check(self.L.hk_actor_forward(C.c_void_p(self.params.data_ptr()), C.c_void_p(obs.data_ptr()),
                                                         C.c_void_p(out.data_ptr()), int(out.stride(0)), n, obs.device.index or 0, stream))
             else:
@@ -231,15 +362,17 @@ class FusedActorPool:
             raise IndexError(f"FusedActorPool slot {i} out of range [0, {len(self)})")
         _pack_on_device(self.L, self._lib, actor, self.table[i], self.device, "FusedActorPool.set")
 
-    def __call__(self, obs, choice, out=None, noise=0.0, noise_clip=None, row0=0):
+    def __call__(self, obs, choice, out=None, noise=0.0, noise_clip=None, row0=0, reset=None):
         """obs [N,18] float32 CUDA, choice int32 / int64 CUDA [N] -> act[i] = actor_{choice[i]}(obs[i]) for choice[i] in
         [0, K); other rows are not written.  out=None: a persistent [N,4] buffer (overwritten by the next call) whose
         skipped rows are 0; or pass `out` = an [N, >= 4] float32 view with unit column stride (e.g. `a8[:, 4:]` of the
-        [N,8] action tensor): columns 0..3 of its written rows change, nothing else.  noise / noise_clip / row0 as for
-        `FusedActor`; a noisy call advances the counter."""
+        [N,8] action tensor): columns 0..3 of its written rows change, nothing else.  noise / noise_clip / row0 / reset
+        as for `FusedActor`; a noisy call advances the counter.  With noise=ExplorationNoise (>= K slots) the rows of
+        snapshot s explore with slot s; rows that are not written keep their state."""
         if not (obs.is_cuda and obs.dtype == torch.float32 and obs.is_contiguous() and obs.dim() == 2 and obs.shape[1] == 18):
             raise ValueError("FusedActorPool expects a contiguous float32 CUDA tensor [N, 18]")
-        sigma, clip = _noise_args(noise, noise_clip)
+        explore = _explore_args(noise, noise_clip, reset)
+        sigma, clip = (None, None) if explore else _noise_args(noise, noise_clip)
         n, k = obs.shape[0], len(self)
         if k == 0:
             raise ValueError("FusedActorPool is empty: add() a snapshot first")
@@ -266,7 +399,14 @@ class FusedActorPool:
         C = self._C
         with torch.cuda.device(obs.device):
             stream = C.c_void_p(torch.cuda.current_stream(obs.device).cuda_stream)
-            if sigma == 0.0:
+            if explore:
+                table, state, rst, _keep = noise._launch_args(n, k, obs.device, reset, "FusedActorPool")
+                self._lib.check(self.L.hk_actor_forward_pool_explore(
+                    C.c_void_p(self.table.data_ptr()), k, C.c_void_p(choice.data_ptr()), C.c_void_p(obs.data_ptr()),
+                    C.c_void_p(out.data_ptr()), int(out.stride(0)), n, C.c_void_p(self._scratch.data_ptr()), self.seed,
+                    C.c_void_p(self.counter.data_ptr()), table, state, rst, int(row0), obs.device.index or 0, stream))
+                self.counter.add_(1)
+            elif sigma == 0.0:
                 self._lib.check(self.L.hk_actor_forward_pool(C.c_void_p(self.table.data_ptr()), k, C.c_void_p(choice.data_ptr()),
                                                              C.c_void_p(obs.data_ptr()), C.c_void_p(out.data_ptr()), int(out.stride(0)),
                                                              n, C.c_void_p(self._scratch.data_ptr()), obs.device.index or 0, stream))

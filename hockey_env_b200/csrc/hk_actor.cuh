@@ -181,7 +181,7 @@ __device__ __forceinline__ void actorTeardown(const TileCtx& c) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// Exploration / target-policy-smoothing noise in the layer-3 epilogue (the `kNoisy` instantiations):
+// Exploration / target-policy-smoothing noise in the layer-3 epilogue (the `kGaussian` instantiations):
 //   act = clamp(tanh(MLP(obs)) + clip(sigma * z, -clip, clip), -1, 1),   z = four standard normals per row.
 // Row i's normals come from ONE Philox4x32-10 call, hk::philox(seed, row0 + i, (uint32_t)ctr,
 // HK_STREAM_ACTOR_NOISE | (uint32_t)(ctr >> 32) << 8), ctr = the call's counter (read from device memory, so a replayed
@@ -190,11 +190,26 @@ __device__ __forceinline__ void actorTeardown(const TileCtx& c) {
 //   r = sqrtf(-2 logf(u1)),   (z_even, z_odd) = (r cospif(2 u2), r sinpif(2 u2)).
 // A row's noise depends on its key only: not on n, the tile order or (in the pool) the grouping; `row0` lets shards of
 // one batch agree.  |z| <= sqrt(48 ln 2) ~ 5.77.
+//
+// Exploration (the `kExplore` instantiations): the same z drives a per-row AR(1) process whose state lives in device
+// memory, with (rho, scale, clip) taken from a slot table in device memory (float4 {rho, scale, clip, reserved} per slot;
+// the single-weight-set kernel reads slot 0, the pool kernel slot s for the rows of snapshot s):
+//   x  = reset[i] ? 0 : state[i][j]
+//   x' = fl(fl(rho * x) + fl(scale * z_j))        (rho == 0: x' = fl(scale * z_j); state and reset are not read)
+//   state[i][j] = x',   act[i][j] = clamp(tanh(MLP(obs[i]))_j + clip(x', +-clip), -1, 1)
+// rho = 0, scale = sigma is the Gaussian epilogue above bit for bit; OU noise dx = -theta x dt + sigma sqrt(dt) dW is
+// rho = 1 - theta dt, scale = sigma sqrt(dt).  `state` is indexed by the local row i (not row0 + i), `reset` may be NULL.
+// The table values are arithmetic operands only (never an index or a trip count), so any values are memory-safe.
+enum NoiseMode { kPlain, kGaussian, kExplore };
+
 struct NoiseKey {
   uint64_t seed;
   long long row0;
   uint32_t c2, c3;   // Philox counter words 2 and 3 (counter low word, stream tag | counter high bits << 8)
-  float sigma, clip; // clip = +inf: no clip
+  float sigma, clip; // clip = +inf: no clip.  kExplore: sigma is the slot's scale
+  float rho;                         // kExplore only: the slot's AR(1) coefficient
+  float4* state;                     // kExplore only: [n] rows of 4 f32
+  const uint8_t* reset;              // kExplore only: [n] or NULL
 };
 
 __device__ __forceinline__ NoiseKey noiseKey(uint64_t seed, const uint64_t* counter, float sigma, float clip, long long row0) {
@@ -224,12 +239,49 @@ __device__ __forceinline__ float addNoise(float a, float z, const NoiseKey& k) {
   return fminf(fmaxf(a + e, -1.0f), 1.0f);
 }
 
+// kExplore: a slot {rho, scale, clip, reserved} of the table into the key
+__device__ __forceinline__ void setSlot(NoiseKey& k, const float4& s) {
+  k.rho = s.x;
+  k.sigma = s.y;
+  k.clip = s.z;
+}
+
+__device__ __forceinline__ NoiseKey exploreKey(uint64_t seed, const uint64_t* counter, const float4* slots, float4* state,
+                                               const uint8_t* reset, long long row0) {
+  NoiseKey k = noiseKey(seed, counter, 0.0f, 0.0f, row0);
+  setSlot(k, slots[0]);
+  k.state = state;
+  k.reset = reset;
+  return k;
+}
+
+// kExplore: one AR(1) step of row `row` (see NoiseKey); returns x', the pre-clip state, and stores it.  The products and
+// the sum are rounded separately (__fmul_rn / __fadd_rn are never contracted into an FMA).
+__device__ __forceinline__ float4 exploreStep(long long row, float z0, float z1, float z2, float z3, const NoiseKey& k) {
+  float4 x = make_float4(__fmul_rn(k.sigma, z0), __fmul_rn(k.sigma, z1), __fmul_rn(k.sigma, z2), __fmul_rn(k.sigma, z3));
+  if (k.rho != 0.0f) {
+    float4 p = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    if (!(k.reset && k.reset[row])) p = k.state[row];
+    x.x = __fadd_rn(__fmul_rn(k.rho, p.x), x.x);
+    x.y = __fadd_rn(__fmul_rn(k.rho, p.y), x.y);
+    x.z = __fadd_rn(__fmul_rn(k.rho, p.z), x.z);
+    x.w = __fadd_rn(__fmul_rn(k.rho, p.w), x.w);
+  }
+  k.state[row] = x;
+  return x;
+}
+
+__device__ __forceinline__ float addExplore(float a, float x, const NoiseKey& k) {
+  const float e = fminf(fmaxf(x, -k.clip), k.clip);
+  return fminf(fmaxf(a + e, -1.0f), 1.0f);
+}
+
 // One tile of 128 rows through the three layers with the weights now in shared memory.  Thread t owns TMEM lane t; `row`
 // is the observation / action row it reads and writes, or -1 for a padding lane (zero input, nothing stored).  The only
 // thing the callers differ in is how a thread finds its row.  Ends in a block barrier: on return every MMA of the tile
-// has completed and every thread is done with the tile's shared memory (the weights may be replaced).  kNoisy adds the
-// noise of `nk` to the four outputs (see NoiseKey); the plain instantiation ignores `nk`.
-template <bool kNoisy>
+// has completed and every thread is done with the tile's shared memory (the weights may be replaced).  kGaussian adds the
+// noise of `nk` to the four outputs, kExplore its AR(1) exploration noise (see NoiseKey); kPlain ignores `nk`.
+template <NoiseMode kMode>
 __device__ __forceinline__ void actorTile(const TileCtx& c, uint32_t& phase, const float* __restrict__ obs,
                                           float* __restrict__ act, int actStride, long long row, const NoiseKey& nk) {
   const int t = threadIdx.x;
@@ -309,7 +361,7 @@ __device__ __forceinline__ void actorTile(const TileCtx& c, uint32_t& phase, con
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
     if (row >= 0) {
       float* dst = act + row * actStride;
-      if constexpr (kNoisy) {
+      if constexpr (kMode == kGaussian) {
         const hk::U4 w = hk::philox(nk.seed, (uint64_t)(nk.row0 + row), nk.c2, nk.c3);
         float z0, z1, z2, z3;
         boxMuller(w.x, w.y, z0, z1);
@@ -318,6 +370,16 @@ __device__ __forceinline__ void actorTile(const TileCtx& c, uint32_t& phase, con
         dst[1] = addNoise(tanhApprox(__uint_as_float(r1) + b3[1]), z1, nk);
         dst[2] = addNoise(tanhApprox(__uint_as_float(r2) + b3[2]), z2, nk);
         dst[3] = addNoise(tanhApprox(__uint_as_float(r3) + b3[3]), z3, nk);
+      } else if constexpr (kMode == kExplore) {
+        const hk::U4 w = hk::philox(nk.seed, (uint64_t)(nk.row0 + row), nk.c2, nk.c3);
+        float z0, z1, z2, z3;
+        boxMuller(w.x, w.y, z0, z1);
+        boxMuller(w.z, w.w, z2, z3);
+        const float4 x = exploreStep(row, z0, z1, z2, z3, nk);
+        dst[0] = addExplore(tanhApprox(__uint_as_float(r0) + b3[0]), x.x, nk);
+        dst[1] = addExplore(tanhApprox(__uint_as_float(r1) + b3[1]), x.y, nk);
+        dst[2] = addExplore(tanhApprox(__uint_as_float(r2) + b3[2]), x.z, nk);
+        dst[3] = addExplore(tanhApprox(__uint_as_float(r3) + b3[3]), x.w, nk);
       } else {
         dst[0] = tanhApprox(__uint_as_float(r0) + b3[0]);
         dst[1] = tanhApprox(__uint_as_float(r1) + b3[1]);
@@ -331,7 +393,7 @@ __device__ __forceinline__ void actorTile(const TileCtx& c, uint32_t& phase, con
 }
 
 // one weight set, rows 0..n-1 in order: tile `tile` holds rows tile * 128 + t
-template <bool kNoisy>
+template <NoiseMode kMode>
 __device__ __forceinline__ void actorMlp(const unsigned char* __restrict__ params, const float* __restrict__ obs,
                                          float* __restrict__ act, int actStride, long long n, const NoiseKey& nk) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -341,21 +403,29 @@ __device__ __forceinline__ void actorMlp(const unsigned char* __restrict__ param
   const long long tiles = (n + kRows - 1) / kRows;
   for (long long tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
     const long long row = tile * kRows + threadIdx.x;
-    actorTile<kNoisy>(c, phase, obs, act, actStride, row < n ? row : -1, nk);
+    actorTile<kMode>(c, phase, obs, act, actStride, row < n ? row : -1, nk);
   }
   actorTeardown(c);
 }
 
 __global__ void __launch_bounds__(kThreads, 1) k_actor_mlp(const unsigned char* __restrict__ params, const float* __restrict__ obs,
                                                            float* __restrict__ act, int actStride, long long n) {
-  actorMlp<false>(params, obs, act, actStride, n, NoiseKey{});
+  actorMlp<kPlain>(params, obs, act, actStride, n, NoiseKey{});
 }
 
 __global__ void __launch_bounds__(kThreads, 1) k_actor_mlp_noisy(const unsigned char* __restrict__ params, const float* __restrict__ obs,
                                                                  float* __restrict__ act, int actStride, long long n, uint64_t seed,
                                                                  const uint64_t* __restrict__ counter, float sigma, float clip,
                                                                  long long row0) {
-  actorMlp<true>(params, obs, act, actStride, n, noiseKey(seed, counter, sigma, clip, row0));
+  actorMlp<kGaussian>(params, obs, act, actStride, n, noiseKey(seed, counter, sigma, clip, row0));
+}
+
+__global__ void __launch_bounds__(kThreads, 1) k_actor_mlp_explore(const unsigned char* __restrict__ params, const float* __restrict__ obs,
+                                                                   float* __restrict__ act, int actStride, long long n, uint64_t seed,
+                                                                   const uint64_t* __restrict__ counter, const float4* __restrict__ slots,
+                                                                   float4* __restrict__ state, const uint8_t* __restrict__ reset,
+                                                                   long long row0) {
+  actorMlp<kExplore>(params, obs, act, actStride, n, exploreKey(seed, counter, slots, state, reset, row0));
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -475,10 +545,11 @@ __global__ void __launch_bounds__(kPoolThreads) k_pool_scatter(const int32_t* __
 // Persistent: CTA b walks the contiguous tile range [b T / G, (b + 1) T / G) of the T = tileOff[K] tiles, so it crosses few
 // group boundaries; it copies a snapshot's weights into shared memory only when the group changes.  Tile j of group s holds
 // rows[groupOff[s] + j * 128 + t]; lanes past the group's end are padding.
-template <bool kNoisy>
+// kExplore: `slots` is the slot table (slot s for the rows of snapshot s); the other modes pass NULL.
+template <NoiseMode kMode>
 __device__ __forceinline__ void actorPoolMlp(const unsigned char* __restrict__ params, int k, const int32_t* __restrict__ scratch,
                                              const float* __restrict__ obs, float* __restrict__ act, int actStride,
-                                             const NoiseKey& nk) {
+                                             const NoiseKey& nk, const float4* __restrict__ slots) {
   extern __shared__ __align__(128) unsigned char smem[];
   const int32_t* groupOff = scratch + poolOffGroup(k);
   const int32_t* tileOff = scratch + poolOffTile(k);
@@ -494,16 +565,18 @@ __device__ __forceinline__ void actorPoolMlp(const unsigned char* __restrict__ p
   }
   int s = lo, loaded = -1;
   uint32_t phase = 0;
+  NoiseKey key = nk;
   for (long long tile = t0; tile < t1; ++tile) {
     while (tile >= tileOff[s + 1]) ++s;
     if (s != loaded) {
       // the previous tile (if any) ended with its layer-3 MMAs complete and a block barrier: the old weights are dead
       loadParams(smem, params + (size_t)s * kParamBytes);
+      if constexpr (kMode == kExplore) setSlot(key, slots[s]);  // uniform over the tile: the rho == 0 branch does not diverge
       loaded = s;
     }
     const int local = (int)(tile - tileOff[s]) * kRows + threadIdx.x;
     const int count = groupOff[s + 1] - groupOff[s];
-    actorTile<kNoisy>(c, phase, obs, act, actStride, local < count ? (long long)rows[groupOff[s] + local] : -1LL, nk);
+    actorTile<kMode>(c, phase, obs, act, actStride, local < count ? (long long)rows[groupOff[s] + local] : -1LL, key);
   }
   actorTeardown(c);
 }
@@ -511,7 +584,7 @@ __device__ __forceinline__ void actorPoolMlp(const unsigned char* __restrict__ p
 __global__ void __launch_bounds__(kThreads, 1) k_actor_pool_mlp(const unsigned char* __restrict__ params, int k,
                                                                 const int32_t* __restrict__ scratch, const float* __restrict__ obs,
                                                                 float* __restrict__ act, int actStride) {
-  actorPoolMlp<false>(params, k, scratch, obs, act, actStride, NoiseKey{});
+  actorPoolMlp<kPlain>(params, k, scratch, obs, act, actStride, NoiseKey{}, nullptr);
 }
 
 __global__ void __launch_bounds__(kThreads, 1) k_actor_pool_mlp_noisy(const unsigned char* __restrict__ params, int k,
@@ -519,7 +592,19 @@ __global__ void __launch_bounds__(kThreads, 1) k_actor_pool_mlp_noisy(const unsi
                                                                       float* __restrict__ act, int actStride, uint64_t seed,
                                                                       const uint64_t* __restrict__ counter, float sigma, float clip,
                                                                       long long row0) {
-  actorPoolMlp<true>(params, k, scratch, obs, act, actStride, noiseKey(seed, counter, sigma, clip, row0));
+  actorPoolMlp<kGaussian>(params, k, scratch, obs, act, actStride, noiseKey(seed, counter, sigma, clip, row0), nullptr);
+}
+
+__global__ void __launch_bounds__(kThreads, 1) k_actor_pool_mlp_explore(const unsigned char* __restrict__ params, int k,
+                                                                        const int32_t* __restrict__ scratch, const float* __restrict__ obs,
+                                                                        float* __restrict__ act, int actStride, uint64_t seed,
+                                                                        const uint64_t* __restrict__ counter, const float4* __restrict__ slots,
+                                                                        float4* __restrict__ state, const uint8_t* __restrict__ reset,
+                                                                        long long row0) {
+  NoiseKey nk = noiseKey(seed, counter, 0.0f, 0.0f, row0);
+  nk.state = state;
+  nk.reset = reset;
+  actorPoolMlp<kExplore>(params, k, scratch, obs, act, actStride, nk, slots);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

@@ -2043,6 +2043,21 @@ static int poolCheck(const char* who, const void* params_dev, int k, const int32
   return HK_OK;
 }
 
+// The grouping kernels (row lists per snapshot in `scratch`) on `st`; returns HK_OK and the grid of the pooled
+// tensor-core kernel in *grid.
+static int poolGroup(const int32_t* choice_dev, int64_t n, int k, int32_t* scratch, int sms, cudaStream_t st, int64_t* grid) {
+  using namespace hk_actor;
+  HK_CUDA(cudaMemsetAsync(scratch, 0, sizeof(int32_t) * (size_t)k, st));  // counts
+  const int64_t chunks = (n + kPoolThreads * kPoolItems - 1) / (kPoolThreads * kPoolItems);
+  const unsigned histBlocks = (unsigned)std::min<int64_t>(chunks, 4 * (int64_t)sms);
+  k_pool_count<<<histBlocks, kPoolThreads, sizeof(int32_t) * (size_t)k, st>>>(choice_dev, (long long)n, k, scratch);
+  k_pool_scan<<<1, kScanThreads, 0, st>>>(scratch, k);
+  k_pool_scatter<<<histBlocks, kPoolThreads, 2 * sizeof(int32_t) * (size_t)k, st>>>(choice_dev, (long long)n, k, scratch);
+  // the tile count is only known on the device: at most ceil(n / 128) + k - 1 tiles (one partial tile per group)
+  *grid = std::min<int64_t>(sms, (n + kRows - 1) / kRows + k);
+  return HK_OK;
+}
+
 // The grouping kernels, then the pooled tensor-core kernel; sigma == 0 runs the plain one (bit-identical to
 // hk_actor_forward_pool).
 static int poolLaunch(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev, int act_stride,
@@ -2054,17 +2069,10 @@ static int poolLaunch(const void* params_dev, int k, const int32_t* choice_dev, 
   static bool configured[64] = {false}, configuredNoisy[64] = {false};
   if (int rc = withNoise ? actorConfigure((const void*)k_actor_pool_mlp_noisy, configuredNoisy, device) : actorConfigure((const void*)k_actor_pool_mlp, configured, device))
     return rc;
-  const int sms = actorSms(device);
   cudaStream_t st = (cudaStream_t)stream;
   int32_t* scratch = (int32_t*)scratch_dev;
-  HK_CUDA(cudaMemsetAsync(scratch, 0, sizeof(int32_t) * (size_t)k, st));  // counts
-  const int64_t chunks = (n + kPoolThreads * kPoolItems - 1) / (kPoolThreads * kPoolItems);
-  const unsigned histBlocks = (unsigned)std::min<int64_t>(chunks, 4 * (int64_t)sms);
-  k_pool_count<<<histBlocks, kPoolThreads, sizeof(int32_t) * (size_t)k, st>>>(choice_dev, (long long)n, k, scratch);
-  k_pool_scan<<<1, kScanThreads, 0, st>>>(scratch, k);
-  k_pool_scatter<<<histBlocks, kPoolThreads, 2 * sizeof(int32_t) * (size_t)k, st>>>(choice_dev, (long long)n, k, scratch);
-  // the tile count is only known on the device: at most ceil(n / 128) + k - 1 tiles (one partial tile per group)
-  const int64_t grid = std::min<int64_t>(sms, (n + kRows - 1) / kRows + k);
+  int64_t grid = 0;
+  if (int rc = poolGroup(choice_dev, n, k, scratch, actorSms(device), st, &grid)) return rc;
   if (withNoise)
     k_actor_pool_mlp_noisy<<<(unsigned)grid, kThreads, kSmemBytes, st>>>((const unsigned char*)params_dev, k, scratch, obs_dev, act_dev,
                                                                          act_stride, seed, counter_dev, sigma, effectiveClip(clip), (long long)row0);
@@ -2091,6 +2099,58 @@ int hk_actor_forward_pool_noisy(const void* params_dev, int k, const int32_t* ch
   if (int rc = deviceCheck(who, device)) return rc;
   return poolLaunch(params_dev, k, choice_dev, obs_dev, act_dev, act_stride, n, scratch_dev, true, seed, counter_dev, sigma, clip, row0,
                     device, stream);
+}
+
+// the explore entry points: counter, slot table and state (reset may be NULL)
+static int exploreCheck(const char* who, const uint64_t* counter_dev, const float* slots_dev, const float* state_dev, int64_t row0) {
+  if (!counter_dev || !slots_dev || !state_dev) return fail(HK_E_INVALID, std::string(who) + ": NULL argument");
+  if (((uintptr_t)counter_dev) & 7u) return fail(HK_E_INVALID, std::string(who) + ": counter needs 8-byte alignment");
+  if ((((uintptr_t)slots_dev) & 15u) || (((uintptr_t)state_dev) & 15u))
+    return fail(HK_E_INVALID, std::string(who) + ": slots and state need 16-byte alignment");
+  if (row0 < 0) return fail(HK_E_INVALID, std::string(who) + ": row0 must be >= 0");
+  return HK_OK;
+}
+
+int hk_actor_forward_explore(const void* params_dev, const float* obs_dev, float* act_dev, int act_stride, int64_t n, uint64_t seed,
+                             const uint64_t* counter_dev, const float* slots_dev, float* state_dev, const uint8_t* reset_dev,
+                             int64_t row0, int device, void* stream) {
+  const char* who = "hk_actor_forward_explore";
+  if (int rc = actorCheck(who, params_dev, obs_dev, act_dev, act_stride, n)) return rc;
+  if (int rc = exploreCheck(who, counter_dev, slots_dev, state_dev, row0)) return rc;
+  if (int rc = deviceCheck(who, device)) return rc;
+  using namespace hk_actor;
+  DeviceGuard guard(device);
+  static bool configured[64] = {false};
+  if (int rc = actorConfigure((const void*)k_actor_mlp_explore, configured, device)) return rc;
+  const unsigned grid = (unsigned)std::min<int64_t>((n + kRows - 1) / kRows, actorSms(device));
+  k_actor_mlp_explore<<<grid, kThreads, kSmemBytes, (cudaStream_t)stream>>>(
+      (const unsigned char*)params_dev, obs_dev, act_dev, act_stride, (long long)n, seed, counter_dev, (const float4*)slots_dev,
+      (float4*)state_dev, reset_dev, (long long)row0);
+  HK_CUDA(cudaGetLastError());
+  return HK_OK;
+}
+
+int hk_actor_forward_pool_explore(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev, float* act_dev,
+                                  int act_stride, int64_t n, void* scratch_dev, uint64_t seed, const uint64_t* counter_dev,
+                                  const float* slots_dev, float* state_dev, const uint8_t* reset_dev, int64_t row0, int device,
+                                  void* stream) {
+  const char* who = "hk_actor_forward_pool_explore";
+  if (int rc = poolCheck(who, params_dev, k, choice_dev, obs_dev, act_dev, act_stride, n, scratch_dev)) return rc;
+  if (int rc = exploreCheck(who, counter_dev, slots_dev, state_dev, row0)) return rc;
+  if (int rc = deviceCheck(who, device)) return rc;
+  using namespace hk_actor;
+  DeviceGuard guard(device);
+  static bool configured[64] = {false};
+  if (int rc = actorConfigure((const void*)k_actor_pool_mlp_explore, configured, device)) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  int32_t* scratch = (int32_t*)scratch_dev;
+  int64_t grid = 0;
+  if (int rc = poolGroup(choice_dev, n, k, scratch, actorSms(device), st, &grid)) return rc;
+  k_actor_pool_mlp_explore<<<(unsigned)grid, kThreads, kSmemBytes, st>>>((const unsigned char*)params_dev, k, scratch, obs_dev, act_dev,
+                                                               act_stride, seed, counter_dev, (const float4*)slots_dev,
+                                                               (float4*)state_dev, reset_dev, (long long)row0);
+  HK_CUDA(cudaGetLastError());
+  return HK_OK;
 }
 
 int hk_actor_pack(const float* w1, const float* b1, const float* w2, const float* b2, const float* w3, const float* b3, void* params_dev,

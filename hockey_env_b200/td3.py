@@ -609,7 +609,7 @@ def _explore(actor, obs, noise_scale, gen):
     return (a + torch.randn(a.shape, device=a.device, generator=gen) * noise_scale).clamp(-1, 1)
 
 
-def train(env_or_pool, learner, ticks, updates_per_tick=1, noise_scale=None, warmup_ticks=8, fused=False):
+def train(env_or_pool, learner, ticks, updates_per_tick=1, noise_scale=None, warmup_ticks=8, fused=False, noise=None):
     """Batched form of TD3Trainer's loop (rl/training/train.py:135-172): every tick all envs act with Gaussian
     exploration noise, their transitions (terminal observation as next_obs on done) go to the learner's device replay
     buffer, and `updates_per_tick` learner steps follow.  Returns the mean critic loss of the last tick (device scalar).
@@ -618,9 +618,19 @@ def train(env_or_pool, learner, ticks, updates_per_tick=1, noise_scale=None, war
     use, seeded with the learner's seed), with the exploration noise drawn in the kernel: one launch per tick.  The
     mirror is repacked on the device (`FusedActor.refresh`: no host sync) at the start of the call and after every tick
     whose updates changed the actor, so every tick acts with the current weights.  The learner itself still trains the
-    fp32 module; only the behaviour policy runs in bf16 / TF32 (TD3 is off-policy)."""
+    fp32 module; only the behaviour policy runs in bf16 / TF32 (TD3 is off-policy).
+
+    noise: an `ExplorationNoise` of N rows (fused=True only, instead of noise_scale): the envs explore with its slot 0
+    (e.g. Ornstein-Uhlenbeck noise), each tick passes the previous tick's done as `reset`, and the rows whose episode
+    ended on the last tick are zeroed before returning, so every episode starts from a zero noise state, across calls
+    too.  `noise.set(0, sigma=...)` between calls anneals it."""
     from .actor import FusedActor
     from .training import OpponentPool
+    if noise is not None:
+        if noise_scale is not None:
+            raise ValueError("train: pass either noise_scale= or noise=, not both")
+        if not fused:
+            raise ValueError("train: noise=ExplorationNoise needs fused=True (its state exists only in the fused launch)")
     pool = env_or_pool if isinstance(env_or_pool, OpponentPool) else None
     env = pool.env if pool else env_or_pool
     buf = learner.replay_buffer
@@ -631,9 +641,11 @@ def train(env_or_pool, learner, ticks, updates_per_tick=1, noise_scale=None, war
             learner.fused_actor = FusedActor(learner.actor, device=learner.device, seed=learner.seed)
         mirror = learner.fused_actor.refresh(learner.actor)
     obs = env.obs.clone()
-    loss = None
+    loss = done = None
     for t in range(ticks):
-        if mirror is not None:
+        if noise is not None:
+            a = mirror(obs, noise=noise, reset=done)
+        elif mirror is not None:
             a = mirror(obs, noise=scale)
         else:
             a = _explore(learner.actor, obs, scale, learner.gen)
@@ -648,17 +660,24 @@ def train(env_or_pool, learner, ticks, updates_per_tick=1, noise_scale=None, war
                 changed |= actor_loss is not None
             if changed and mirror is not None:
                 mirror.refresh(learner.actor)
+    if noise is not None and done is not None:
+        noise.reset(done)  # episodes that ended on the last tick start the next call from x = 0
     return loss
 
 
-def train_population(env_or_pool, population, ticks, updates_per_tick=1, noise_scale=None, warmup_ticks=8):
+def train_population(env_or_pool, population, ticks, updates_per_tick=1, noise_scale=None, warmup_ticks=8, noise=None):
     """`train(..., fused=True)` for a `FusedTD3Population`: the env's N rows are split into K equal contiguous blocks, and
     block m acts through member m -- one noisy `FusedActorPool` launch per tick with the constant choice row // (N / K),
     exploration noise keyed on the global row.  The transitions go to the population's buffer (block m to member m),
     `updates_per_tick` population launches follow each tick after `warmup_ticks`, and after a tick whose updates stepped
-    any actor one hk_actor_pack_many launch repacks all K slots.  The exploration sigma is one scalar for the population
-    (noise_scale, or the members' action_noise_scale, which must then be equal).  An `OpponentPool` works as with
-    `train` (player-1 columns only).  Returns the [K] critic losses of the last update (device tensor; None if none ran)."""
+    any actor one hk_actor_pack_many launch repacks all K slots.  Without `noise=`, the exploration sigma is one scalar for the
+    population (noise_scale, or the members' action_noise_scale, which must then be equal).  An `OpponentPool` works as with
+    `train` (player-1 columns only).  Returns the [K] critic losses of the last update (device tensor; None if none ran).
+
+    noise: an `ExplorationNoise` of N rows and K slots (instead of noise_scale): block m explores with slot m, so the
+    members may explore differently (their action_noise_scale is then not consulted), and each tick passes the previous
+    tick's done as `reset` (rows whose episode ended on the last tick are zeroed before returning, as in `train`).
+    `noise.set(m, ...)` changes member m's exploration (a PBT explore step) between calls."""
     from .actor import FusedActorPool
     from .training import OpponentPool
     pool = env_or_pool if isinstance(env_or_pool, OpponentPool) else None
@@ -666,7 +685,13 @@ def train_population(env_or_pool, population, ticks, updates_per_tick=1, noise_s
     k, n = population.k, env.num_envs
     if n % k:
         raise ValueError(f"train_population: {n} envs do not split into {k} equal blocks")
-    if noise_scale is None:
+    if noise is not None:
+        if noise_scale is not None:
+            raise ValueError("train_population: pass either noise_scale= or noise=, not both")
+        if noise.slots != k or noise.n != n:
+            raise ValueError(f"train_population: noise= needs an ExplorationNoise of {n} rows and {k} slots (one per member), "
+                             f"got {noise.n} rows and {noise.slots} slots")
+    elif noise_scale is None:
         scales = {c.action_noise_scale for c in population.configs}
         if len(scales) != 1:
             raise ValueError(f"train_population: the members' action_noise_scale differ ({sorted(scales)}); the pooled actor "
@@ -679,9 +704,12 @@ def train_population(env_or_pool, population, ticks, updates_per_tick=1, noise_s
     acting = population.refresh_pool(population.fused_pool)
     choice = (torch.arange(n, device=env.device) // (n // k)).to(torch.int32)
     obs = env.obs.clone()
-    loss = None
+    loss = done = None
     for t in range(ticks):
-        a = acting(obs, choice, noise=noise_scale)
+        if noise is not None:
+            a = acting(obs, choice, noise=noise, reset=done)
+        else:
+            a = acting(obs, choice, noise=noise_scale)
         nobs, reward, done, _, _ = pool.step(a) if pool else env.step(a.contiguous())
         nxt = torch.where(done.to(torch.bool).unsqueeze(1), env.final_obs, nobs) if env.final_obs is not None else nobs
         buf.push(obs, a, reward, nxt, done)
@@ -693,4 +721,6 @@ def train_population(env_or_pool, population, ticks, updates_per_tick=1, noise_s
                 changed |= any(population.last_do_actor)
             if changed:
                 population.refresh_pool(acting)
+    if noise is not None and done is not None:
+        noise.reset(done)  # episodes that ended on the last tick start the next call from x = 0
     return loss

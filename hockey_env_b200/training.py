@@ -20,7 +20,7 @@ The dense networks are plain torch modules (library matmuls): they are the ops n
 import torch
 
 from . import _lib
-from .actor import FusedActor, FusedActorPool
+from .actor import ExplorationNoise, FusedActor, FusedActorPool
 from .env import HockeyVecEnv, Mode
 
 
@@ -219,10 +219,15 @@ class DeviceReplayBuffer:
         return self.obs[idx], self.action[idx], self.reward[idx], self.next_obs[idx], self.done[idx]
 
 
-def behaviour_actions(actor, obs, noise=0.0):
+def behaviour_actions(actor, obs, noise=0.0, reset=None):
     """The behaviour policy of one tick: actor(obs), plus Gaussian exploration noise of std `noise` clamped to [-1, 1]
     when noise > 0.  A `FusedActor` draws the noise in its kernel epilogue (one launch); any other module runs, then
-    torch's randn / add / clamp."""
+    torch's randn / add / clamp.  noise=ExplorationNoise (a `FusedActor` only: its state lives in the fused launch)
+    explores through slot 0, with `reset` = the previous step's done tensor (None on the first tick)."""
+    if isinstance(noise, ExplorationNoise):
+        if not isinstance(actor, FusedActor):
+            raise ValueError("noise=ExplorationNoise needs a FusedActor: the noise state exists only in the fused launch")
+        return actor(obs, noise=noise, reset=reset)
     if not noise:
         return actor(obs)
     if isinstance(actor, FusedActor):
@@ -234,17 +239,21 @@ def behaviour_actions(actor, obs, noise=0.0):
 @torch.no_grad()
 def collect(pool_or_env, actor, buffer, steps, noise=0.0):
     """`steps` ticks of experience collection: actor -> env -> buffer, all on the device.  `actor` is a module or a
-    `FusedActor`; `noise` > 0 adds Gaussian exploration noise of that std (see `behaviour_actions`).  With auto-reset
+    `FusedActor`; `noise` > 0 adds Gaussian exploration noise of that std (see `behaviour_actions`), an
+    `ExplorationNoise` its per-env process, reset for the envs whose episode ended on the previous tick.  With auto-reset
     the transition of a finished episode stores the TERMINAL observation (`final_obs`) as next_obs, as the reference's
     loop does (rl/training/train.py:136-160)."""
     env = pool_or_env.env if isinstance(pool_or_env, OpponentPool) else pool_or_env
     obs = env.obs.clone()
+    done = None
     for _ in range(steps):
-        a1 = behaviour_actions(actor, obs, noise)
+        a1 = behaviour_actions(actor, obs, noise, reset=done if isinstance(noise, ExplorationNoise) else None)
         nobs, reward, done, _, _ = pool_or_env.step(a1) if isinstance(pool_or_env, OpponentPool) else env.step(a1.contiguous())
         nxt = torch.where(done.to(torch.bool).unsqueeze(1), env.final_obs, nobs) if env.final_obs is not None else nobs
         buffer.push(obs, a1, reward, nxt, done)
         obs = nobs.clone()
+    if isinstance(noise, ExplorationNoise) and done is not None:
+        noise.reset(done)  # episodes that ended on the last tick start the next call from x = 0
     return buffer
 
 

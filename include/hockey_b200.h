@@ -248,6 +248,30 @@ int hk_actor_forward_pool_noisy(const void* params_dev, int k, const int32_t* ch
                                 int act_stride, int64_t n, void* scratch_dev, uint64_t seed, const uint64_t* counter_dev, float sigma,
                                 float clip, int64_t row0, int device, void* stream);
 
+/* The same two kernels with exploration noise from a per-slot AR(1) process whose state lives on the device (Gaussian
+ * and Ornstein-Uhlenbeck exploration, set per slot).  For each written row i (local index, 0 <= i < n) and column j:
+ *   x    = reset[i] ? 0 : state[i][j]
+ *   x'   = fl(fl(rho_s * x) + fl(scale_s * z_ij))       (rho_s == 0: x' = fl(scale_s * z_ij); state and reset not read)
+ *   state[i][j] = x'                                     (before the clip; written for every row the call writes)
+ *   act[i][j]   = clamp(tanh(MLP(obs[i]))_j + clip(x', +-clip_s), -1, 1)
+ * z_ij are the normals of hk_actor_forward_noisy (same key: seed, row0 + i, *counter_dev), so a slot with rho = 0,
+ * scale = sigma, clip = c gives actions bit-identical to hk_actor_forward_noisy(sigma, c) for c > 0.  OU noise
+ * dx = -theta x dt + sigma sqrt(dt) dW is rho = 1 - theta dt, scale = sigma sqrt(dt).
+ * slots_dev: f32 {rho, scale, clip, reserved} per slot (16-byte aligned; clip = +inf: no clip), READ ON THE DEVICE AT
+ * EVERY LAUNCH, so rewriting it changes the noise of a captured graph's next replay.  hk_actor_forward_explore reads
+ * slot 0; hk_actor_forward_pool_explore reads slot s for the rows with choice s (the table holds >= k slots).
+ * state_dev: f32 [n, 4] (16-byte aligned), indexed by the local row; rows the call does not write (pool choice outside
+ * [0, k)) keep their state.  reset_dev: u8 [n] or NULL (e.g. the done tensor of the previous hk_step).  Table values
+ * are never used as indices: out-of-contract values give unspecified actions, not a fault.  Other arguments and error
+ * rules as for the noisy calls; no allocation, no host synchronisation; graph-capturable. */
+int hk_actor_forward_explore(const void* params_dev, const float* obs_dev, float* act_dev, int act_stride, int64_t n,
+                             uint64_t seed, const uint64_t* counter_dev, const float* slots_dev, float* state_dev,
+                             const uint8_t* reset_dev, int64_t row0, int device, void* stream);
+int hk_actor_forward_pool_explore(const void* params_dev, int k, const int32_t* choice_dev, const float* obs_dev,
+                                  float* act_dev, int act_stride, int64_t n, void* scratch_dev, uint64_t seed,
+                                  const uint64_t* counter_dev, const float* slots_dev, float* state_dev,
+                                  const uint8_t* reset_dev, int64_t row0, int device, void* stream);
+
 /* Pack an ActorNetwork's fp32 parameters on the device into one hk_actor_param_bytes() block, byte-identical to
  * hockey_env_b200.actor.FusedActor.pack: w1 [256, 18], b1 [256], w2 [256, 256], b2 [256], w3 [4, 256], b3 [4], contiguous
  * f32 device arrays (4-byte aligned).  params_dev: 16-byte aligned; may point into a pool table (slot s at
