@@ -99,6 +99,7 @@ HK_NI_FASTA void tickFinish(const Scene& S, const Config& cfg, Env& e, uint64_t 
   st.velIters += (int)e.nVelIters;
   st.toi += (int)e.nToiEvents;
   st.overflow += (int)e.nOverflow;
+  HK_WORK(g_work.sweeps = (int)e.nVelIters; g_work.toi = (int)e.nToiEvents; g_work.goal = e.done && e.winner != 0);
   e.nVelIters = e.nToiEvents = e.nOverflow = 0;
   if (e.has1 == HK_MAX_TIME_KEEP_PUCK && had1 != HK_MAX_TIME_KEEP_PUCK) st.touch1 += 1;
   if (e.has2 == HK_MAX_TIME_KEEP_PUCK && had2 != HK_MAX_TIME_KEEP_PUCK) st.touch2 += 1;

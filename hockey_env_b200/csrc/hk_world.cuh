@@ -26,7 +26,18 @@ extern long long g_toi_dbg[16];
 #define HK_TOI_DBG(k) g_toi_dbg[k]++
 #define HK_ITER_HIST(w, n) g_iter_hist[w][n]++
 #define HK_NVC_HIST(n) g_nvc_hist[n]++
+// work record of the tick being stepped (the host build steps one env at a time; tests/hostsim copies it out per env):
+// kind = island solve (1..8: solveKind, 9 / 10: one contact with one / two points, 11: generic loop, 0: none), shape =
+// its dbgShape, sweeps / toi = the tick's velocity sweeps and TOI events, maxSub = the highest TOI sub-step count of any
+// pair, skipAfter = TOI evaluations skipped by toiSeparatedAfterEvent, events = bit 0: a puck x static event, bit 1: a
+// racket x static event, goal = the tick ended the episode with a winner
+struct WorkRecord {
+  int kind, shape, sweeps, toi, maxSub, skipAfter, events, goal;
+};
+inline WorkRecord g_work;  // defined here: a host build that never reads it needs no definition of its own
+#define HK_WORK(...) __VA_ARGS__
 #else
+#define HK_WORK(...)
 #define HK_ITER_HIST(w, n)
 #define HK_NVC_HIST(n)
 #define HK_TOI_DBG(k)
@@ -1778,6 +1789,7 @@ HK_HD_NOINLINE void solveIslandsEnd(const Scene& S, Env& e, float h, int posIter
     }
     HK_ITER_HIST(0, itc);
     HK_NVC_HIST(nvc);
+    HK_WORK(g_work.kind = nvc == 1 ? 8 + vcs[0].count : (solveKind(vcs, nvc) ? solveKind(vcs, nvc) : 11); g_work.shape = (int)e.dbgShape);
     // StoreImpulses
     for (int k = 0; k < nvc; ++k) {
       Manifold& m = e.mf[vcs[k].slot];
@@ -2097,8 +2109,10 @@ HK_HD_NOINLINE void solveTOI(const Scene& S, const Config& cfg, const Cache& cac
         // target + tolerance (+ margin) the answer is alpha = 1.
         bool skip = !e.toiEventSeen && alpha0 == 0.0f && ((solvedMask >> bi) & 1u) &&
                     toiProvablySeparated(S, e, pid, fA, bi, pB.radius);
-        if (!skip && bi == freshBody && (freshMask & bit) && sepKnown(e, pid))
+        if (!skip && bi == freshBody && (freshMask & bit) && sepKnown(e, pid)) {
           skip = toiSeparatedAfterEvent(S, e, pid, bi, pB.radius, freshC, freshA);
+          HK_WORK(g_work.skipAfter += skip ? 1 : 0);
+        }
         HK_TOI_DBG(bi == B_PUCK ? 0 : 1);
         if (skip) {
           state = TOI_SEPARATED;
@@ -2155,6 +2169,11 @@ HK_HD_NOINLINE void solveTOI(const Scene& S, const Config& cfg, const Cache& cac
     updateContact(S, cfg, cache, e, minPid);
     toiFlag &= ~(1u << minPid);
     if (minPid < 16) toiCountLo += 1ull << (4 * minPid); else toiCountHi += 1ull << (4 * (minPid - 16));
+    HK_WORK({
+      const int sub = (int)(((minPid < 16 ? toiCountLo : toiCountHi) >> (4 * (minPid & 15))) & 15u);
+      if (sub > g_work.maxSub) g_work.maxSub = sub;
+      g_work.events |= bi == B_PUCK ? 1 : 2;
+    });
     if (!(e.enabled & (1u << minPid)) || !(e.touch & (1u << minPid))) {
       e.enabled &= ~(1u << minPid);
       // restore sweeps (awake/sleep changes made by Update persist, as in b2World::SolveTOI)

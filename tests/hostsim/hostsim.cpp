@@ -14,6 +14,9 @@ namespace hk { long long g_fast_bail[16]; long long g_iter_hist[2][182]; long lo
 
 using namespace hk;
 
+// what one env's last tick did: the WorkRecord of the tier that finished it, then that tier
+enum { WORK_WORDS = 9, TIER_FAST = 0, TIER_TOUCH = 1, TIER_GENERAL = 2 };
+
 struct HostBatch {
   Scene S;
   Config cfg;
@@ -24,6 +27,7 @@ struct HostBatch {
   int use_fast = 0;
   long long nFast = 0, nSlow = 0, nLong = 0, nTouch = 0;
   int mid_budget = 24;
+  std::vector<int32_t> work;  // [n][WORK_WORDS]: hs_last_work
   Cache cacheOf(int64_t i) { Cache c; c.base = cache.data() + i; c.stride = (size_t)n; return c; }
 };
 
@@ -41,6 +45,7 @@ void* hs_create(int64_t n, int mode, int keep_mode, uint64_t seed, int64_t env_i
   b->n = n; b->env_id_offset = env_id_offset;
   b->envs.resize(n);
   b->cache.assign((size_t)n * 27 * 6, 0);
+  b->work.assign((size_t)n * WORK_WORDS, 0);
   std::memset(b->stats, 0, sizeof(b->stats));
   for (int64_t i = 0; i < n; ++i) { std::memset(&b->envs[i], 0, sizeof(Env)); envCreate(b->S, b->cfg, b->envs[i], (uint64_t)(env_id_offset + i)); }
   return b;
@@ -74,19 +79,22 @@ void hs_step(void* h, const float* action, int stride, int pol1, int pol2, int f
     Env e;
     groupsToEnv(g, e);
     TickStats st; tickStatsZero(st);
+    int tier = TIER_GENERAL;
+    std::memset(&g_work, 0, sizeof(g_work));  // every attempt starts a fresh record: the one that finishes the tick keeps it
     bool done_fast = false;
     int bail = 15;
     if (b->use_fast) {
       Env w = e;
       TickStats st2; tickStatsZero(st2);
-      if (envTickFast(b->S, b->cfg, w, (uint64_t)(b->env_id_offset + i), (size_t)i, io, true, st2)) { e = w; st = st2; done_fast = true; }
+      if (envTickFast(b->S, b->cfg, w, (uint64_t)(b->env_id_offset + i), (size_t)i, io, true, st2)) { e = w; st = st2; done_fast = true; tier = TIER_FAST; }
       else bail = w.bailKind;
     }
     bool done_touch = false;
     if (b->use_fast && !done_fast && bailClass(bail) == 0) {  // the touch tier (k_touch) takes work class 0 first
       Env w = e;
       TickStats st2; tickStatsZero(st2);
-      if (envTickTouch(b->S, b->cfg, b->cacheOf(i), w, (uint64_t)(b->env_id_offset + i), (size_t)i, io, true, st2, nullptr)) { e = w; st = st2; done_touch = true; }
+      std::memset(&g_work, 0, sizeof(g_work));
+      if (envTickTouch(b->S, b->cfg, b->cacheOf(i), w, (uint64_t)(b->env_id_offset + i), (size_t)i, io, true, st2, nullptr)) { e = w; st = st2; done_touch = true; tier = TIER_TOUCH; }
     }
     if (done_fast) b->nFast++;
     else if (done_touch) b->nTouch++;
@@ -94,15 +102,21 @@ void hs_step(void* h, const float* action, int stride, int pol1, int pol2, int f
       // the kernel cascade: budgeted middle tier, then the unlimited tier, each from the stored state
       Env w = e;
       TickStats st2; tickStatsZero(st2);
+      std::memset(&g_work, 0, sizeof(g_work));
       if (envTick(b->S, b->cfg, b->cacheOf(i), w, (uint64_t)(b->env_id_offset + i), (size_t)i, io, true, st2, b->mid_budget, false)) { e = w; st = st2; b->nSlow++; }
-      else { b->nLong++; envTick(b->S, b->cfg, b->cacheOf(i), e, (uint64_t)(b->env_id_offset + i), (size_t)i, io, true, st); }
+      else { b->nLong++; std::memset(&g_work, 0, sizeof(g_work)); envTick(b->S, b->cfg, b->cacheOf(i), e, (uint64_t)(b->env_id_offset + i), (size_t)i, io, true, st); }
     } else { b->nSlow++; envTick(b->S, b->cfg, b->cacheOf(i), e, (uint64_t)(b->env_id_offset + i), (size_t)i, io, true, st); }
     b->envs[i] = e;
     addStats(b->stats, st);
+    const int32_t rec[WORK_WORDS] = {g_work.kind, g_work.shape, g_work.sweeps, g_work.toi, g_work.maxSub, g_work.skipAfter, g_work.events, g_work.goal, tier};
+    std::memcpy(&b->work[(size_t)i * WORK_WORDS], rec, sizeof(rec));
   }
 }
 void hs_bail_counts(long long* out) { for (int i = 0; i < 16; ++i) out[i] = hk::g_fast_bail[i]; }
 void hs_iter_hist(long long* out) { for (int w = 0; w < 2; ++w) for (int i = 0; i < 182; ++i) out[w * 182 + i] = hk::g_iter_hist[w][i]; for (int i = 0; i < 16; ++i) out[364 + i] = hk::g_period_hist[i]; }
+// [n][9] int32 of each env's last tick: island solve kind and shape (contacts | points << 4), sweeps, TOI events, highest sub-step count, TOI evaluations
+// skipped after an event, event bodies (1: puck, 2: racket), goal, tier that finished it (0 fast, 1 touch, 2 general)
+void hs_last_work(void* h, int32_t* out) { HostBatch* b = (HostBatch*)h; std::memcpy(out, b->work.data(), b->work.size() * sizeof(int32_t)); }
 void hs_toi_dbg(long long* out) { for (int i = 0; i < 16; ++i) out[i] = hk::g_toi_dbg[i]; }
 void hs_set_fast(void* h, int on) { ((HostBatch*)h)->use_fast = on; }
 void hs_fast_counts(void* h, long long* out) { out[0] = ((HostBatch*)h)->nFast; out[1] = ((HostBatch*)h)->nSlow; out[2] = ((HostBatch*)h)->nLong; out[3] = ((HostBatch*)h)->nTouch; }

@@ -10,19 +10,21 @@ import numpy as np
 import oracle_lib as O
 
 _ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-_DIR = os.path.join(_ROOT, "tests", "hostsim")
-_SO = os.path.join(_DIR, "libhostsim.so")
-_CSRC = os.path.join(_ROOT, "hockey_env_b200", "csrc")
 
 
-def build(force=False):
-    srcs = [os.path.join(_DIR, "hostsim.cpp"), os.path.join(_ROOT, "include", "hockey_b200.h")]
-    srcs += [os.path.join(_CSRC, f) for f in os.listdir(_CSRC) if f.endswith(".cuh")]
-    if not force and os.path.exists(_SO) and all(os.path.getmtime(_SO) >= os.path.getmtime(s) for s in srcs):
-        return _SO
+def build(force=False, root=_ROOT):
+    """compile <root>/tests/hostsim/hostsim.cpp (which includes <root>/hockey_env_b200/csrc and <root>/include by
+    relative path) into libhostsim.so next to it; `root` other than the repository builds a copy, e.g. a mutant"""
+    d = os.path.join(root, "tests", "hostsim")
+    so = os.path.join(d, "libhostsim.so")
+    csrc = os.path.join(root, "hockey_env_b200", "csrc")
+    srcs = [os.path.join(d, "hostsim.cpp"), os.path.join(root, "include", "hockey_b200.h")]
+    srcs += [os.path.join(csrc, f) for f in os.listdir(csrc) if f.endswith(".cuh")]
+    if not force and os.path.exists(so) and all(os.path.getmtime(so) >= os.path.getmtime(s) for s in srcs):
+        return so
     subprocess.check_call(["g++", "-std=c++17", "-O2", "-ffp-contract=off", "-fno-fast-math", "-fPIC", "-shared",
-                           "-x", "c++", "-o", _SO, os.path.join(_DIR, "hostsim.cpp")])
-    return _SO
+                           "-x", "c++", "-o", so, os.path.join(d, "hostsim.cpp")])
+    return so
 
 
 _lib = None
@@ -31,37 +33,50 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(_SO)
-        vp, i64, u64, i32 = C.c_void_p, C.c_int64, C.c_uint64, C.c_int
-        L.hs_create.restype = vp
-        L.hs_create.argtypes = [i64, i32, i32, u64, i64]
-        L.hs_destroy.argtypes = [vp]
-        L.hs_reset.argtypes = [vp, vp, vp, vp]
-        L.hs_reset_seeded.argtypes = [vp, vp, vp, vp, vp]
-        L.hs_get_obs.argtypes = [vp, vp, vp]
-        L.hs_step.argtypes = [vp, vp, i32, i32, i32, i32] + [vp] * 8
-        L.hs_get_state.argtypes = [vp, vp]
-        L.hs_set_state.argtypes = [vp, vp]
-        L.hs_set_obs_state.argtypes = [vp, vp]
-        L.hs_get_stats.argtypes = [vp, vp]
-        L.hs_clear_stats.argtypes = [vp]
-        L.hs_scene.argtypes = [vp, vp, i64]
-        L.hs_scene_size.restype = i64
-        L.hs_set_fast.argtypes = [vp, i32]
-        L.hs_fast_counts.argtypes = [vp, vp]
-        L.hs_set_mid_budget.argtypes = [vp, i32]
-        _lib = L
+        _lib = load(build())
     return _lib
+
+
+def load(so):
+    """ctypes handle of a built libhostsim.so with the argument types set"""
+    L = C.CDLL(so)
+    vp, i64, u64, i32 = C.c_void_p, C.c_int64, C.c_uint64, C.c_int
+    L.hs_create.restype = vp
+    L.hs_create.argtypes = [i64, i32, i32, u64, i64]
+    L.hs_destroy.argtypes = [vp]
+    L.hs_reset.argtypes = [vp, vp, vp, vp]
+    L.hs_reset_seeded.argtypes = [vp, vp, vp, vp, vp]
+    L.hs_get_obs.argtypes = [vp, vp, vp]
+    L.hs_step.argtypes = [vp, vp, i32, i32, i32, i32] + [vp] * 8
+    L.hs_get_state.argtypes = [vp, vp]
+    L.hs_set_state.argtypes = [vp, vp]
+    L.hs_set_obs_state.argtypes = [vp, vp]
+    L.hs_get_stats.argtypes = [vp, vp]
+    L.hs_clear_stats.argtypes = [vp]
+    L.hs_scene.argtypes = [vp, vp, i64]
+    L.hs_scene_size.restype = i64
+    L.hs_set_fast.argtypes = [vp, i32]
+    L.hs_fast_counts.argtypes = [vp, vp]
+    L.hs_set_mid_budget.argtypes = [vp, i32]
+    L.hs_last_work.argtypes = [vp, vp]
+    return L
 
 
 _p = O._p
 
+# columns of HostSimBatch.last_work(): what each env's last tick did (tests/hostsim/hostsim.cpp, hk_world.cuh WorkRecord)
+W_KIND, W_SHAPE, W_SWEEPS, W_TOI, W_MAXSUB, W_SKIP_AFTER, W_EVENTS, W_GOAL, W_TIER = range(9)
+# W_KIND: 1..8 = solveKind (two contacts (1,1) (1,2) (2,1) (2,2), three contacts (1,1,1) (1,1,2) (1,2,1) (2,1,1)),
+# 9 = one contact with one point, 10 = one contact with two points, 11 = the generic loop, 0 = no island solve;
+# W_SHAPE: contacts | points << 4 of that solve; W_EVENTS: bit 0 a puck x static TOI event, bit 1 a racket x static one
+KIND_1C1P, KIND_1C2P, KIND_GENERIC = 9, 10, 11
+TIER_FAST, TIER_TOUCH, TIER_GENERAL = 0, 1, 2
+
 
 class HostSimBatch:
-    def __init__(self, n, mode=0, keep_mode=True, seed=0, env_id_offset=0, fast=False):
+    def __init__(self, n, mode=0, keep_mode=True, seed=0, env_id_offset=0, fast=False, L=None):
         self.n = int(n)
-        self.L = lib()
+        self.L = lib() if L is None else L  # L: another build (load()), e.g. of a mutated copy of the headers
         self.h = self.L.hs_create(self.n, int(mode), int(bool(keep_mode)), int(seed), int(env_id_offset))
         self.L.hs_set_fast(self.h, int(bool(fast)))
 
@@ -123,6 +138,12 @@ class HostSimBatch:
         c = np.zeros(4, np.int64)
         self.L.hs_fast_counts(self.h, _p(c))
         return int(c[3])
+
+    def last_work(self):
+        """[n, 9] int32 record of each env's last tick (columns W_*)"""
+        w = np.zeros((self.n, 9), np.int32)
+        self.L.hs_last_work(self.h, _p(w))
+        return w
 
     def stats(self):
         s = np.zeros(16, np.float64)
